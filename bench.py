@@ -5,6 +5,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm
     torchrun ... bench.py --gpus N --steps K --warmup W            # N > 1 (driver launches this)
     python bench.py --impl reference [...]                         # CPU reference arm
+    python bench.py [...] --dump-outputs DIR                       # also write the last step's results
 
 A "step" is one search of the 173-query CAsT-19 batch over the whole collection.  The collection
 (fixed total size, so scaling is "strong") is row-sharded over the N ranks and resident in HBM;
@@ -87,7 +88,12 @@ def parse_args():
                          "host buffers) after the main run and reports it under `inproc`")
     ap.add_argument("--sustain-seconds", type=float, default=2.0,
                     help="length of the extra back-to-back run reported under `sustained` (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the results of the last one to DIR/scores.npy (float32) and "
+                         "DIR/ids.npy (float64), for output-for-output comparison of two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.config != "c4":
         c = CONFIGS[args.config]
         args.rows, args.nq, args.k = c["rows"], c["nq"], c["k"]
@@ -126,6 +132,28 @@ def ncu_traffic_per_launch(rows_per_launch: float, kernel: str = "umma_score_sel
         return per_row * rows_per_launch
     except Exception:
         return None
+
+
+DUMP_MAX_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir: str, D, I) -> None:
+    """Write what a caller of the timed path receives, (D [nq,k] scores, I [nq,k] ids), as DIR/scores.npy
+    (float32) and DIR/ids.npy (float64: exact for every id below 2**53).  When the files would exceed
+    64 MB in all, only a fixed sample of query rows (seed 0, ascending) is written, and their indices go to
+    DIR/query_rows.npy (float64)."""
+    D = np.asarray(D, dtype=np.float32)
+    I = np.asarray(I).astype(np.float64)
+    nq, k = D.shape
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_MAX_BYTES - 4096          # room for the .npy headers
+    if nq * k * (4 + 8) > budget:
+        max_rows = budget // (k * (4 + 8) + 8)
+        rows = np.sort(np.random.default_rng(0).choice(nq, size=max_rows, replace=False))
+        D, I = D[rows], I[rows]
+        np.save(os.path.join(out_dir, "query_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "scores.npy"), D)
+    np.save(os.path.join(out_dir, "ids.npy"), I)
 
 
 class ClockSampler:
@@ -283,14 +311,16 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    # The requested steps / warm-ups are honoured (a step = one search of the bounded row sample, ~1.3 s on 16
-    # cores; capped so that the run always ends within a few minutes).  `ms_per_step` is what a step really took;
-    # `value` is the metric of the full workload (q/s scaled by rows: exhaustive search is linear in N) and
-    # `ms_per_step_scaled_to_full_rows` the corresponding time of one full-size search.
-    steps = max(1, min(args.steps, 60))
+    # A step = one search of the bounded row sample, ~1.3 s on 16 cores; exactly --steps of them are timed.
+    # `ms_per_step` is what a step really took; `value` is the metric of the full workload (q/s scaled by rows:
+    # exhaustive search is linear in N) and `ms_per_step_scaled_to_full_rows` the corresponding time of one
+    # full-size search.
+    steps = args.steps
     warmup = max(1, min(args.warmup, 10))
     sample_rows = min(args.cpu_sample_rows, args.rows)
-    cb, _ = cpu_reference_search(sample_rows, args.nq, args.k, steps, warmup, args.rows)
+    cb, (_, _, Dc, Ic) = cpu_reference_search(sample_rows, args.nq, args.k, steps, warmup, args.rows)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, Dc, Ic)
     line = {
         "impl": "reference", "metric": metric_name(args), "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
         "steps": steps, "warmup": warmup,
@@ -428,6 +458,8 @@ def run_b2f_arm(args):
     barrier()
     sampler.mark()
     dev_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:      # every rank holds the same merged result
+        dump_outputs(args.dump_outputs, Dd.cpu().numpy(), Id.cpu().numpy())
     launches, score_ms, score_launches = index.stat("launches"), index.stat("score_ms"), index.stat("score_launches")
     score_rows, select_ms = index.stat("score_rows"), index.stat("select_ms")
     passes_per_search, qs_passes = index.stat("passes") / max(args.steps, 1), index.stat("qs_passes") / max(args.steps, 1)
@@ -634,6 +666,8 @@ def run_sweep(args, index, sharded, stream, barrier, dev, world, rank, n_local, 
                        "sorted_desc": bool((Dd[:, 1:] <= Dd[:, :-1]).all().item())})
         if rank == 0:
             print(json.dumps(points[-1]), file=sys.stderr, flush=True)
+    if args.dump_outputs and rank == 0:      # the last search of the last batch size
+        dump_outputs(args.dump_outputs, Dd.cpu().numpy(), Id.cpu().numpy())
     if rank == 0:
         best = max(points, key=lambda p: p["queries_per_s"])
         cross = next((p["nq"] for p in points if p["bound"] == "tensor"), None)
