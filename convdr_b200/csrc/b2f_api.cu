@@ -131,7 +131,8 @@ struct Workspace {
   float* q32 = nullptr;
   __nv_bfloat16* q16 = nullptr;
   float* qnorm = nullptr;
-  float* qerr = nullptr;      // [nq] upper bound of ||q - bf16(q)||
+  float* qerr = nullptr;      // [nq] upper bound of ||q - bf16(q)|| (int8 shadow: of ||q - sq q8||)
+  float* qscale = nullptr;    // [nq] int8 shadow: query scales sq (the int8 codes live in q16's buffer)
   int* ovf_all = nullptr;
   int* ovf_host = nullptr;  // pinned
   // per-shard results of one search
@@ -181,7 +182,11 @@ struct Shard {
   int sm_count = 148;
   int max_pairs = 74;
   float* x32 = nullptr;
-  __nv_bfloat16* x16 = nullptr;
+  __nv_bfloat16* x16 = nullptr;     // bf16 shadow (format 1)
+  int8_t* x8 = nullptr;              // int8 shadow (format 2) ...
+  float* tscale = nullptr;           // ... and its per-32-row-tile scales
+  int fmt = 0;                       // shadow format of the buffers: 0 none / not chosen yet, 1 bf16, 2 int8
+  double rho = 0;                    // AUTO: median 2 eps8 / sigma of the probe (0: not measured)
   int64_t n = 0, cap = 0;
   unsigned int* maxnorm2 = nullptr;  // device, float bits: [0] max ||p||^2, [1] max ||(p - mu) - shadow||^2, [2] max ||p - mu||^2
   float* mu = nullptr;               // device [768]: the shard's centre (zeros until set / when centring is off)
@@ -285,7 +290,7 @@ struct b2f_index {
   std::mutex ntotal_mutex;     // b2f_add_flat_file may run on several shards at once (one host thread each)
   // options
   int path = B2F_PATH_AUTO;
-  int shadow = 1;
+  int shadow = kShadowAuto;   // 0 none, 1 bf16, 2 int8, 3 AUTO (per shard, from its first rows; DESIGN.md section 4)
   int growth = 32;
   int64_t margin_ppm = 1000000;
   int keep_on_reset = 1;
@@ -341,33 +346,42 @@ int ensure_capacity(b2f_index* idx, Shard& S, int64_t need) {
   CU_TRY(cudaSetDevice(S.dev));
   int64_t ncap = std::max<int64_t>(need, S.cap + S.cap / 2);
   if (S.n == 0) {   // nothing to keep: release first, so that regrowing a large empty shard never holds both copies
-    dev_free(S.x32); dev_free(S.x16); dev_free(S.idmap);
+    dev_free(S.x32); dev_free(S.x16); dev_free(S.x8); dev_free(S.tscale); dev_free(S.idmap);
     S.cap = 0;
     ncap = need;
   }
   float* n32 = nullptr;
   __nv_bfloat16* n16 = nullptr;
+  int8_t* n8 = nullptr;
+  float* nts = nullptr;
   int64_t* nid = nullptr;
   B2F_TRY(dev_alloc(&n32, static_cast<size_t>(ncap) * kD));
-  if (idx->shadow) {
-    int rc = dev_alloc(&n16, static_cast<size_t>(shadow_rows_padded(ncap)) * kD);
-    if (rc != B2F_OK) { dev_free(n32); return rc; }
+  // the shadow in the shard's format; under AUTO an empty shard has none yet (ingest_rows allocates it once the
+  // first rows have decided the format, so a reserve() never commits bf16-sized memory for an int8 shard)
+  int rc = B2F_OK;
+  if (S.fmt == kShadowBf16) rc = dev_alloc(&n16, static_cast<size_t>(shadow_rows_padded(ncap)) * kD);
+  if (S.fmt == kShadowInt8) {
+    rc = dev_alloc(&n8, static_cast<size_t>(shadow_rows_padded(ncap)) * kD);
+    if (rc == B2F_OK) rc = dev_alloc(&nts, static_cast<size_t>(shadow_rows_padded(ncap) / kShadowTileRows + 16));
   }
-  if (S.has_ids) {
-    int rc = dev_alloc(&nid, static_cast<size_t>(ncap));
-    if (rc != B2F_OK) { dev_free(n32); dev_free(n16); return rc; }
-  }
+  if (rc == B2F_OK && S.has_ids) rc = dev_alloc(&nid, static_cast<size_t>(ncap));
+  if (rc != B2F_OK) { dev_free(n32); dev_free(n16); dev_free(n8); dev_free(nts); return rc; }
   if (S.n > 0) {
     CU_TRY(cudaMemcpyAsync(n32, S.x32, static_cast<size_t>(S.n) * kD * 4, cudaMemcpyDeviceToDevice, S.stream));
     if (n16 && S.x16)
       CU_TRY(cudaMemcpyAsync(n16, S.x16, static_cast<size_t>(shadow_rows_padded(S.n)) * kD * 2,
                              cudaMemcpyDeviceToDevice, S.stream));  // tiles are stored in row order
+    if (n8 && S.x8) {
+      CU_TRY(cudaMemcpyAsync(n8, S.x8, static_cast<size_t>(shadow_rows_padded(S.n)) * kD, cudaMemcpyDeviceToDevice, S.stream));
+      CU_TRY(cudaMemcpyAsync(nts, S.tscale, static_cast<size_t>(shadow_rows_padded(S.n) / kShadowTileRows) * 4,
+                             cudaMemcpyDeviceToDevice, S.stream));
+    }
     if (nid && S.idmap)
       CU_TRY(cudaMemcpyAsync(nid, S.idmap, static_cast<size_t>(S.n) * 8, cudaMemcpyDeviceToDevice, S.stream));
     CU_TRY(cudaStreamSynchronize(S.stream));
   }
-  dev_free(S.x32); dev_free(S.x16); dev_free(S.idmap);
-  S.x32 = n32; S.x16 = n16; S.idmap = nid; S.cap = ncap;
+  dev_free(S.x32); dev_free(S.x16); dev_free(S.x8); dev_free(S.tscale); dev_free(S.idmap);
+  S.x32 = n32; S.x16 = n16; S.x8 = n8; S.tscale = nts; S.idmap = nid; S.cap = ncap;
   return B2F_OK;
 }
 
@@ -401,6 +415,55 @@ int launch_grid_rows(const Shard& S, int64_t rows) {
   return static_cast<int>(std::min<int64_t>(std::max<int64_t>(blocks, 1), static_cast<int64_t>(S.sm_count) * 8));
 }
 
+bool has_shadow(const Shard& S) { return S.x16 != nullptr || S.x8 != nullptr; }
+
+// AUTO format choice at the first ingest of a shard (DESIGN.md section 4): 64 evenly spaced rows among the first
+// m <= 65,536 act as pseudo-queries; with sigma_j the spread of their centred scores over 4096 sample rows and
+// eps8_j the int8 margin from the sample's own bounds (int8 tiles of the first m rows, not stored), int8 is chosen
+// when the median of 2 eps8_j / sigma_j is <= 1.2 (tools/margin_model.py: ~0.8 for isotropic rows, ~1.9 for rows
+// with a common mean, where the int8 margin would let tens of thousands of rows per query through).  Fewer than
+// 4096 rows or no spread (all-equal rows): bf16.  Only speed depends on this choice, never the results.
+int choose_format(Shard& S, int64_t n, int* fmt) {
+  const int64_t m = std::min<int64_t>(n, kMuRows);
+  S.rho = 0;
+  *fmt = kShadowBf16;
+  if (m < 4096) return B2F_OK;
+  constexpr int kProbeQ = 64, kProbeRows = 4096;
+  // scratch: the partial column sums of the centre are consumed by now (stream order)
+  unsigned char* scratch = reinterpret_cast<unsigned char*>(S.mu_part);
+  unsigned int* bounds = reinterpret_cast<unsigned int*>(scratch);
+  double* stat = reinterpret_cast<double*>(scratch + 64);
+  float* qstat = reinterpret_cast<float*>(scratch + 64 + 16 * kProbeQ);
+  CU_TRY(cudaMemsetAsync(scratch, 0, 64 + 24 * kProbeQ, S.stream));
+  convert_rows_i8_kernel<<<launch_grid_rows(S, m / kShadowTileRows), 256, 0, S.stream>>>(S.x32, nullptr, nullptr, 0, m,
+                                                                                              bounds, S.mu);
+  shadow_probe_kernel<<<dim3(16, kProbeQ), 256, 0, S.stream>>>(S.x32, m, kProbeRows, S.mu, stat, qstat);
+  CU_TRY(cudaGetLastError());
+  unsigned char host[64 + 24 * kProbeQ];
+  CU_TRY(cudaMemcpyAsync(host, scratch, sizeof(host), cudaMemcpyDeviceToHost, S.stream));
+  CU_TRY(cudaStreamSynchronize(S.stream));
+  unsigned int hb[3];
+  std::memcpy(hb, host, sizeof(hb));
+  auto bits2f = [](unsigned int u) { float f; std::memcpy(&f, &u, 4); return static_cast<double>(f); };
+  const double E8 = std::sqrt(bits2f(hb[1])), P = std::sqrt(bits2f(hb[2]));
+  std::vector<double> rho(kProbeQ);
+  for (int j = 0; j < kProbeQ; ++j) {
+    double s1, s2;
+    float qn, qe;
+    std::memcpy(&s1, host + 64 + 16 * j, 8);
+    std::memcpy(&s2, host + 64 + 16 * j + 8, 8);
+    std::memcpy(&qn, host + 64 + 16 * kProbeQ + 8 * j, 4);
+    std::memcpy(&qe, host + 64 + 16 * kProbeQ + 8 * j + 4, 4);
+    const double mean = s1 / kProbeRows, var = std::max(0.0, s2 / kProbeRows - mean * mean);
+    const double eps = (qn + qe) * E8 + qe * P;
+    rho[j] = var > 0 ? 2 * eps / std::sqrt(var) : HUGE_VAL;
+  }
+  std::nth_element(rho.begin(), rho.begin() + kProbeQ / 2, rho.end());
+  S.rho = rho[kProbeQ / 2];
+  if (std::isfinite(S.rho) && S.rho <= 1.2) *fmt = kShadowInt8;
+  return B2F_OK;
+}
+
 // Append rows already resident at x32[S.n .. S.n+n): build shadow + norm bound.
 int ingest_rows(b2f_index* idx, Shard& S, int64_t n) {
   if (!S.mu_set) {
@@ -414,10 +477,29 @@ int ingest_rows(b2f_index* idx, Shard& S, int64_t n) {
       col_mean_final_kernel<<<(kD + 255) / 256, 256, 0, S.stream>>>(S.mu_part, blocks, m, S.mu);
       CU_TRY(cudaGetLastError());
     }
+    if (S.n == 0) {
+      // the shadow format of these rows (AUTO: from the rows themselves); buffers of another format are replaced
+      int fmt = idx->shadow;
+      if (fmt == kShadowAuto) B2F_TRY(choose_format(S, n, &fmt));
+      if (fmt != S.fmt || (fmt == kShadowBf16 && !S.x16) || (fmt == kShadowInt8 && !S.x8)) {
+        dev_free(S.x16); dev_free(S.x8); dev_free(S.tscale);
+        S.fmt = fmt;
+        if (fmt == kShadowBf16) B2F_TRY(dev_alloc(&S.x16, static_cast<size_t>(shadow_rows_padded(S.cap)) * kD));
+        if (fmt == kShadowInt8) {
+          B2F_TRY(dev_alloc(&S.x8, static_cast<size_t>(shadow_rows_padded(S.cap)) * kD));
+          B2F_TRY(dev_alloc(&S.tscale, static_cast<size_t>(shadow_rows_padded(S.cap) / kShadowTileRows + 16)));
+        }
+      }
+    }
     S.mu_set = true;
   }
-  convert_rows_kernel<<<launch_grid_rows(S, n), 256, 0, S.stream>>>(S.x32, idx->shadow ? S.x16 : nullptr, S.n, n,
-                                                                    S.maxnorm2, S.mu);
+  if (S.fmt == kShadowInt8) {
+    const int64_t tiles = (S.n + n + kShadowTileRows - 1) / kShadowTileRows - S.n / kShadowTileRows;
+    convert_rows_i8_kernel<<<launch_grid_rows(S, tiles), 256, 0, S.stream>>>(S.x32, S.x8, S.tscale, S.n, n,
+                                                                                S.maxnorm2, S.mu);
+  } else {
+    convert_rows_kernel<<<launch_grid_rows(S, n), 256, 0, S.stream>>>(S.x32, S.x16, S.n, n, S.maxnorm2, S.mu);
+  }
   CU_TRY(cudaGetLastError());
   return B2F_OK;
 }
@@ -425,13 +507,14 @@ int ingest_rows(b2f_index* idx, Shard& S, int64_t n) {
 int ensure_query_ws(Shard& S, int64_t nq, int k) {
   Workspace& W = S.ws;
   if (nq > W.nq_cap) {
-    dev_free(W.q32); dev_free(W.q16); dev_free(W.qnorm); dev_free(W.qerr);
+    dev_free(W.q32); dev_free(W.q16); dev_free(W.qnorm); dev_free(W.qerr); dev_free(W.qscale);
     if (W.ovf_host) { cudaFreeHost(W.ovf_host); W.ovf_host = nullptr; W.ovf_all = nullptr; }
     const int64_t cap = std::max<int64_t>(nq, 256);
     B2F_TRY(dev_alloc(&W.q32, static_cast<size_t>(cap) * kD));
     B2F_TRY(dev_alloc(&W.q16, static_cast<size_t>(cap + kUmmaMaxQ + 16) * kD));
     B2F_TRY(dev_alloc(&W.qnorm, static_cast<size_t>(cap + kUmmaMaxQ + 16)));
     B2F_TRY(dev_alloc(&W.qerr, static_cast<size_t>(cap + kUmmaMaxQ + 16)));
+    B2F_TRY(dev_alloc(&W.qscale, static_cast<size_t>(cap + kUmmaMaxQ + 16)));
     // per-query overflow flags live in mapped pinned host memory: the last kernel of a pass writes them
     // straight to the host (no copy operation on the stream), the host reads them after the sync
     CU_TRY(cudaHostAlloc(reinterpret_cast<void**>(&W.ovf_host), static_cast<size_t>(cap) * kMaxPending * sizeof(int),
@@ -505,6 +588,13 @@ int ensure_pin(Shard& S, size_t bytes) {
 //     where p stands for the centred row p - mu and p^ for its bf16 shadow,
 //     E = max ||p - p^|| and P = max ||p|| (kept per shard at add time), e_q = ||q - q^||, g = 1.1e-4 >= 768 * 2^-23
 //     (fp32 accumulation of 768 exact products inside the tensor core, truncation allowed).
+//   mode 4 (int8 tensor):  q^ = sq q8, p^ = st p8 (real products of the fp32 scales and the int8 codes); the tensor
+//     core sums the 768 code products exactly in int32, so s~ = q^ . p^ exactly and
+//       |s~ - s| <= |q^ . (p^ - p)| + |(q^ - q) . p| <= (||q|| + e_q) E8 + e_q P,
+//     with E8 = max ||p - p^|| (slot [1] of an int8 shard, kept at add time), e_q = ||q - q^||, ||q^|| <= ||q|| + e_q.
+//     No accumulation term.  What is compared and recorded are fp32 images of s~: the threshold test is exact on
+//     s~ (i8_threshold), the recorded score fl(fl(acc) fl(sq st)) is within 2^-23 |s~| of it, and
+//     |s~| <= ||q^|| ||p^|| <= (||q|| + e_q)(P + E8): the term 2^-21 (||q|| + e_q)(P + E8) covers it 4x over.
 // Every factor is an upper bound and every operation rounds up; `scale` (margin_ppm) multiplies the result.
 __global__ void pass_init_kernel(const float* __restrict__ qnorm, const float* __restrict__ qerr,
                                  const unsigned int* __restrict__ maxnorm2_bits, int mode, float scale, float u_scan,
@@ -543,6 +633,13 @@ __global__ void pass_init_kernel(const float* __restrict__ qnorm, const float* _
       const float a = __fmul_ru(__fmul_ru(qnorm[q], E), 1.00390625f);   // ||bf16(q)|| <= (1 + 2^-8) ||q||
       const float b = __fmul_ru(qerr[q], P);
       const float c = __fmul_ru(__fmul_ru(qnorm[q], P), 1.1e-4f);
+      eps = __fadd_ru(__fadd_ru(a, b), c);
+    } else if (mode == 4) {
+      const float E = __fsqrt_ru(__uint_as_float(maxnorm2_bits[1]));
+      const float qh = __fadd_ru(qnorm[q], qerr[q]);
+      const float a = __fmul_ru(qh, E);
+      const float b = __fmul_ru(qerr[q], P);
+      const float c = __fmul_ru(__fmul_ru(qh, __fadd_ru(P, E)), 4.76837158203125e-7f);   // 2^-21
       eps = __fadd_ru(__fadd_ru(a, b), c);
     }
     margin[q] = __fmul_ru(__fmul_ru(eps, 2.0f), scale);
@@ -629,7 +726,11 @@ PassPlan make_plan(const b2f_index* idx, const Shard& S, int path, int k, int64_
     // survivors within the margin of the k-th score: ~k * (e^(z * 2eps / sigma) - 1) with z ~ 5 the tail slope
     // at rank 100 of 4e7: ~200 for isotropic unit rows, ~700 for LayerNorm-like rows with a common mean after
     // centring (DESIGN.md section 4) — 4096 leaves a factor of 5
-    p.S = static_cast<int>(round_up(std::max(4096, 4 * k), 256));
+    // int8 shadow: a margin ~4x wider (2 eps / sigma ~0.8 instead of ~0.2 on isotropic rows): the rescoring
+    // window holds ~650 rows per query at k = 100 and ~4.5k at k = 1000 on 8.8 M rows, so S follows 8k (up to the
+    // 8192 records finalize_kernel keeps in shared memory)
+    const int s_k = S.fmt == kShadowInt8 ? std::max(4 * k, std::min(8 * k, 8192)) : 4 * k;
+    p.S = static_cast<int>(round_up(std::max(4096, s_k), 256));
     // expected appends per (query, area) in a phase: 2 (margin) * (growth-1) * k / areas; x2 safety
     // (with in-kernel tightening the pass rate follows k/rows_seen, far fewer appends; keep the bound)
     const int64_t expect = 4ll * (std::max(2, idx->growth) - 1) * k / S.max_pairs;
@@ -657,7 +758,7 @@ int pass_variant(const b2f_index* idx, const PassPlan& plan, int nqp) {
 // D_out/I_out with row stride out_stride.
 int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q32p, const __nv_bfloat16* q16p,
                  const float* qnormp, const float* qerrp, int nqp, int k, float* D_out, int64_t* I_out, int64_t out_stride,
-                 int* ovf_dst) {
+                 int* ovf_dst, const float* qscalep = nullptr) {
   Workspace& W = S.ws;
   Stats& st = S.stats;   // per shard: shards may be enqueued from different host threads
   const int64_t N = S.n;
@@ -678,7 +779,8 @@ int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q3
   }
   const int n_areas = 2 * S.max_pairs;   // TS: two per CTA pair (one per half tile); QS: one per CTA
   const int cap_h = plan.cap_p / 2;       // TS: slots per (query, pair, half tile)
-  const int margin_mode = plan.exact ? 0 : (plan.path == B2F_PATH_UMMA_BF16 ? (idx->worst_case_margin ? 3 : 2) : 1);
+  const bool i8 = S.fmt == kShadowInt8;
+  const int margin_mode = plan.exact ? 0 : (plan.path == B2F_PATH_UMMA_BF16 ? (i8 ? 4 : (idx->worst_case_margin ? 3 : 2)) : 1);
   pass_init_kernel<<<nqp, 128, 0, s>>>(qnormp, qerrp, S.maxnorm2, margin_mode,
                                        static_cast<float>(idx->margin_ppm * 1e-6 * 1.0000001), static_cast<float>(kUScan),
                                        W.margin, W.cnt, W.ovf, (tensor || tensor_qs) ? W.cnt2 : nullptr, n_areas,
@@ -688,13 +790,16 @@ int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q3
   if (tensor_qs) {
     // ---- QS: one launch over the whole shard, then the fused last step ----
     const int n_cols = static_cast<int>(round_up(nqp, 16));
-    const QsPlan qp = umma_qs_plan(n_cols, idx->umma_variant == 1 ? kNumKBlocks : idx->qs_resident_kb, idx->qs_q_stages,
-                                   idx->qs_half_stage);
+    // int8: 6 K-blocks of 128 bytes; the tensor maps only move bytes, so they describe the int8 rows as bf16 pairs
+    const int n_kb = i8 ? kShadow8KBlocks : kNumKBlocks;
+    const QsPlan qp = umma_qs_plan(n_cols, idx->umma_variant == 1 ? n_kb : std::min(idx->qs_resident_kb * n_kb / kNumKBlocks, n_kb),
+                                   idx->qs_q_stages, i8 ? 0 : idx->qs_half_stage, n_kb);
     CUtensorMap tmap_p, tmap_ph, tmap_q;
-    const uint64_t srows = static_cast<uint64_t>(shadow_rows_padded(N)) * kNumKBlocks;
-    B2F_TRY(make_tmap_bf16(&tmap_p, S.x16, srows, kBlockK, kShadowTileRows));        // one K-block of a 32-row tile
-    B2F_TRY(make_tmap_bf16(&tmap_ph, S.x16, srows, kBlockK, kShadowTileRows, true)); // half a K-block of a 32-row tile
-    B2F_TRY(make_tmap_bf16(&tmap_q, q16p, static_cast<uint64_t>(n_cols), kD, static_cast<uint32_t>(n_cols / 2)));
+    const void* shadow = i8 ? static_cast<const void*>(S.x8) : static_cast<const void*>(S.x16);
+    const uint64_t srows = static_cast<uint64_t>(shadow_rows_padded(N)) * n_kb;
+    B2F_TRY(make_tmap_bf16(&tmap_p, shadow, srows, kBlockK, kShadowTileRows));        // one K-block of a 32-row tile
+    B2F_TRY(make_tmap_bf16(&tmap_ph, shadow, srows, kBlockK, kShadowTileRows, true)); // half a K-block of a 32-row tile
+    B2F_TRY(make_tmap_bf16(&tmap_q, q16p, static_cast<uint64_t>(n_cols), i8 ? kD / 2 : kD, static_cast<uint32_t>(n_cols / 2)));
     const int te = static_cast<int>((N + kQsTileRows - 1) / kQsTileRows);
     UmmaQsArgs a;
     a.n_rows = N; a.tile_begin = 0; a.tile_end = te; a.n_cols = n_cols; a.nq = nqp;
@@ -708,14 +813,16 @@ int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q3
     // histogram: 2 * pairs * 32 rows per quarter, about half of which score above the histogram floor), the
     // other quarters wait until every query has a threshold (bounded: first_wait_cycles).  Shards too small
     // to fill the first tiles do not wait.
-    a.x16_bytes = reinterpret_cast<const unsigned char*>(S.x16);
-    a.pf_limit_bytes = shadow_rows_padded(N) * static_cast<int64_t>(kD) * 2;
+    a.x16_bytes = static_cast<const unsigned char*>(shadow);
+    a.pf_limit_bytes = shadow_rows_padded(N) * static_cast<int64_t>(kD) * (i8 ? 1 : 2);
+    a.qscale = qscalep; a.tscale = S.tscale;
     a.prefetch = idx->l2_prefetch;
     a.dense_quarters = std::min(4, std::max(1, (4 * k + 2 * pairs * 32 - 1) / (2 * pairs * 32)));
     a.first_wait_cycles = (idx->tighten && N >= 4ll * pairs * kQsTileRows && a.dense_quarters < 4) ? 100000 : 0;
     {
       ProfScope ps(idx, S, 0);
-      umma_qs_score_select_kernel<<<2 * pairs, kQsThreads, qp.smem_bytes, s>>>(tmap_p, tmap_ph, tmap_q, a);
+      if (i8) umma_qs_score_select_kernel<true><<<2 * pairs, kQsThreads, qp.smem_bytes, s>>>(tmap_p, tmap_ph, tmap_q, a);
+      else umma_qs_score_select_kernel<false><<<2 * pairs, kQsThreads, qp.smem_bytes, s>>>(tmap_p, tmap_ph, tmap_q, a);
     }
     CU_TRY(cudaGetLastError());
     st.score_rows += static_cast<double>(N);
@@ -741,8 +848,11 @@ int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q3
   CUtensorMap tmap_p;
   if (tensor) {
     // shadow = [row tiles x 12 K-blocks x tile rows, 64 columns] bf16; box = 128 x 128 B = 16 KB
-    B2F_TRY(make_tmap_bf16(&tmap_p, S.x16, static_cast<uint64_t>(shadow_rows_padded(N)) * kNumKBlocks, kBlockK,
-                           kKBlocksPerStage * kTileRowsCta));
+    // (int8: 6 K-blocks of 128 bytes per tile, boxes of 3 K-blocks = 12 KB)
+    if (i8) B2F_TRY(make_tmap_bf16(&tmap_p, S.x8, static_cast<uint64_t>(shadow_rows_padded(N)) * kShadow8KBlocks, kBlockK,
+                                   3 * kTileRowsCta));
+    else B2F_TRY(make_tmap_bf16(&tmap_p, S.x16, static_cast<uint64_t>(shadow_rows_padded(N)) * kNumKBlocks, kBlockK,
+                                kKBlocksPerStage * kTileRowsCta));
   }
 
   // Phase boundaries in rows.  Dense phase first, then geometric growth (or, in exact mode,
@@ -764,6 +874,7 @@ int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q3
       if (end < N) end = static_cast<int64_t>(te) * kTileRows;  // phases end on tile boundaries
       UmmaArgs a;
       a.n_rows = N; a.tile_begin = tb; a.tile_end = te; a.nq = nqp; a.q16 = q16p;
+      a.qscale = qscalep; a.tscale = S.tscale;
       a.dense = dense ? 1 : 0; a.cand = W.cand[cur]; a.C = C; a.S = plan.S; a.cap_p = cap_h;
       a.max_pairs = n_areas; a.cnt2 = W.cnt2; a.tau = W.tau; a.ovf = W.ovf; a.err = W.err;
       a.tighten = idx->tighten; a.tighten_adaptive = idx->tighten_adaptive; a.k = k; a.margin = W.margin; a.hist = W.hist; a.hkey0 = W.hkey0; a.hshift = W.hshift;
@@ -774,7 +885,8 @@ int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q3
       a.first_wait_cycles = (one_launch && N >= 8ll * pairs * kTileRows && 4ll * k <= static_cast<int64_t>(pairs) * kTileRows) ? 100000 : 0;
       {
         ProfScope ps(idx, S, 0);
-        umma_score_select_kernel<<<2 * pairs, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
+        if (i8) umma_score_select_kernel<true><<<2 * pairs, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
+        else umma_score_select_kernel<false><<<2 * pairs, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
       }
       st.score_rows += static_cast<double>(std::min<int64_t>(N, static_cast<int64_t>(te) * kTileRows) - begin);
     } else {
@@ -858,10 +970,10 @@ int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q3
 int resolve_path(const b2f_index* idx, const Shard& S, int64_t nq) {
   int path = idx->path;
   if (path == B2F_PATH_AUTO) {
-    if (!S.x16) path = B2F_PATH_SCAN_F32;
+    if (!has_shadow(S)) path = B2F_PATH_SCAN_F32;
     else path = (nq <= idx->scan_max_auto) ? B2F_PATH_SCAN_F32 : B2F_PATH_UMMA_BF16;
   }
-  if (path == B2F_PATH_UMMA_BF16 && !S.x16) path = B2F_PATH_SCAN_F32;
+  if (path == B2F_PATH_UMMA_BF16 && !has_shadow(S)) path = B2F_PATH_SCAN_F32;
   return path;
 }
 
@@ -885,15 +997,21 @@ int enqueue_search(b2f_index* idx, Shard& S, const float* q_d, int64_t nq, int k
   B2F_TRY(ensure_pass_ws(S, plan.qp, plan.C));
   B2F_TRY(upload_segs(S));
   const int64_t nq_pad = round_up(nq, 16) + kUmmaMaxQ;
-  prep_queries_kernel<<<static_cast<int>((nq_pad * 32 + 127) / 128), 128, 0, s>>>(
-      q_d, static_cast<int>(nq), static_cast<int>(nq_pad), W.q16, W.qnorm, W.qerr);
+  if (S.fmt == kShadowInt8)   // int8 codes in the bf16 query buffer (half its size)
+    prep_queries_i8_kernel<<<static_cast<int>((nq_pad * 32 + 127) / 128), 128, 0, s>>>(
+        q_d, static_cast<int>(nq), static_cast<int>(nq_pad), reinterpret_cast<int8_t*>(W.q16), W.qscale, W.qnorm, W.qerr);
+  else
+    prep_queries_kernel<<<static_cast<int>((nq_pad * 32 + 127) / 128), 128, 0, s>>>(
+        q_d, static_cast<int>(nq), static_cast<int>(nq_pad), W.q16, W.qnorm, W.qerr);
   CU_TRY(cudaGetLastError());
   S.stats.launches += 1;
   if (plan.path == B2F_PATH_UMMA_BF16) {
     static bool attr_set[64] = {false};
     if (!attr_set[S.dev & 63]) {
-      CU_TRY(cudaFuncSetAttribute(umma_score_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kUmmaSmemBytes));
-      CU_TRY(cudaFuncSetAttribute(umma_qs_score_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kQsSmemLimit));
+      CU_TRY(cudaFuncSetAttribute(umma_score_select_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kUmmaSmemBytes));
+      CU_TRY(cudaFuncSetAttribute(umma_score_select_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kUmmaSmemBytes));
+      CU_TRY(cudaFuncSetAttribute(umma_qs_score_select_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kQsSmemLimit));
+      CU_TRY(cudaFuncSetAttribute(umma_qs_score_select_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kQsSmemLimit));
       CU_TRY(cudaFuncSetAttribute(finalize_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * 8192 * 8));   // P + PS records
       CU_TRY(cudaFuncSetAttribute(bootstrap_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 16384 * 8));
       attr_set[S.dev & 63] = true;
@@ -908,8 +1026,11 @@ int enqueue_search(b2f_index* idx, Shard& S, const float* q_d, int64_t nq, int k
   }
   for (int64_t q0 = 0; q0 < nq; q0 += plan.qp) {
     const int nqp = static_cast<int>(std::min<int64_t>(plan.qp, nq - q0));
-    B2F_TRY(enqueue_pass(idx, S, plan, q_d + q0 * kD, W.q16 + q0 * kD, W.qnorm + q0, W.qerr + q0, nqp, k, D_d + q0 * k,
-                         I_d + q0 * k, k, ovf_slot + q0));
+    // the pass's queries: bf16 rows, or int8 rows (half the bytes) in the same buffer
+    const __nv_bfloat16* q16p = S.fmt == kShadowInt8 ? reinterpret_cast<const __nv_bfloat16*>(reinterpret_cast<const int8_t*>(W.q16) + q0 * kD)
+                                                     : W.q16 + q0 * kD;
+    B2F_TRY(enqueue_pass(idx, S, plan, q_d + q0 * kD, q16p, W.qnorm + q0, W.qerr + q0, nqp, k, D_d + q0 * k,
+                         I_d + q0 * k, k, ovf_slot + q0, W.qscale + q0));
   }
   return B2F_OK;
 }
@@ -1119,7 +1240,7 @@ void b2f_destroy(b2f_index* idx) {
     cudaSetDevice(S.dev);
     if (S.stream) cudaStreamSynchronize(S.stream);
     Workspace& W = S.ws;
-    dev_free(S.x32); dev_free(S.x16); dev_free(S.idmap); dev_free(S.maxnorm2); dev_free(S.segs_d);
+    dev_free(S.x32); dev_free(S.x16); dev_free(S.x8); dev_free(S.tscale); dev_free(S.idmap); dev_free(S.maxnorm2); dev_free(S.segs_d);
     dev_free(S.mu); dev_free(S.mu_part);
     for (int b = 0; b < kLoadBufs; ++b) {
       if (S.load_bufs[b]) cudaFreeHost(S.load_bufs[b]);
@@ -1283,7 +1404,7 @@ int b2f_reset(b2f_index* idx) {
     CU_TRY(cudaMemsetAsync(S.mu, 0, kD * sizeof(float), S.stream));
     S.mu_set = false;
     if (!idx->keep_on_reset) {
-      dev_free(S.x32); dev_free(S.x16); dev_free(S.idmap);
+      dev_free(S.x32); dev_free(S.x16); dev_free(S.x8); dev_free(S.tscale); dev_free(S.idmap);
       S.cap = 0;
     }
   }
@@ -1637,11 +1758,15 @@ int b2f_set_option(b2f_index* idx, const char* key, int64_t value) {
     idx->path = static_cast<int>(value);
   } else if (k == "shadow") {
     if (idx->ntotal > 0) return fail(B2F_ERR_INVALID, "shadow can only be changed on an empty index");
-    idx->shadow = value ? 1 : 0;
-    if (!idx->shadow)
-      for (Shard& S : idx->shards) { cudaSetDevice(S.dev); dev_free(S.x16); }
-    else
-      for (Shard& S : idx->shards) { cudaSetDevice(S.dev); dev_free(S.x32); dev_free(S.x16); dev_free(S.idmap); S.cap = 0; }
+    if (value < 0 || value > 3) return fail(B2F_ERR_INVALID, "shadow must be 0 (none), 1 (bf16), 2 (int8) or 3 (auto)");
+    idx->shadow = static_cast<int>(value);
+    for (Shard& S : idx->shards) {
+      cudaSetDevice(S.dev);
+      dev_free(S.x32); dev_free(S.x16); dev_free(S.x8); dev_free(S.tscale); dev_free(S.idmap);
+      S.cap = 0;
+      S.fmt = idx->shadow == kShadowAuto ? 0 : idx->shadow;
+      S.mu_set = false;
+    }
   } else if (k == "growth") {
     if (value < 2 || value > 1024) return fail(B2F_ERR_INVALID, "growth must be in [2, 1024]");
     idx->growth = static_cast<int>(value);
@@ -1712,7 +1837,9 @@ int b2f_get_stat(const b2f_index* idx, const char* key, double* out) {
     s.qs_passes = idx->shards[0].stats.qs_passes;
     s.phases = idx->shards[0].stats.phases;
   }
-  if (k == "launches") *out = s.launches;
+  if (k == "shadow_format") *out = idx->shards.empty() ? 0 : idx->shards[0].fmt;   // 0 none, 1 bf16, 2 int8
+  else if (k == "shadow_rho") *out = idx->shards.empty() ? 0 : idx->shards[0].rho;  // AUTO: median 2 eps8 / sigma
+  else if (k == "launches") *out = s.launches;
   else if (k == "phases") *out = s.phases;
   else if (k == "candidates") *out = s.candidates;
   else if (k == "fallback_queries") *out = s.fallback_queries;

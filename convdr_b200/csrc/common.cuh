@@ -29,6 +29,20 @@ __host__ __device__ __forceinline__ int64_t shadow_index(int64_t row, int col) {
 __host__ __device__ __forceinline__ int64_t shadow_rows_padded(int64_t rows) {
   return (rows + kShadowTileRows - 1) / kShadowTileRows * kShadowTileRows;
 }
+// The int8 shadow keeps the same byte geometry: K-blocks of 128 int8 values (128 bytes, the same swizzle span),
+// 6 of them per row, so a 32-row K-block piece is still 4 KB.  Each 32-row tile has one fp32 scale st; the
+// shadow row is p8 with p - mu ~= st * p8 (element (row, col) at shadow8_index, in bytes).
+constexpr int kShadow8KBlock = 128;
+constexpr int kShadow8KBlocks = kD / kShadow8KBlock;   // 6
+__host__ __device__ __forceinline__ int64_t shadow8_index(int64_t row, int col) {
+  const int64_t tile = row / kShadowTileRows;
+  const int r = static_cast<int>(row % kShadowTileRows);
+  const int kb = col / kShadow8KBlock, c = col % kShadow8KBlock;
+  return ((tile * kShadow8KBlocks + kb) * kShadowTileRows + r) * kShadow8KBlock + c;
+}
+
+// Shadow formats of a shard (option "shadow"; 3 = AUTO picks 1 or 2 per shard at its first ingest).
+enum ShadowFormat { kShadowNone = 0, kShadowBf16 = 1, kShadowInt8 = 2, kShadowAuto = 3 };
 
 // ---------------------------------------------------------------------------------------------
 // Candidate records.  A candidate is one 64-bit word:

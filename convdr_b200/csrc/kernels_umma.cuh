@@ -25,6 +25,7 @@
 #pragma once
 #include <cuda.h>
 #include "common.cuh"
+#include "kernels_util.cuh"
 
 namespace b2f {
 
@@ -98,6 +99,8 @@ struct UmmaArgs {
   unsigned int* hist;         // [nq][kHistStride], initialised by pass_init_kernel / bootstrap_select_kernel
   const uint32_t* hkey0;      // [nq] key of the bootstrap's k-th best approximate score (0xffffffff: none yet)
   const int* hshift;          // [nq] log2(keys per bucket)
+  const float* qscale;        // int8 shadow: [nq] query scales sq (q16 then points at the int8 codes)
+  const float* tscale;        // int8 shadow: [row tiles of 32] tile scales st
 };
 
 // ------------------------------------------------------------------------------------------
@@ -220,6 +223,21 @@ __host__ __device__ __forceinline__ uint32_t umma_idesc_bf16(int m, int n) {
          (static_cast<uint32_t>(m >> 4) << 24);
 }
 
+// kind::i8: D = s32 (bits [4,6) = 2), A = B = signed 8-bit (bits [7,10), [10,13) = 1); the rest as for bf16.
+__host__ __device__ __forceinline__ uint32_t umma_idesc_i8(int m, int n) {
+  return (2u << 4) | (1u << 7) | (1u << 10) | (static_cast<uint32_t>(n >> 3) << 17) |
+         (static_cast<uint32_t>(m >> 4) << 24);
+}
+__device__ __forceinline__ void umma_i8_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc,
+                                            uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+
 constexpr uint64_t kHintEvictFirst = 0x12F0000000000000ull;
 constexpr uint64_t kHintEvictLast = 0x14F0000000000000ull;
 
@@ -230,6 +248,15 @@ __device__ __forceinline__ void umma_bf16_2sm_ts(uint32_t tmem_d, uint32_t tmem_
       "{\n\t.reg .pred p;\n\t"
       "setp.ne.b32 p, %4, 0;\n\t"
       "tcgen05.mma.cta_group::2.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+__device__ __forceinline__ void umma_i8_2sm_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc,
+                                               uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::i8 [%0], [%1], %2, %3, p;\n\t}"
       ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
@@ -313,6 +340,49 @@ __device__ __forceinline__ bool any_ge32(const uint32_t* v, float tau) {
   return r != 0u;
 }
 
+// The same chains on int32 accumulators against an integer threshold (int8 shadow, i8_threshold).
+__device__ __forceinline__ bool any_ge32_s32(const uint32_t* v, int tau) {
+  uint32_t r;
+  asm("{\n\t.reg .pred p, q;\n\t"
+      "setp.ge.s32 p, %1, %33;\n\t"
+      "setp.ge.s32 q, %2, %33;\n\t"
+      "setp.ge.or.s32 p, %3, %33, p;\n\t"
+      "setp.ge.or.s32 q, %4, %33, q;\n\t"
+      "setp.ge.or.s32 p, %5, %33, p;\n\t"
+      "setp.ge.or.s32 q, %6, %33, q;\n\t"
+      "setp.ge.or.s32 p, %7, %33, p;\n\t"
+      "setp.ge.or.s32 q, %8, %33, q;\n\t"
+      "setp.ge.or.s32 p, %9, %33, p;\n\t"
+      "setp.ge.or.s32 q, %10, %33, q;\n\t"
+      "setp.ge.or.s32 p, %11, %33, p;\n\t"
+      "setp.ge.or.s32 q, %12, %33, q;\n\t"
+      "setp.ge.or.s32 p, %13, %33, p;\n\t"
+      "setp.ge.or.s32 q, %14, %33, q;\n\t"
+      "setp.ge.or.s32 p, %15, %33, p;\n\t"
+      "setp.ge.or.s32 q, %16, %33, q;\n\t"
+      "setp.ge.or.s32 p, %17, %33, p;\n\t"
+      "setp.ge.or.s32 q, %18, %33, q;\n\t"
+      "setp.ge.or.s32 p, %19, %33, p;\n\t"
+      "setp.ge.or.s32 q, %20, %33, q;\n\t"
+      "setp.ge.or.s32 p, %21, %33, p;\n\t"
+      "setp.ge.or.s32 q, %22, %33, q;\n\t"
+      "setp.ge.or.s32 p, %23, %33, p;\n\t"
+      "setp.ge.or.s32 q, %24, %33, q;\n\t"
+      "setp.ge.or.s32 p, %25, %33, p;\n\t"
+      "setp.ge.or.s32 q, %26, %33, q;\n\t"
+      "setp.ge.or.s32 p, %27, %33, p;\n\t"
+      "setp.ge.or.s32 q, %28, %33, q;\n\t"
+      "setp.ge.or.s32 p, %29, %33, p;\n\t"
+      "setp.ge.or.s32 q, %30, %33, q;\n\t"
+      "setp.ge.or.s32 p, %31, %33, p;\n\t"
+      "setp.ge.or.s32 q, %32, %33, q;\n\t"
+      "or.pred p, p, q;\n\t"
+      "selp.u32 %0, 1, 0, p;\n\t}"
+      : "=r"(r)
+      : "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]), "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]), "r"(v[16]), "r"(v[17]), "r"(v[18]), "r"(v[19]), "r"(v[20]), "r"(v[21]), "r"(v[22]), "r"(v[23]), "r"(v[24]), "r"(v[25]), "r"(v[26]), "r"(v[27]), "r"(v[28]), "r"(v[29]), "r"(v[30]), "r"(v[31]), "r"(tau));
+  return r != 0u;
+}
+
 // ------------------------------------------------------------------------------------------
 // The kernel.  Grid = 2 * (number of CTA pairs), cluster (2,1,1), 384 threads:
 //   warp 0 lane 0 : TMA producer (both CTAs stream their own 32 rows of every tile)
@@ -325,21 +395,34 @@ __device__ __forceinline__ bool any_ge32(const uint32_t* v, float tau) {
 //                   instruction overhead in a warp that the scheduler cannot hide: two warps per TMEM lane
 //                   quarter halve it and overlap each other's latencies)
 //   warp 12       : refresher (in-kernel threshold tightening)
+// I8: int8 shadow and queries (kind::i8, s32 accumulators).  A 32-row tile is 6 K-blocks of 128 bytes, walked in 2
+// stages of 3 K-blocks (12 KB boxes, 18 of them in the ring); the queries take 192 TMEM columns (4 codes per
+// column, so a K-step of 32 codes is still 8 columns).  Each epilogue thread's 32 rows are one shadow tile: its
+// float threshold becomes ONE integer threshold per tile (i8_threshold), the compare chain stays one instruction
+// per score, and the float score is only formed for a hit.
 // ------------------------------------------------------------------------------------------
+template <bool I8>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
     umma_score_select_kernel(const __grid_constant__ CUtensorMap tmap_p, const UmmaArgs a) {
+  constexpr int NKB = I8 ? kShadow8KBlocks : kNumKBlocks;        // K-blocks of 128 bytes per row
+  constexpr int KBPS = I8 ? 3 : kKBlocksPerStage;                // K-blocks per ring stage
+  constexpr int STAGE_BYTES = KBPS * kSubTileBytes;
+  constexpr int STAGES_PER_TILE = NKB / KBPS;
+  constexpr int NST = I8 ? 18 : kNumStages;
+  constexpr int COLS_A = I8 ? kD / 4 : kTmemColsA;                // query columns in TMEM
+  static_assert(NST * STAGE_BYTES <= kNumStages * kStageBytes, "ring fits the bf16 layout's shared memory");
   extern __shared__ unsigned char umma_smem_raw[];
   const uint32_t raw = smem_u32(umma_smem_raw);
   const uint32_t base = (raw + 1023u) & ~1023u;  // 1024-byte alignment for the 128B swizzle atoms
   unsigned char* base_ptr = umma_smem_raw + (base - raw);
-  const uint32_t smem_b = base;                                   // [kNumStages][16 KB]
-  const uint32_t tail = smem_b + kNumStages * kStageBytes;
-  const uint32_t bar_full = tail;                                 // [kNumStages]
-  const uint32_t bar_empty = tail + 8 * kNumStages;               // [kNumStages]
-  const uint32_t bar_qready = tail + 16 * kNumStages;
+  const uint32_t smem_b = base;                                   // [NST][STAGE_BYTES]
+  const uint32_t tail = smem_b + NST * STAGE_BYTES;
+  const uint32_t bar_full = tail;                                 // [NST]
+  const uint32_t bar_empty = tail + 8 * NST;                      // [NST]
+  const uint32_t bar_qready = tail + 16 * NST;
   const uint32_t bar_tfull = bar_qready + 8;                      // [2]
   const uint32_t bar_tempty = bar_tfull + 16;                     // [2]
-  uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(base_ptr + kNumStages * kStageBytes + 16 * kNumStages + 40);
+  uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(base_ptr + NST * STAGE_BYTES + 16 * NST + 40);
   volatile int* epi_done_s = reinterpret_cast<volatile int*>(tmem_ptr_s + 1);     // epilogue warps that finished
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -351,7 +434,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
   if (warp == 0 && lane == 0) prefetch_tmap(&tmap_p);
   if (warp == 3 && lane == 0) *epi_done_s = 0;
   if (warp == 1 && lane == 0) {
-    for (int s = 0; s < kNumStages; ++s) {
+    for (int s = 0; s < NST; ++s) {
       mbar_init(bar_full + 8 * s, 2);   // leader's expect_tx arrive + peer's remote arrive
       mbar_init(bar_empty + 8 * s, 1);  // one multicast commit
     }
@@ -379,20 +462,20 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
     for (int tile = a.tile_begin + pair; tile < a.tile_end; tile += npairs) {
       // shadow layout (common.cuh): CTA tile = 2*tile + rank; kKBlocksPerStage consecutive K-blocks
       // of it are 128 consecutive 128-byte rows = one contiguous 16 KB box
-      const int row0 = (tile * 2 + static_cast<int>(cta_rank)) * kNumKBlocks * kTileRowsCta;
-      for (int st = 0; st < kStagesPerTile; ++st) {
+      const int row0 = (tile * 2 + static_cast<int>(cta_rank)) * NKB * kTileRowsCta;
+      for (int st = 0; st < STAGES_PER_TILE; ++st) {
         mbar_wait(bar_empty + 8 * stage, phase ^ 1u, a.err);
         const uint32_t full_leader = mapa_u32(bar_full + 8 * stage, 0);
-        if (leader) mbar_arrive_expect_tx(bar_full + 8 * stage, 2u * kStageBytes);
+        if (leader) mbar_arrive_expect_tx(bar_full + 8 * stage, 2u * STAGE_BYTES);
         else mbar_arrive_cluster(full_leader);
-        tma_load_2d_2sm(smem_b + stage * kStageBytes, &tmap_p, full_leader, 0,
-                        row0 + st * (kKBlocksPerStage * kTileRowsCta), kHintEvictFirst);
-        if (++stage == kNumStages) { stage = 0; phase ^= 1u; }
+        tma_load_2d_2sm(smem_b + stage * STAGE_BYTES, &tmap_p, full_leader, 0,
+                        row0 + st * (KBPS * kTileRowsCta), kHintEvictFirst);
+        if (++stage == NST) { stage = 0; phase ^= 1u; }
       }
     }
   } else if (warp == 1 && leader) {
     // ===================== MMA issuer (leader CTA; the whole warp waits, one elected lane issues) =====
-    const uint32_t idesc = umma_idesc_bf16(256, kTileRows);
+    const uint32_t idesc = I8 ? umma_idesc_i8(256, kTileRows) : umma_idesc_bf16(256, kTileRows);
     const bool elected = elect_one();
     mbar_wait(bar_qready, 0, a.err);   // both CTAs have their queries in TMEM
     tc_fence_after();
@@ -403,24 +486,25 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
       mbar_wait(bar_tempty + 8 * as, aph ^ 1u, a.err);   // epilogue has drained this accumulator stage
       tc_fence_after();
       const uint32_t tmem_d = tmem_base + kTmemColD + as * kTileRows;
-      for (int st = 0; st < kStagesPerTile; ++st) {
+      for (int st = 0; st < STAGES_PER_TILE; ++st) {
         mbar_wait(bar_full + 8 * stage, phase, a.err);
         tc_fence_after();
         if (elected) {
 #pragma unroll
-          for (int j = 0; j < kKBlocksPerStage; ++j) {
-            const uint64_t bdesc = umma_desc_sw128(smem_b + stage * kStageBytes + j * kSubTileBytes);
+          for (int j = 0; j < KBPS; ++j) {
+            const uint64_t bdesc = umma_desc_sw128(smem_b + stage * STAGE_BYTES + j * kSubTileBytes);
 #pragma unroll
-            for (int k = 0; k < kBlockK / 16; ++k) {   // UMMA K = 16 bf16: 8 TMEM columns of A, 32 bytes of B
-              const int kstep = (st * kKBlocksPerStage + j) * (kBlockK / 16) + k;
-              umma_bf16_2sm_ts(tmem_d, tmem_base + 8 * kstep, bdesc + 2 * k, idesc, kstep != 0);
+            for (int k = 0; k < 4; ++k) {   // UMMA K = 16 bf16 / 32 int8: 8 TMEM columns of A, 32 bytes of B
+              const int kstep = (st * KBPS + j) * 4 + k;
+              if (I8) umma_i8_2sm_ts(tmem_d, tmem_base + 8 * kstep, bdesc + 2 * k, idesc, kstep != 0);
+              else umma_bf16_2sm_ts(tmem_d, tmem_base + 8 * kstep, bdesc + 2 * k, idesc, kstep != 0);
             }
           }
-          umma_commit_pair(bar_empty + 8 * stage);                            // frees this smem stage in both CTAs
-          if (st == kStagesPerTile - 1) umma_commit_pair(bar_tfull + 8 * as); // accumulator ready
+          umma_commit_pair(bar_empty + 8 * stage);                             // frees this smem stage in both CTAs
+          if (st == STAGES_PER_TILE - 1) umma_commit_pair(bar_tfull + 8 * as); // accumulator ready
         }
         __syncwarp();
-        if (++stage == kNumStages) { stage = 0; phase ^= 1u; }
+        if (++stage == NST) { stage = 0; phase ^= 1u; }
       }
     }
   } else if (warp >= 4 && warp < 4 + kUmmaEpiWarps) {
@@ -431,14 +515,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
     const int q = static_cast<int>(cta_rank) * 128 + ew * 32 + lane;
     const bool q_ok = q < a.nq;
     {
-      const uint4* src = reinterpret_cast<const uint4*>(a.q16 + static_cast<int64_t>(q_ok ? q : 0) * kD);
+      const uint4* src = reinterpret_cast<const uint4*>(reinterpret_cast<const unsigned char*>(a.q16) +
+                                                        static_cast<int64_t>(q_ok ? q : 0) * kD * (I8 ? 1 : 2));
       // three 128-byte chunks (3 x 8 independent 16-byte loads) in flight per round: 4 L2 round trips
       // for the whole 1536-byte query row instead of 12
       constexpr int kQChunk = 3;
-      static_assert((kTmemColsA / 32) % kQChunk == 0, "query row = whole rounds");
+      static_assert((COLS_A / 32) % kQChunk == 0, "query row = whole rounds");
 #pragma unroll 1
-      static_assert((kTmemColsA / 64) % kQChunk == 0, "each of the two warps of a quarter loads whole rounds");
-      for (int c0 = half * (kTmemColsA / 64); c0 < (half + 1) * (kTmemColsA / 64); c0 += kQChunk) {   // 32 columns = 64 bf16 = 128 bytes per chunk
+      static_assert((COLS_A / 64) % kQChunk == 0, "each of the two warps of a quarter loads whole rounds");
+      for (int c0 = half * (COLS_A / 64); c0 < (half + 1) * (COLS_A / 64); c0 += kQChunk) {   // 32 columns = 128 bytes per chunk
         uint32_t w[kQChunk][32];
 #pragma unroll
         for (int u = 0; u < kQChunk; ++u)
@@ -476,6 +561,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
       }
     };
     const uint32_t tempty_leader = mapa_u32(bar_tempty, 0);
+    const float sq = I8 ? a.qscale[q_ok ? q : 0] : 0.f;
     int it = 0;
     for (int tile = a.tile_begin + pair; tile < a.tile_end; tile += npairs, ++it) {
       const uint32_t as = static_cast<uint32_t>(it) % kAccStages, aph = (static_cast<uint32_t>(it) / kAccStages) & 1u;
@@ -499,7 +585,59 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
       tmem_ld_wait();
       const int64_t row0 = static_cast<int64_t>(tile) * kTileRows + kHalfRows * half;
       const int n_valid = static_cast<int>(max(static_cast<int64_t>(0), min(static_cast<int64_t>(kHalfRows), a.n_rows - row0)));
-      if (a.dense) {
+      if constexpr (I8) {
+        // one integer threshold for this (query, shadow tile); scores as floats only where they are stored
+        const float st = n_valid > 0 ? __ldg(a.tscale + (row0 >> 5)) : 0.f;
+        if (a.dense) {
+          if (q_ok && n_mine + kHalfRows <= a.cap_p) {
+            uint64_t* dst = my_list + n_mine;
+#pragma unroll
+            for (int c = 0; c < kHalfRows; c += 2) {
+              ulonglong2 o;
+              o.x = (c < n_valid) ? pack_cand(i8_score(static_cast<int>(v[c]), sq, st), static_cast<uint32_t>(row0 + c)) : 0ull;
+              o.y = (c + 1 < n_valid) ? pack_cand(i8_score(static_cast<int>(v[c + 1]), sq, st), static_cast<uint32_t>(row0 + c + 1)) : 0ull;
+              *reinterpret_cast<ulonglong2*>(dst + c) = o;
+            }
+          }
+          n_mine += kHalfRows;
+        } else {
+          const int T = i8_threshold(tau, sq, st);
+          if (__any_sync(0xffffffffu, any_ge32_s32(v, T))) {
+            uint32_t m = 0;
+#pragma unroll
+            for (int c = 0; c < kHalfRows; ++c) m |= (static_cast<int>(v[c]) >= T) ? (1u << c) : 0u;
+            if (n_valid < kHalfRows) m &= (n_valid > 0) ? ((1u << n_valid) - 1u) : 0u;   // shard tail
+            uint32_t any = __reduce_or_sync(0xffffffffu, m);
+            if (__popc(any) > 6) {   // busy word: unrolled predicated stores, v[] stays in registers
+              if (m) {
+#pragma unroll
+                for (int c = 0; c < kHalfRows; ++c) {
+                  if ((m >> c) & 1u) {
+                    const uint32_t bits = __float_as_uint(i8_score(static_cast<int>(v[c]), sq, st));
+                    const int slot = n_mine + __popc(m & ((1u << c) - 1u));
+                    if (slot < a.cap_p) my_list[slot] = pack_cand(__uint_as_float(bits), static_cast<uint32_t>(row0 + c));
+                    count_hit(bits);
+                  }
+                }
+                n_mine += __popc(m);
+              }
+              any = 0;
+            }
+            while (any) {
+              const int c = __ffs(any) - 1;
+              any &= any - 1;
+              const uint32_t acc = tmem_ld_x1(col0 + c);
+              tmem_ld_wait();
+              if ((m >> c) & 1u) {
+                const uint32_t bits = __float_as_uint(i8_score(static_cast<int>(acc), sq, st));
+                if (n_mine < a.cap_p) my_list[n_mine] = pack_cand(__uint_as_float(bits), static_cast<uint32_t>(row0 + c));
+                ++n_mine;
+                count_hit(bits);
+              }
+            }
+          }
+        }
+      } else if (a.dense) {
         // bootstrap: every score of this half tile goes to the private area (zeros for rows past the end)
         if (q_ok && n_mine + kHalfRows <= a.cap_p) {
           uint64_t* dst = my_list + n_mine;

@@ -40,6 +40,8 @@ constexpr int kQsTailBytes = 4096;               // barriers, thresholds, counte
 constexpr int kQsSmemLimit = 232448;
 constexpr int kQsThreads = 416;                  // 4 service warps + 8 epilogue warps (two per TMEM lane quarter) + refresher
 constexpr int kQsEpiWarps = 8;
+constexpr int kQsEpiWarpsI8Scratch = 8 * 128 * 4;   // [8 epilogue warps][<= 128 query columns] int thresholds
+constexpr int kQsTailBytesI8 = kQsTailBytes + kQsEpiWarpsI8Scratch;   // int8 shadow: tail + that scratch
 constexpr int kQsRefresherWarp = 12;             // the highest warp id: the scheduler prefers it over the epilogue
                                                  // warps of its quarter, so thresholds never wait behind appends
 
@@ -72,6 +74,8 @@ struct UmmaQsArgs {
   int half_stage;             // 1: ring stages are 8 KB half K-blocks (64B swizzle), 2 MMAs per stage; 0: 16 KB, 4 MMAs
   int dense_quarters;         // first tile of a CTA: lane quarters [0, dense_quarters) pass unfiltered
   int first_wait_cycles;      // the other quarters wait this long at most for every threshold to exist (0: no wait)
+  const float* qscale;        // int8 shadow: [n_cols] query scales sq (0 for padded columns)
+  const float* tscale;        // int8 shadow: [row tiles of 32] tile scales st
 };
 
 struct QsPlan { int a_stages, q_stages, resident_kb, smem_bytes, half_stage; };
@@ -80,27 +84,30 @@ struct QsPlan { int a_stages, q_stages, resident_kb, smem_bytes, half_stage; };
 // half_stage_mode: 0 never, 1 = use 8 KB half stages (128 rows x 32 K-elements, 64B swizzle) when the queries are
 // fully resident and only <= 5 full 16 KB stages fit (161..176+ queries): 11 half stages keep 88 KB in flight
 // instead of 80 KB and recycle ring slots at twice the granularity.
-inline QsPlan umma_qs_plan(int n_cols, int resident_kb, int q_stages, int half_stage_mode = 0) {
+// n_kb: K-blocks of 128 bytes per row (12 for bf16, 6 for int8 rows and queries: half the query bytes, so the int8
+// layout keeps every query resident next to a 9-stage ring at 173 queries).
+inline QsPlan umma_qs_plan(int n_cols, int resident_kb, int q_stages, int half_stage_mode = 0, int n_kb = kNumKBlocks) {
   const int qkb = (n_cols / 2) * 128;
   if (resident_kb < 0) resident_kb = 0;
-  if (resident_kb > kNumKBlocks) resident_kb = kNumKBlocks;
+  if (resident_kb > n_kb) resident_kb = n_kb;
   if (q_stages < 2) q_stages = 2;
   if (q_stages > kQsMaxQStages) q_stages = kQsMaxQStages;
+  const int tail_bytes = n_kb == kNumKBlocks ? kQsTailBytes : kQsTailBytesI8;
   QsPlan p;
   for (;;) {
-    const int qs = resident_kb == kNumKBlocks ? 0 : q_stages;
-    const int avail = kQsSmemLimit - 1024 - kQsTailBytes - (resident_kb + qs) * qkb;
+    const int qs = resident_kb == n_kb ? 0 : q_stages;
+    const int avail = kQsSmemLimit - 1024 - tail_bytes - (resident_kb + qs) * qkb;
     int a = avail / kQsStageBytes;
     if (a > kQsMaxAStages) a = kQsMaxAStages;
     if (a >= 4 || resident_kb == 0) {
       p.a_stages = a; p.q_stages = qs; p.resident_kb = resident_kb; p.half_stage = 0;
-      if (half_stage_mode && resident_kb == kNumKBlocks && a <= 5) {
+      if (half_stage_mode && resident_kb == n_kb && a <= 5) {
         int ah = avail / (kQsStageBytes / 2);
         if (ah > kQsMaxAStages) ah = kQsMaxAStages;
         if (ah * (kQsStageBytes / 2) > a * kQsStageBytes) { p.half_stage = 1; p.a_stages = ah; }
       }
       p.smem_bytes = (resident_kb + qs) * qkb + (p.half_stage ? p.a_stages * (kQsStageBytes / 2) : a * kQsStageBytes) +
-                     kQsTailBytes + 1024;
+                     tail_bytes + 1024;
       return p;
     }
     --resident_kb;   // too many resident K-blocks for this batch size: stream more of them
@@ -155,6 +162,35 @@ __device__ __forceinline__ bool any_ge16(const uint32_t (&v)[16], const float (&
   return r != 0u;
 }
 
+// The same chain on the int32 accumulators of the int8 engine against integer thresholds (i8_threshold).
+__device__ __forceinline__ bool any_ge16_s32(const uint32_t (&v)[16], const int (&t)[16]) {
+  uint32_t r;
+  asm("{\n\t.reg .pred p;\n\t"
+      "setp.ge.s32 p, %1, %17;\n\t"
+      "setp.ge.or.s32 p, %2, %18, p;\n\t"
+      "setp.ge.or.s32 p, %3, %19, p;\n\t"
+      "setp.ge.or.s32 p, %4, %20, p;\n\t"
+      "setp.ge.or.s32 p, %5, %21, p;\n\t"
+      "setp.ge.or.s32 p, %6, %22, p;\n\t"
+      "setp.ge.or.s32 p, %7, %23, p;\n\t"
+      "setp.ge.or.s32 p, %8, %24, p;\n\t"
+      "setp.ge.or.s32 p, %9, %25, p;\n\t"
+      "setp.ge.or.s32 p, %10, %26, p;\n\t"
+      "setp.ge.or.s32 p, %11, %27, p;\n\t"
+      "setp.ge.or.s32 p, %12, %28, p;\n\t"
+      "setp.ge.or.s32 p, %13, %29, p;\n\t"
+      "setp.ge.or.s32 p, %14, %30, p;\n\t"
+      "setp.ge.or.s32 p, %15, %31, p;\n\t"
+      "setp.ge.or.s32 p, %16, %32, p;\n\t"
+      "selp.u32 %0, 1, 0, p;\n\t}"
+      : "=r"(r)
+      : "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]),
+        "r"(v[8]), "r"(v[9]), "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]),
+        "r"(t[0]), "r"(t[1]), "r"(t[2]), "r"(t[3]), "r"(t[4]), "r"(t[5]), "r"(t[6]), "r"(t[7]),
+        "r"(t[8]), "r"(t[9]), "r"(t[10]), "r"(t[11]), "r"(t[12]), "r"(t[13]), "r"(t[14]), "r"(t[15]));
+  return r != 0u;
+}
+
 // ------------------------------------------------------------------------------------------
 // Grid = 2 * (number of CTA pairs), cluster (2,1,1), 384 threads:
 //   warp 0 lane 0 : passage producer (TMA; both CTAs stream their own 128 rows of every tile)
@@ -165,7 +201,13 @@ __device__ __forceinline__ bool any_ge16(const uint32_t (&v)[16], const float (&
 //                   quarter take alternate 16-query chunks of the row
 //   warp 12       : refresher — raises the global thresholds from the hit histogram and refreshes the
 //                   CTA's shared-memory copy of all thresholds
+// I8: int8 shadow and queries (kind::i8, s32 accumulators, 6 K-blocks of 128 bytes; the byte geometry of every
+// stage, box and K-step is the bf16 one).  The epilogue compares the raw int32 accumulators with integer
+// thresholds: once per tile the warp's lanes convert the float thresholds of its query columns for the tile scale
+// (one 32-row shadow tile per warp) into a per-warp shared-memory scratch, which every lane reads per 16-query
+// chunk with 4 LDS.128 — the same cost as the float thresholds of the bf16 path.
 // ------------------------------------------------------------------------------------------
+template <bool I8>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
     umma_qs_score_select_kernel(const __grid_constant__ CUtensorMap tmap_p,
                                 const __grid_constant__ CUtensorMap tmap_ph /* 32-column boxes, 64B swizzle */,
@@ -201,6 +243,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
   int* cnt_s = reinterpret_cast<int*>(tail_ptr + 512 + 1024);            // [kQsMaxCols]
   uint32_t* hkey0_s = reinterpret_cast<uint32_t*>(tail_ptr + 512 + 2048);  // [kQsMaxCols]
   const uint32_t tau_s_addr = tail + 512;
+  int* thr_s = reinterpret_cast<int*>(tail_ptr + kQsTailBytes);          // int8: [kQsEpiWarps][128] integer thresholds
+  constexpr int NKB = I8 ? kShadow8KBlocks : kNumKBlocks;                 // K-blocks of 128 bytes per row
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t cta_rank = cluster_ctarank();
@@ -255,7 +299,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
       // shadow layout (common.cuh): this CTA's 128 rows are 4 consecutive 32-row tiles; K-block kb of
       // each is a contiguous 4 KB piece -> 4 TMA boxes per 16 KB stage (rows past the end: zero fill)
       const int t32 = (tile * 2 + static_cast<int>(cta_rank)) * (kQsTileRowsCta / kShadowTileRows);
-      for (int kb = 0; kb < kNumKBlocks; ++kb) {
+      for (int kb = 0; kb < NKB; ++kb) {
         for (int h = 0; h < n_sub; ++h) {
           mbar_wait(bar_aempty + 8 * stage, phase ^ 1u, a.err);
           const uint32_t full_leader = mapa_u32(bar_afull + 8 * stage, 0);
@@ -265,12 +309,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
 #pragma unroll
             for (int j = 0; j < kQsTileRowsCta / kShadowTileRows; ++j)
               tma_load_2d_2sm(smem_a + stage * a_stage_bytes + j * (kShadowTileRows * 64), &tmap_ph, full_leader, 32 * h,
-                              ((t32 + j) * kNumKBlocks + kb) * kShadowTileRows, kHintEvictFirst);
+                              ((t32 + j) * NKB + kb) * kShadowTileRows, kHintEvictFirst);
           } else {
 #pragma unroll
             for (int j = 0; j < kQsTileRowsCta / kShadowTileRows; ++j)
               tma_load_2d_2sm(smem_a + stage * a_stage_bytes + j * (kShadowTileRows * 128), &tmap_p, full_leader, 0,
-                              ((t32 + j) * kNumKBlocks + kb) * kShadowTileRows, kHintEvictFirst);
+                              ((t32 + j) * NKB + kb) * kShadowTileRows, kHintEvictFirst);
           }
           if (++stage == static_cast<uint32_t>(a.a_stages)) { stage = 0; phase ^= 1u; }
         }
@@ -286,10 +330,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
         tma_load_2d_2sm(smem_qres + kb * qkb_bytes, &tmap_q, qres_leader, kb * kBlockK,
                         static_cast<int>(cta_rank) * n_half, kHintEvictLast);
     }
-    if (R < kNumKBlocks) {
+    if (R < NKB) {
       uint32_t stage = 0, phase = 0;
       for (int tile = a.tile_begin + pair; tile < a.tile_end; tile += npairs) {
-        for (int kb = R; kb < kNumKBlocks; ++kb) {
+        for (int kb = R; kb < NKB; ++kb) {
           mbar_wait(bar_qempty + 8 * stage, phase ^ 1u, a.err);
           const uint32_t full_leader = mapa_u32(bar_qfull + 8 * stage, 0);
           if (leader) mbar_arrive_expect_tx(bar_qfull + 8 * stage, 2u * qkb_bytes);
@@ -308,7 +352,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
     // of the same unit.  This warp uses the LSU path instead: one `prefetch.global.L2` per 128-byte line of
     // the CTA's tile `prefetch` rounds ahead (a tile is ONE contiguous 192 KB region of the shadow: 4
     // consecutive 32-row tiles x 12 K-blocks x 4 KB), paced by the producer's progress mark.
-    constexpr int64_t kTileBytesCta = static_cast<int64_t>(kQsTileRowsCta) * kD * 2;     // 196,608
+    constexpr int64_t kTileBytesCta = static_cast<int64_t>(kQsTileRowsCta) * kD * (I8 ? 1 : 2);     // 196,608 (bf16)
     int it_pf = 0;
     for (int tile = a.tile_begin + pair; tile < a.tile_end; tile += npairs, ++it_pf) {
       while (it_pf > *prod_it_s + a.prefetch) __nanosleep(400);
@@ -321,7 +365,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
     }
   } else if (warp == 1 && leader) {
     // ===================== MMA issuer (leader CTA; the whole warp waits, one elected lane issues) =====
-    const uint32_t idesc = umma_idesc_bf16(256, a.n_cols);
+    const uint32_t idesc = I8 ? umma_idesc_i8(256, a.n_cols) : umma_idesc_bf16(256, a.n_cols);
     const bool elected = elect_one();
     if (R > 0) {
       mbar_wait(bar_qres, 0, a.err);
@@ -334,7 +378,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
       mbar_wait(bar_tempty + 8 * as, aph ^ 1u, a.err);   // epilogue has drained this accumulator
       tc_fence_after();
       const uint32_t tmem_d = tmem_base + as * kQsAccStride;
-      for (int kb = 0; kb < kNumKBlocks; ++kb) {
+      for (int kb = 0; kb < NKB; ++kb) {
         const bool streamed = kb >= R;
         if (streamed) mbar_wait(bar_qfull + 8 * sq, pq, a.err);
         for (int h = 0; h < n_sub; ++h) {
@@ -344,15 +388,16 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
             const uint32_t a_addr = smem_a + sa * a_stage_bytes;
             const uint64_t adesc = a.half_stage ? umma_desc_sw64(a_addr) : umma_desc_sw128(a_addr);
             const uint64_t bdesc = umma_desc_sw128(streamed ? smem_qring + sq * qkb_bytes : smem_qres + kb * qkb_bytes);
-            const int k_steps = a.half_stage ? 2 : 4;     // UMMA K = 16 bf16 = 32 bytes = 2 descriptor units
+            const int k_steps = a.half_stage ? 2 : 4;     // UMMA K = 16 bf16 / 32 int8 = 32 bytes = 2 descriptor units
             for (int k = 0; k < k_steps; ++k) {
               const int kq = a.half_stage ? 2 * h + k : k;   // position of this K-step inside the query K-block
-              umma_bf16_2sm(tmem_d, adesc + 2 * k, bdesc + 2 * kq, idesc, (kb | h | k) != 0);
+              if (I8) umma_i8_2sm(tmem_d, adesc + 2 * k, bdesc + 2 * kq, idesc, (kb | h | k) != 0);
+              else umma_bf16_2sm(tmem_d, adesc + 2 * k, bdesc + 2 * kq, idesc, (kb | h | k) != 0);
             }
             umma_commit_pair(bar_aempty + 8 * sa);                 // frees the passage stage in both CTAs
             if (h == n_sub - 1) {
               if (streamed) umma_commit_pair(bar_qempty + 8 * sq);   // and the query stage
-              if (kb == kNumKBlocks - 1) umma_commit_pair(bar_tfull + 8 * as);  // accumulator ready
+              if (kb == NKB - 1) umma_commit_pair(bar_tfull + 8 * as);  // accumulator ready
             }
           }
           __syncwarp();
@@ -411,9 +456,56 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
       const bool row_ok = row64 < a.n_rows;
       const uint32_t row = static_cast<uint32_t>(row64);
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(ew * 32) << 16) + as * kQsAccStride;
+      // int8: this warp's 32 rows are one shadow tile with one scale
+      const float st = (I8 && row64 - lane < a.n_rows) ? __ldg(a.tscale + ((row64 - lane) >> 5)) : 0.f;
+      int* thr_w = thr_s + (warp - 4) * 128;
+      if constexpr (I8) {
+        // this warp's query columns: 16 * half + 32 * i + j (i-th chunk, j < 16); thresholds only rise, so converting
+        // them once per tile (a snapshot) keeps every filter valid
+        const int n_own = 16 * ((a.n_cols - 16 * half + 31) / 32);
+        for (int x = lane; x < n_own; x += 32) {
+          const int col = 16 * half + 32 * (x >> 4) + (x & 15);
+          thr_w[x] = i8_threshold(*reinterpret_cast<volatile float*>(tau_s + col), __ldg(a.qscale + col), st);
+        }
+        __syncwarp();
+      }
       for (int c0 = 16 * half; c0 < a.n_cols; c0 += 32) {
         uint32_t v[16];
         tmem_ld_x16(taddr + c0, v);
+        if constexpr (I8) {
+          const int* thr = thr_w + 16 * ((c0 - 16 * half) >> 5);
+          int t[16];
+#pragma unroll
+          for (int u = 0; u < 4; ++u) {
+            const int4 f = *reinterpret_cast<const int4*>(thr + 4 * u);
+            t[4 * u] = f.x; t[4 * u + 1] = f.y; t[4 * u + 2] = f.z; t[4 * u + 3] = f.w;
+          }
+          tmem_ld_wait();
+          const bool mine = row_ok && any_ge16_s32(v, t);
+          if (__any_sync(0xffffffffu, mine)) {
+            uint32_t m = 0;
+#pragma unroll
+            for (int j = 0; j < 16; ++j) m |= (static_cast<int>(v[j]) >= t[j]) ? (1u << j) : 0u;
+            if (!row_ok) m = 0;
+            uint32_t any = __reduce_or_sync(0xffffffffu, m);
+            if (__popc(any) > 4) {
+              // busy chunk (loose thresholds early in a pass): unrolled, v[] stays in registers
+#pragma unroll
+              for (int j = 0; j < 16; ++j)
+                if ((any >> j) & 1u)
+                  hit(c0 + j, (m >> j) & 1u, __float_as_uint(i8_score(static_cast<int>(v[j]), __ldg(a.qscale + c0 + j), st)), row);
+              any = 0;
+            }
+            while (any) {   // the recorded score is formed on this rare path only
+              const int j = __ffs(any) - 1;
+              any &= any - 1;
+              const uint32_t acc = tmem_ld_x1(taddr + c0 + j);
+              tmem_ld_wait();
+              hit(c0 + j, (m >> j) & 1u, __float_as_uint(i8_score(static_cast<int>(acc), __ldg(a.qscale + c0 + j), st)), row);
+            }
+          }
+          continue;
+        }
         // thresholds of these 16 queries (volatile: the refresher warp rewrites them while we run)
         float t[16];
 #pragma unroll

@@ -1,5 +1,6 @@
 // kernels_util.cuh — ingest-side kernels: bf16 shadow + norm bound, synthetic rows, query prep.
 #pragma once
+#include <climits>
 #include "common.cuh"
 
 namespace b2f {
@@ -103,6 +104,148 @@ __global__ void __launch_bounds__(256) convert_rows_kernel(const float* __restri
   if (lane == 0 && cmax > 0.f) atomicMax(maxnorm2_bits + 2, __float_as_uint(cmax));
 }
 
+// Symmetric int8 code of v for the scale 1/inv (inv = 127 / max|v| over the scale's group; 0 for an all-zero group).
+__device__ __forceinline__ int quant8(float v, float inv) {
+  return max(-127, min(127, __float2int_rn(v * inv)));
+}
+
+// int8 shadow (DESIGN.md section 4): one warp per 32-row tile of rows [tile_row0, row0 + n_rows), where tile_row0 is
+// row0 rounded down to the tile — a tile that an earlier add left partly filled is re-quantised with the scale of
+// all its rows.  Pass 1: st = max|d| / 127 over the tile (d = fl32(x - mu)); pass 2: p8 = rint(d / st), the
+// K-block-major int8 row (common.cuh shadow8_index) and the same three bounds as convert_rows_kernel, with slot [1]
+// an upper bound of max ||(x - mu) - st * p8||^2: fma(-st, p8, d) rounds the exact difference once (relative 2^-24,
+// covered by norm2_upper), plus 2^-24 ||d|| for the rounding of the fp32 subtraction.  Any p8 is valid — the bound
+// measures the error that was made.  x8 == nullptr: bounds only (used by the format choice).
+__global__ void __launch_bounds__(256) convert_rows_i8_kernel(const float* __restrict__ x32, int8_t* __restrict__ x8,
+                                                              float* __restrict__ tscale, int64_t row0, int64_t n_rows,
+                                                              unsigned int* __restrict__ maxnorm2_bits,
+                                                              const float* __restrict__ mu) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+  const int64_t nwarps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
+  const int64_t end = row0 + n_rows;
+  const int64_t t_begin = row0 / kShadowTileRows, t_end = (end + kShadowTileRows - 1) / kShadowTileRows;
+  float4 m4[kF4PerLane];
+#pragma unroll
+  for (int i = 0; i < kF4PerLane; ++i) m4[i] = __ldg(reinterpret_cast<const float4*>(mu) + lane + 32 * i);
+  float wmax = 0.f, emax = 0.f, cmax = 0.f;
+  for (int64_t t = t_begin + warp; t < t_end; t += nwarps) {
+    const int64_t r0 = t * kShadowTileRows, r1 = min(end, r0 + kShadowTileRows);
+    float amax = 0.f;
+    for (int64_t r = r0; r < r1; ++r) {
+      const float4* src = reinterpret_cast<const float4*>(x32 + r * kD);
+#pragma unroll
+      for (int i = 0; i < kF4PerLane; ++i) {
+        const float4 v = __ldg(src + lane + 32 * i);
+        amax = fmaxf(amax, fmaxf(fmaxf(fabsf(__fsub_rn(v.x, m4[i].x)), fabsf(__fsub_rn(v.y, m4[i].y))),
+                                 fmaxf(fabsf(__fsub_rn(v.z, m4[i].z)), fabsf(__fsub_rn(v.w, m4[i].w)))));
+      }
+    }
+#pragma unroll
+    for (int s = 16; s >= 1; s >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, s));
+    const float st = amax / 127.f;
+    const float inv = amax > 0.f ? 127.f / amax : 0.f;
+    if (x8 && lane == 0) tscale[t] = st;
+    for (int64_t r = r0; r < r1; ++r) {
+      const float4* src = reinterpret_cast<const float4*>(x32 + r * kD);
+      float ss = 0.f, es = 0.f, cs = 0.f;
+#pragma unroll
+      for (int i = 0; i < kF4PerLane; ++i) {
+        const float4 v = __ldg(src + lane + 32 * i);
+        ss += v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w;
+        float4 d;
+        d.x = __fsub_rn(v.x, m4[i].x); d.y = __fsub_rn(v.y, m4[i].y); d.z = __fsub_rn(v.z, m4[i].z); d.w = __fsub_rn(v.w, m4[i].w);
+        cs += d.x * d.x + d.y * d.y + d.z * d.z + d.w * d.w;
+        const int a = quant8(d.x, inv), b = quant8(d.y, inv), c = quant8(d.z, inv), e = quant8(d.w, inv);
+        const float ex = fmaf(-st, static_cast<float>(a), d.x), ey = fmaf(-st, static_cast<float>(b), d.y);
+        const float ez = fmaf(-st, static_cast<float>(c), d.z), ew = fmaf(-st, static_cast<float>(e), d.w);
+        es += ex * ex + ey * ey + ez * ez + ew * ew;
+        if (x8) {
+          const uint32_t packed = (static_cast<uint32_t>(a) & 0xffu) | ((static_cast<uint32_t>(b) & 0xffu) << 8) |
+                                  ((static_cast<uint32_t>(c) & 0xffu) << 16) | (static_cast<uint32_t>(e) << 24);
+          *reinterpret_cast<uint32_t*>(x8 + shadow8_index(r, 4 * (lane + 32 * i))) = packed;
+        }
+      }
+#pragma unroll
+      for (int s = 16; s >= 1; s >>= 1) {
+        ss += __shfl_xor_sync(0xffffffffu, ss, s);
+        es += __shfl_xor_sync(0xffffffffu, es, s);
+        cs += __shfl_xor_sync(0xffffffffu, cs, s);
+      }
+      const float cn = __fsqrt_ru(norm2_upper(cs));
+      const float e = __fadd_ru(__fsqrt_ru(norm2_upper(es)), __fmul_ru(cn, 6.0e-8f));
+      wmax = fmaxf(wmax, norm2_upper(ss));
+      emax = fmaxf(emax, __fmul_ru(e, e));
+      cmax = fmaxf(cmax, __fmul_ru(__fmul_ru(cn, cn), 1.0000002f));
+    }
+  }
+  if (lane == 0 && wmax > 0.f) atomicMax(maxnorm2_bits, __float_as_uint(wmax));
+  if (lane == 0 && emax > 0.f) atomicMax(maxnorm2_bits + 1, __float_as_uint(emax));
+  if (lane == 0 && cmax > 0.f) atomicMax(maxnorm2_bits + 2, __float_as_uint(cmax));
+}
+
+// Format choice (AUTO): 64 of the first m rows act as pseudo-queries q_j (uncentred, like real queries).  For every
+// j this kernel accumulates, over `n_s` evenly spaced sample rows, the sum and the sum of squares of the centred
+// scores q_j . (p - mu) in fp64 (stat[2j], stat[2j+1]) and writes ||q_j|| and ||q_j - sq q8_j|| (qstat[2j], +1).
+// One warp per (j, sample row); blocks of 8 warps share j.
+__global__ void __launch_bounds__(256) shadow_probe_kernel(const float* __restrict__ x32, int64_t m, int n_s,
+                                                           const float* __restrict__ mu, double* __restrict__ stat,
+                                                           float* __restrict__ qstat) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int j = blockIdx.y;
+  const float4* q4 = reinterpret_cast<const float4*>(x32 + (m * j / 64) * kD);
+  float4 q[kF4PerLane];
+  float amax = 0.f, qq = 0.f;
+#pragma unroll
+  for (int i = 0; i < kF4PerLane; ++i) {
+    q[i] = __ldg(q4 + lane + 32 * i);
+    amax = fmaxf(amax, fmaxf(fmaxf(fabsf(q[i].x), fabsf(q[i].y)), fmaxf(fabsf(q[i].z), fabsf(q[i].w))));
+    qq += q[i].x * q[i].x + q[i].y * q[i].y + q[i].z * q[i].z + q[i].w * q[i].w;
+  }
+  double s1 = 0.0, s2 = 0.0;
+  for (int r = blockIdx.x * 8 + w; r < n_s; r += gridDim.x * 8) {
+    const float4* p4 = reinterpret_cast<const float4*>(x32 + (m * r / n_s) * kD);
+    const float4* m4 = reinterpret_cast<const float4*>(mu);
+    float acc = 0.f;
+#pragma unroll
+    for (int i = 0; i < kF4PerLane; ++i) {
+      const float4 p = __ldg(p4 + lane + 32 * i), c = __ldg(m4 + lane + 32 * i);
+      acc += q[i].x * (p.x - c.x) + q[i].y * (p.y - c.y) + q[i].z * (p.z - c.z) + q[i].w * (p.w - c.w);
+    }
+#pragma unroll
+    for (int s = 16; s >= 1; s >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, s);
+    s1 += acc;
+    s2 += static_cast<double>(acc) * acc;
+  }
+  if (lane == 0) {
+    atomicAdd(stat + 2 * j, s1);
+    atomicAdd(stat + 2 * j + 1, s2);
+  }
+  if (blockIdx.x == 0 && w == 0) {
+#pragma unroll
+    for (int s = 16; s >= 1; s >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, s));
+    const float sq = amax / 127.f, inv = amax > 0.f ? 127.f / amax : 0.f;
+    float es = 0.f;
+#pragma unroll
+    for (int i = 0; i < kF4PerLane; ++i) {
+      const float ex = fmaf(-sq, static_cast<float>(quant8(q[i].x, inv)), q[i].x);
+      const float ey = fmaf(-sq, static_cast<float>(quant8(q[i].y, inv)), q[i].y);
+      const float ez = fmaf(-sq, static_cast<float>(quant8(q[i].z, inv)), q[i].z);
+      const float ew = fmaf(-sq, static_cast<float>(quant8(q[i].w, inv)), q[i].w);
+      es += ex * ex + ey * ey + ez * ez + ew * ew;
+    }
+#pragma unroll
+    for (int s = 16; s >= 1; s >>= 1) {
+      es += __shfl_xor_sync(0xffffffffu, es, s);
+      qq += __shfl_xor_sync(0xffffffffu, qq, s);
+    }
+    if (lane == 0) {
+      qstat[2 * j] = __fsqrt_ru(norm2_upper(qq));
+      qstat[2 * j + 1] = __fsqrt_ru(norm2_upper(es));
+    }
+  }
+}
+
 // Synthetic rows (see include/b2f.h b2f_add_synthetic).  One warp per row; lane l produces
 // float4 chunks l, l+32, ..., l+160; chunk c of row r is Philox4x32-10(counter = (r_lo, r_hi, c, 0),
 // key = (seed_lo ^ stream_lo, seed_hi ^ stream_hi ^ 0x5eed)).  With mean_shift = M > 0 every component t
@@ -204,6 +347,73 @@ __global__ void __launch_bounds__(128) prep_queries_kernel(const float* __restri
     qnorm[q] = __fsqrt_ru(norm2_upper(ss));
     qerr[q] = __fsqrt_ru(norm2_upper(es));
   }
+}
+
+// Query preparation for an int8 shadow: per query the scale sq = max|q| / 127, the row-major int8 code q8
+// (zero rows and sq = 0 for q >= nq), an upper bound of ||q|| and one of ||q - sq q8||.
+__global__ void __launch_bounds__(128) prep_queries_i8_kernel(const float* __restrict__ q32, int nq, int nq_pad,
+                                                              int8_t* __restrict__ q8, float* __restrict__ qscale,
+                                                              float* __restrict__ qnorm, float* __restrict__ qerr) {
+  const int lane = threadIdx.x & 31;
+  const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (q >= nq_pad) return;
+  uint32_t* dst = reinterpret_cast<uint32_t*>(q8 + static_cast<int64_t>(q) * kD);
+  if (q >= nq) {
+#pragma unroll
+    for (int i = 0; i < kF4PerLane; ++i) dst[lane + 32 * i] = 0u;
+    if (lane == 0) qscale[q] = 0.f;
+    return;
+  }
+  const float4* src = reinterpret_cast<const float4*>(q32 + static_cast<int64_t>(q) * kD);
+  float4 v[kF4PerLane];
+  float amax = 0.f, ss = 0.f, es = 0.f;
+#pragma unroll
+  for (int i = 0; i < kF4PerLane; ++i) {
+    v[i] = __ldg(src + lane + 32 * i);
+    amax = fmaxf(amax, fmaxf(fmaxf(fabsf(v[i].x), fabsf(v[i].y)), fmaxf(fabsf(v[i].z), fabsf(v[i].w))));
+    ss += v[i].x * v[i].x + v[i].y * v[i].y + v[i].z * v[i].z + v[i].w * v[i].w;
+  }
+#pragma unroll
+  for (int s = 16; s >= 1; s >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, s));
+  const float sq = amax / 127.f, inv = amax > 0.f ? 127.f / amax : 0.f;
+#pragma unroll
+  for (int i = 0; i < kF4PerLane; ++i) {
+    const int a = quant8(v[i].x, inv), b = quant8(v[i].y, inv), c = quant8(v[i].z, inv), e = quant8(v[i].w, inv);
+    const float ex = fmaf(-sq, static_cast<float>(a), v[i].x), ey = fmaf(-sq, static_cast<float>(b), v[i].y);
+    const float ez = fmaf(-sq, static_cast<float>(c), v[i].z), ew = fmaf(-sq, static_cast<float>(e), v[i].w);
+    es += ex * ex + ey * ey + ez * ez + ew * ew;
+    dst[lane + 32 * i] = (static_cast<uint32_t>(a) & 0xffu) | ((static_cast<uint32_t>(b) & 0xffu) << 8) |
+                         ((static_cast<uint32_t>(c) & 0xffu) << 16) | (static_cast<uint32_t>(e) << 24);
+  }
+#pragma unroll
+  for (int s = 16; s >= 1; s >>= 1) {
+    ss += __shfl_xor_sync(0xffffffffu, ss, s);
+    es += __shfl_xor_sync(0xffffffffu, es, s);
+  }
+  if (lane == 0) {
+    qscale[q] = sq;
+    qnorm[q] = __fsqrt_ru(norm2_upper(ss));
+    qerr[q] = __fsqrt_ru(norm2_upper(es));
+  }
+}
+
+// Integer threshold of the int8 tensor engine.  A prefilter score is s~ = acc * c with acc the exact int32 dot
+// product of the codes and c = sq * st (real product of the query and tile scales).  Returns T with
+// "acc * c >= tau  =>  acc >= T" for every integer acc: T = floor of a value <= tau / c (c rounded towards the side
+// that makes the quotient smaller for the sign of tau, the division rounded down); -inf and NaN pass everything.
+__device__ __forceinline__ int i8_threshold(float tau, float sq, float st) {
+  if (!(tau > -INFINITY)) return INT_MIN;
+  const float c = tau >= 0.f ? __fmul_ru(sq, st) : __fmul_rd(sq, st);
+  if (c == 0.f) return tau > 0.f ? INT_MAX : INT_MIN;   // tau > 0: c is exactly 0, every score is 0 < tau
+  const float x = __fdiv_rd(tau, c);
+  if (x >= 2147483520.f) return INT_MAX;
+  if (x < -2147483520.f) return INT_MIN;
+  return static_cast<int>(floorf(x));
+}
+// The score recorded for a hit: fl(fl(acc) * fl(sq * st)); |acc| <= 768 * 127^2 < 2^24, so fl(acc) is exact and the
+// recorded value is within 2^-23 |s~| of s~ (covered by the relative term of the int8 margin, pass_init_kernel).
+__device__ __forceinline__ float i8_score(int acc, float sq, float st) {
+  return __fmul_rn(static_cast<float>(acc), __fmul_rn(sq, st));
 }
 
 }  // namespace b2f

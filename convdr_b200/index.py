@@ -254,6 +254,8 @@ class FlatIPIndex:
 
     # -- knobs / introspection --------------------------------------------------------------------
     def set_option(self, key: str, value) -> None:
+        """Engine knob (include/b2f.h b2f_set_option), e.g. "shadow": 0 none, 1 bf16, 2 int8, 3 AUTO (default:
+        int8 or bf16 per shard, chosen from its first rows; stat "shadow_format" tells which)."""
         if key == "path" and isinstance(value, str):
             value = PATHS[value]
         self._options[key] = int(value)

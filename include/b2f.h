@@ -213,8 +213,11 @@ int b2f_num_shards(const b2f_index* idx);
 void* b2f_stream(b2f_index* idx, int shard);
 
 /* Tuning knobs:
- *   "path" (B2F_PATH_*; AUTO = the tensor engine whenever the bf16 shadow exists),
- *   "shadow" (keep the bf16 copy, default 1), "keep_on_reset" (default 1),
+ *   "path" (B2F_PATH_*; AUTO = the tensor engine whenever a shadow exists),
+ *   "shadow" (the prefilter copy the tensor engine streams: 0 none, 1 bf16, 2 int8 with one scale per
+ *       32-row tile (half the bytes per row, a ~4x wider error margin), 3 AUTO (default): int8 when the
+ *       first rows of a shard leave the int8 margin narrow against the spread of the scores, bf16
+ *       otherwise; results never depend on it; empty index only), "keep_on_reset" (default 1),
  *   "scan_max_auto" (largest batch AUTO sends to the SIMT scan, default 0 = never),
  *   "center" (default 1: the shadow holds rows minus the mean of the first rows added, so the error
  *       margin follows ||p - mean|| instead of ||p||; empty index only),
@@ -245,7 +248,8 @@ int b2f_set_option(b2f_index* idx, const char* key, int64_t value);
  * area was too small), "overflow_survivors" (more rows within the error margin of the k-th score
  * than the survivor buffer holds); "path", "passes", "qs_passes"; with "profile" on also "score_ms",
  * "score_launches", "score_rows" (scoring kernels: device time, launches, rows
- * streamed) and "select_ms" (refresh + final kernels).                         */
+ * streamed) and "select_ms" (refresh + final kernels); "shadow_format" (first shard: 0 none,
+ * 1 bf16, 2 int8) and "shadow_rho" (AUTO: median 2 eps8 / sigma of the probe, 0 if not measured). */
 int b2f_get_stat(const b2f_index* idx, const char* key, double* out);
 
 void b2f_destroy(b2f_index* idx);
