@@ -26,6 +26,15 @@ SYMBOLS = {
     "b2f_search_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
     "b2f_search_device_async": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
     "b2f_search_finish": (C.c_int, [C.c_void_p]),
+    "b2f_selector_create": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
+                                      C.c_void_p, C.c_int64, C.POINTER(C.c_void_p)]),
+    "b2f_selector_count": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
+    "b2f_selector_destroy": (None, [C.c_void_p]),
+    "b2f_search_sel": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
+    "b2f_search_device_async_sel": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p,
+                                              C.c_void_p]),
+    "b2f_search_xchg_async_sel": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p,
+                                            C.c_void_p, C.c_int]),
     "b2f_merge_packed_device_async": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_int64,
                                                 C.c_int, C.c_void_p, C.c_void_p]),
     "b2f_xchg_create": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_void_p]),

@@ -37,6 +37,7 @@
 #include "common.cuh"
 #include "kernels_scan.cuh"
 #include "kernels_select.cuh"
+#include "kernels_selector.cuh"
 #include "kernels_umma.cuh"
 #include "kernels_umma_qs.cuh"
 #include "kernels_util.cuh"
@@ -258,6 +259,28 @@ struct ShardWorker {
 
 struct Pending {
   const float* q; int64_t nq; int k; float* D; int64_t* I; int slot;
+  const b2f_selector* sel;   // the overflow re-run filters with it too
+};
+
+namespace {
+// One shard's part of a selector (kernels_selector.cuh): the row bitmap and the lists of the tiles that hold a
+// selected row, in ascending order.
+struct SelShard {
+  int dev = 0;
+  int64_t count = 0;                 // selected rows
+  uint32_t* bits = nullptr;          // [round_up(n, kQsTileRows) / 32]
+  int* qs_tiles = nullptr;           // QS tiles (kQsTileRows rows)
+  int* ts_tiles = nullptr;           // TS tiles (kTileRows rows)
+  int n_qs = 0, n_ts = 0;
+  std::vector<int> ts_host;          // host copy: the phased TS schedules walk a sub-range per phase
+};
+}  // namespace
+
+struct b2f_selector {
+  b2f_index* idx = nullptr;
+  uint64_t generation = 0;           // the index generation it was built against
+  int64_t count = 0;
+  std::vector<SelShard> parts;       // one per shard
 };
 
 struct b2f_index {
@@ -287,6 +310,7 @@ struct b2f_index {
     struct Deferred { bool valid = false; unsigned int seq = 0; int64_t nq = 0; int k = 0; float* D = nullptr; int64_t* I = nullptr; } deferred;
   } xchg;
   int64_t ntotal = 0;
+  std::atomic<uint64_t> generation{0};   // bumped by every add and reset: a selector built before is stale
   std::mutex ntotal_mutex;     // b2f_add_flat_file may run on several shards at once (one host thread each)
   // options
   int path = B2F_PATH_AUTO;
@@ -758,7 +782,7 @@ int pass_variant(const b2f_index* idx, const PassPlan& plan, int nqp) {
 // D_out/I_out with row stride out_stride.
 int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q32p, const __nv_bfloat16* q16p,
                  const float* qnormp, const float* qerrp, int nqp, int k, float* D_out, int64_t* I_out, int64_t out_stride,
-                 int* ovf_dst, const float* qscalep = nullptr) {
+                 int* ovf_dst, const float* qscalep, const SelShard* sel) {
   Workspace& W = S.ws;
   Stats& st = S.stats;   // per shard: shards may be enqueued from different host threads
   const int64_t N = S.n;
@@ -800,8 +824,10 @@ int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q3
     B2F_TRY(make_tmap_bf16(&tmap_p, shadow, srows, kBlockK, kShadowTileRows));        // one K-block of a 32-row tile
     B2F_TRY(make_tmap_bf16(&tmap_ph, shadow, srows, kBlockK, kShadowTileRows, true)); // half a K-block of a 32-row tile
     B2F_TRY(make_tmap_bf16(&tmap_q, q16p, static_cast<uint64_t>(n_cols), i8 ? kD / 2 : kD, static_cast<uint32_t>(n_cols / 2)));
-    const int te = static_cast<int>((N + kQsTileRows - 1) / kQsTileRows);
+    // filtered: the launch walks the listed tiles only
+    const int te = sel ? sel->n_qs : static_cast<int>((N + kQsTileRows - 1) / kQsTileRows);
     UmmaQsArgs a;
+    a.sel_bits = sel ? sel->bits : nullptr; a.tile_list = sel ? sel->qs_tiles : nullptr;
     a.n_rows = N; a.tile_begin = 0; a.tile_end = te; a.n_cols = n_cols; a.nq = nqp;
     a.a_stages = qp.a_stages; a.q_stages = qp.q_stages; a.resident_kb = qp.resident_kb; a.q16 = q16p;
     a.half_stage = qp.half_stage;
@@ -816,16 +842,29 @@ int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q3
     a.x16_bytes = static_cast<const unsigned char*>(shadow);
     a.pf_limit_bytes = shadow_rows_padded(N) * static_cast<int64_t>(kD) * (i8 ? 1 : 2);
     a.qscale = qscalep; a.tscale = S.tscale;
-    a.prefetch = idx->l2_prefetch;
-    a.dense_quarters = std::min(4, std::max(1, (4 * k + 2 * pairs * 32 - 1) / (2 * pairs * 32)));
-    a.first_wait_cycles = (idx->tighten && N >= 4ll * pairs * kQsTileRows && a.dense_quarters < 4) ? 100000 : 0;
+    a.prefetch = sel ? 0 : idx->l2_prefetch;
+    if (!sel) {
+      a.dense_quarters = std::min(4, std::max(1, (4 * k + 2 * pairs * 32 - 1) / (2 * pairs * 32)));
+      a.first_wait_cycles = (idx->tighten && N >= 4ll * pairs * kQsTileRows && a.dense_quarters < 4) ? 100000 : 0;
+    } else {
+      // the same protocol on the selected rows: a quarter of the first listed tiles holds about `density` x 32 of them
+      const double rows_q = 2.0 * pairs * 32 * static_cast<double>(sel->count) / (static_cast<double>(te) * kQsTileRows);
+      a.dense_quarters = static_cast<int>(std::min(4.0, std::max(1.0, std::ceil(4.0 * k / rows_q))));
+      a.first_wait_cycles = (idx->tighten && te >= 4 * pairs && a.dense_quarters < 4) ? 100000 : 0;
+    }
     {
       ProfScope ps(idx, S, 0);
-      if (i8) umma_qs_score_select_kernel<true><<<2 * pairs, kQsThreads, qp.smem_bytes, s>>>(tmap_p, tmap_ph, tmap_q, a);
-      else umma_qs_score_select_kernel<false><<<2 * pairs, kQsThreads, qp.smem_bytes, s>>>(tmap_p, tmap_ph, tmap_q, a);
+      const dim3 g(2 * pairs);
+      if (sel) {
+        if (i8) umma_qs_score_select_kernel<true, true><<<g, kQsThreads, qp.smem_bytes, s>>>(tmap_p, tmap_ph, tmap_q, a);
+        else umma_qs_score_select_kernel<false, true><<<g, kQsThreads, qp.smem_bytes, s>>>(tmap_p, tmap_ph, tmap_q, a);
+      } else {
+        if (i8) umma_qs_score_select_kernel<true, false><<<g, kQsThreads, qp.smem_bytes, s>>>(tmap_p, tmap_ph, tmap_q, a);
+        else umma_qs_score_select_kernel<false, false><<<g, kQsThreads, qp.smem_bytes, s>>>(tmap_p, tmap_ph, tmap_q, a);
+      }
     }
     CU_TRY(cudaGetLastError());
-    st.score_rows += static_cast<double>(N);
+    st.score_rows += sel ? static_cast<double>(te) * kQsTileRows : static_cast<double>(N);
     st.launches += 1;
     st.phases += 1;
     st.qs_passes += 1;
@@ -872,35 +911,60 @@ int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q3
       const int tb = static_cast<int>(begin / kTileRows);
       const int te = static_cast<int>((end + kTileRows - 1) / kTileRows);
       if (end < N) end = static_cast<int64_t>(te) * kTileRows;  // phases end on tile boundaries
+      // filtered: the listed tiles of [tb, te)
+      int lb = tb, le = te;
+      if (sel) {
+        lb = static_cast<int>(std::lower_bound(sel->ts_host.begin(), sel->ts_host.end(), tb) - sel->ts_host.begin());
+        le = static_cast<int>(std::lower_bound(sel->ts_host.begin(), sel->ts_host.end(), te) - sel->ts_host.begin());
+      }
       UmmaArgs a;
-      a.n_rows = N; a.tile_begin = tb; a.tile_end = te; a.nq = nqp; a.q16 = q16p;
+      a.n_rows = N; a.tile_begin = lb; a.tile_end = le; a.nq = nqp; a.q16 = q16p;
+      a.sel_bits = sel ? sel->bits : nullptr; a.tile_list = sel ? sel->ts_tiles : nullptr;
       a.qscale = qscalep; a.tscale = S.tscale;
       a.dense = dense ? 1 : 0; a.cand = W.cand[cur]; a.C = C; a.S = plan.S; a.cap_p = cap_h;
       a.max_pairs = n_areas; a.cnt2 = W.cnt2; a.tau = W.tau; a.ovf = W.ovf; a.err = W.err;
       a.tighten = idx->tighten; a.tighten_adaptive = idx->tighten_adaptive; a.k = k; a.margin = W.margin; a.hist = W.hist; a.hkey0 = W.hkey0; a.hshift = W.hshift;
-      const int pairs = std::min(S.max_pairs, te - tb);
+      const int pairs = std::min(S.max_pairs, le - lb);
       // wait for the first thresholds after the first tile: only when that tile's rows can place them (about half of
       // pairs * 64 rows score above the histogram floor) and the shard is long enough to be worth it
       a.count_exact_lower_bound = one_launch ? 1 : 0;
-      a.first_wait_cycles = (one_launch && N >= 8ll * pairs * kTileRows && 4ll * k <= static_cast<int64_t>(pairs) * kTileRows) ? 100000 : 0;
-      {
-        ProfScope ps(idx, S, 0);
-        if (i8) umma_score_select_kernel<true><<<2 * pairs, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
-        else umma_score_select_kernel<false><<<2 * pairs, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
+      if (!sel) {
+        a.first_wait_cycles = (one_launch && N >= 8ll * pairs * kTileRows && 4ll * k <= static_cast<int64_t>(pairs) * kTileRows) ? 100000 : 0;
+      } else {   // the same rule on the selected rows of the listed tiles
+        const double density = static_cast<double>(sel->count) / (static_cast<double>(sel->n_ts) * kTileRows);
+        a.first_wait_cycles = (one_launch && le - lb >= 8 * pairs && 4.0 * k <= pairs * kTileRows * density) ? 100000 : 0;
       }
-      st.score_rows += static_cast<double>(std::min<int64_t>(N, static_cast<int64_t>(te) * kTileRows) - begin);
+      if (pairs > 0) {   // a filtered phase may hold no listed tile
+        ProfScope ps(idx, S, 0);
+        const dim3 g(2 * pairs);
+        if (sel) {
+          if (i8) umma_score_select_kernel<true, true><<<g, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
+          else umma_score_select_kernel<false, true><<<g, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
+        } else {
+          if (i8) umma_score_select_kernel<true, false><<<g, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
+          else umma_score_select_kernel<false, false><<<g, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
+        }
+      }
+      st.score_rows += sel ? static_cast<double>(le - lb) * kTileRows
+                           : static_cast<double>(std::min<int64_t>(N, static_cast<int64_t>(te) * kTileRows) - begin);
     } else {
       ScanArgs a;
       a.x32 = S.x32; a.row_begin = begin; a.row_end = end; a.q32 = q32p; a.nq_pass = nqp;
       a.dense = dense ? 1 : 0; a.dense_row0 = 0; a.cand = W.cand[cur]; a.cnt = W.cnt; a.C = C;
-      a.tau = W.tau; a.tauP = W.tauP; a.ovf = W.ovf;
+      a.tau = W.tau; a.tauP = W.tauP; a.ovf = W.ovf; a.sel_bits = sel ? sel->bits : nullptr;
       const int64_t groups = (end - begin + kScanRows - 1) / kScanRows;
       const int blocks = static_cast<int>(std::min<int64_t>((groups + 7) / 8, static_cast<int64_t>(S.sm_count)));
       const size_t sm = scan_smem_bytes(nqp, plan.exact);
       {
         ProfScope ps(idx, S, 0);
-        if (plan.exact) scan_kernel<true><<<std::max(blocks, 1), kScanThreads, sm, s>>>(a);
-        else scan_kernel<false><<<std::max(blocks, 1), kScanThreads, sm, s>>>(a);
+        const dim3 g(std::max(blocks, 1));
+        if (sel) {
+          if (plan.exact) scan_kernel<true, true><<<g, kScanThreads, sm, s>>>(a);
+          else scan_kernel<false, true><<<g, kScanThreads, sm, s>>>(a);
+        } else {
+          if (plan.exact) scan_kernel<true, false><<<g, kScanThreads, sm, s>>>(a);
+          else scan_kernel<false, false><<<g, kScanThreads, sm, s>>>(a);
+        }
       }
       st.score_rows += static_cast<double>(end - begin);
       if (dense) n_override = static_cast<int>(end - begin);
@@ -978,14 +1042,15 @@ int resolve_path(const b2f_index* idx, const Shard& S, int64_t nq) {
 }
 
 // Enqueue the whole search of one shard.  q_d: fp32 queries on the shard's device.
+// sel: this shard's part of a selector, or null (no filter).
 int enqueue_search(b2f_index* idx, Shard& S, const float* q_d, int64_t nq, int k, float* D_d, int64_t* I_d,
-                   int slot = 0) {
+                   int slot = 0, const SelShard* sel = nullptr) {
   CU_TRY(cudaSetDevice(S.dev));
   Workspace& W = S.ws;
   cudaStream_t s = S.stream;
   int* ovf_slot_host = W.ovf_host + static_cast<size_t>(slot) * W.nq_cap;
   int* ovf_slot = W.ovf_all + static_cast<size_t>(slot) * W.nq_cap;
-  if (S.n == 0) {
+  if (S.n == 0 || (sel && sel->count == 0)) {   // nothing to search: padding only
     fill_pad_kernel<<<static_cast<int>((nq * k + 255) / 256), 256, 0, s>>>(D_d, I_d, nq * k);
     CU_TRY(cudaGetLastError());
     std::memset(ovf_slot_host, 0, sizeof(int) * nq);   // no kernel writes the flags of an empty shard
@@ -1008,10 +1073,14 @@ int enqueue_search(b2f_index* idx, Shard& S, const float* q_d, int64_t nq, int k
   if (plan.path == B2F_PATH_UMMA_BF16) {
     static bool attr_set[64] = {false};
     if (!attr_set[S.dev & 63]) {
-      CU_TRY(cudaFuncSetAttribute(umma_score_select_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kUmmaSmemBytes));
-      CU_TRY(cudaFuncSetAttribute(umma_score_select_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kUmmaSmemBytes));
-      CU_TRY(cudaFuncSetAttribute(umma_qs_score_select_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kQsSmemLimit));
-      CU_TRY(cudaFuncSetAttribute(umma_qs_score_select_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kQsSmemLimit));
+      CU_TRY(cudaFuncSetAttribute(umma_score_select_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kUmmaSmemBytes));
+      CU_TRY(cudaFuncSetAttribute(umma_score_select_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kUmmaSmemBytes));
+      CU_TRY(cudaFuncSetAttribute(umma_score_select_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kUmmaSmemBytes));
+      CU_TRY(cudaFuncSetAttribute(umma_score_select_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kUmmaSmemBytes));
+      CU_TRY(cudaFuncSetAttribute(umma_qs_score_select_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kQsSmemLimit));
+      CU_TRY(cudaFuncSetAttribute(umma_qs_score_select_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kQsSmemLimit));
+      CU_TRY(cudaFuncSetAttribute(umma_qs_score_select_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kQsSmemLimit));
+      CU_TRY(cudaFuncSetAttribute(umma_qs_score_select_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kQsSmemLimit));
       CU_TRY(cudaFuncSetAttribute(finalize_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * 8192 * 8));   // P + PS records
       CU_TRY(cudaFuncSetAttribute(bootstrap_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 16384 * 8));
       attr_set[S.dev & 63] = true;
@@ -1019,8 +1088,10 @@ int enqueue_search(b2f_index* idx, Shard& S, const float* q_d, int64_t nq, int k
   } else {
     static bool attr_set2[64] = {false};
     if (!attr_set2[S.dev & 63]) {
-      CU_TRY(cudaFuncSetAttribute(scan_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));
-      CU_TRY(cudaFuncSetAttribute(scan_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));
+      CU_TRY(cudaFuncSetAttribute(scan_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));
+      CU_TRY(cudaFuncSetAttribute(scan_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));
+      CU_TRY(cudaFuncSetAttribute(scan_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));
+      CU_TRY(cudaFuncSetAttribute(scan_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));
       attr_set2[S.dev & 63] = true;
     }
   }
@@ -1030,7 +1101,7 @@ int enqueue_search(b2f_index* idx, Shard& S, const float* q_d, int64_t nq, int k
     const __nv_bfloat16* q16p = S.fmt == kShadowInt8 ? reinterpret_cast<const __nv_bfloat16*>(reinterpret_cast<const int8_t*>(W.q16) + q0 * kD)
                                                      : W.q16 + q0 * kD;
     B2F_TRY(enqueue_pass(idx, S, plan, q_d + q0 * kD, q16p, W.qnorm + q0, W.qerr + q0, nqp, k, D_d + q0 * k,
-                         I_d + q0 * k, k, ovf_slot + q0, W.qscale + q0));
+                         I_d + q0 * k, k, ovf_slot + q0, W.qscale + q0, sel));
   }
   return B2F_OK;
 }
@@ -1038,12 +1109,12 @@ int enqueue_search(b2f_index* idx, Shard& S, const float* q_d, int64_t nq, int k
 // After the stream drained: re-run any query whose candidate list overflowed on the exact engine
 // (bounded phases, cannot overflow).  Normally a no-op.
 int finish_search(b2f_index* idx, Shard& S, const float* q_d, int64_t nq, int k, float* D_d, int64_t* I_d,
-                  int slot = 0, bool* reran = nullptr) {
+                  int slot = 0, bool* reran = nullptr, const SelShard* sel = nullptr) {
   CU_TRY(cudaSetDevice(S.dev));
   CU_TRY(cudaStreamSynchronize(S.stream));
   if (idx->profile) collect_prof(idx, S);
   if (reran) *reran = false;
-  if (S.n == 0) return B2F_OK;
+  if (S.n == 0 || (sel && sel->count == 0)) return B2F_OK;
   Workspace& W = S.ws;
   const int* flags = W.ovf_host + static_cast<size_t>(slot) * W.nq_cap;
   std::vector<int64_t> bad;
@@ -1058,7 +1129,8 @@ int finish_search(b2f_index* idx, Shard& S, const float* q_d, int64_t nq, int k,
   S.stats.fallback_queries += static_cast<double>(bad.size());
   static bool attr_set3[64] = {false};
   if (!attr_set3[S.dev & 63]) {
-    CU_TRY(cudaFuncSetAttribute(scan_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));
+    CU_TRY(cudaFuncSetAttribute(scan_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));
+    CU_TRY(cudaFuncSetAttribute(scan_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));
     attr_set3[S.dev & 63] = true;
   }
   const PassPlan plan = make_plan(idx, S, B2F_PATH_SCAN_EXACT, k, 0);
@@ -1069,7 +1141,8 @@ int finish_search(b2f_index* idx, Shard& S, const float* q_d, int64_t nq, int k,
     for (int i = 0; i < nb; ++i)
       CU_TRY(cudaMemcpyAsync(W.fbq + static_cast<size_t>(i) * kD, q_d + bad[b0 + i] * kD, kD * 4,
                              cudaMemcpyDeviceToDevice, s));
-    B2F_TRY(enqueue_pass(idx, S, plan, W.fbq, nullptr, W.qnorm /*unused: exact*/, W.qerr, nb, k, W.fbD, W.fbI, k, nullptr));
+    B2F_TRY(enqueue_pass(idx, S, plan, W.fbq, nullptr, W.qnorm /*unused: exact*/, W.qerr, nb, k, W.fbD, W.fbI, k, nullptr,
+                         nullptr, sel));
     for (int i = 0; i < nb; ++i) {
       // cudaMemcpyDefault: D_d / I_d may be mapped pinned host memory (b2f_search writes results there directly)
       CU_TRY(cudaMemcpyAsync(D_d + bad[b0 + i] * k, W.fbD + static_cast<size_t>(i) * k, sizeof(float) * k,
@@ -1114,7 +1187,8 @@ int settle_pending(b2f_index* idx) {
   Shard& S = idx->shards[0];
   std::vector<Pending> todo;
   todo.swap(idx->pending);
-  for (const Pending& p : todo) B2F_TRY(finish_search(idx, S, p.q, p.nq, p.k, p.D, p.I, p.slot));
+  for (const Pending& p : todo)
+    B2F_TRY(finish_search(idx, S, p.q, p.nq, p.k, p.D, p.I, p.slot, nullptr, p.sel ? &p.sel->parts[0] : nullptr));
   return B2F_OK;
 }
 
@@ -1125,6 +1199,15 @@ bool search_would_realloc(const b2f_index* idx, const Shard& S, int64_t nq, int 
   if (S.n == 0) return false;
   const PassPlan plan = make_plan(idx, S, resolve_path(idx, S, nq), k, nq);
   return plan.qp > W.qp_cap || plan.C > W.C;
+}
+
+// A selector filters only the index it was built for, and only while no row was added or removed since.
+int check_selector(const b2f_index* idx, const b2f_selector* sel) {
+  if (!sel) return B2F_OK;
+  if (sel->idx != idx) return fail(B2F_ERR_INVALID, "selector was built for another index");
+  if (sel->generation != idx->generation.load())
+    return fail(B2F_ERR_INVALID, "stale selector: rows were added to or removed from the index after it was built");
+  return B2F_OK;
 }
 
 int check_args_search(const b2f_index* idx, const void* q, int64_t nq, int k, const void* D, const void* I) {
@@ -1294,6 +1377,7 @@ static int add_impl(b2f_index* idx, const float* x_host, const int64_t* ids_host
   if (n < 0 || (n > 0 && !x_host)) return fail(B2F_ERR_INVALID, "bad add arguments");
   if (n == 0) return B2F_OK;
   B2F_TRY(settle_pending(idx));
+  ++idx->generation;
   const int G = static_cast<int>(idx->shards.size());
   if (ids_host) {
     for (Shard& S : idx->shards)
@@ -1343,6 +1427,7 @@ int b2f_add_device(b2f_index* idx, int shard, const float* x_dev, int64_t n) {
   B2F_TRY(settle_pending(idx));
   Shard& S = idx->shards[shard];
   if (S.has_ids && S.n > 0) return fail(B2F_ERR_INVALID, "index uses explicit ids");
+  ++idx->generation;
   CU_TRY(cudaSetDevice(S.dev));
   B2F_TRY(ensure_capacity(idx, S, S.n + n));
   CU_TRY(cudaMemcpyAsync(S.x32 + S.n * kD, x_dev, static_cast<size_t>(n) * kD * 4, cudaMemcpyDeviceToDevice, S.stream));
@@ -1362,6 +1447,7 @@ int b2f_add_synthetic(b2f_index* idx, int shard, int64_t first_row, int64_t n, u
   B2F_TRY(settle_pending(idx));
   Shard& S = idx->shards[shard];
   if (S.has_ids && S.n > 0) return fail(B2F_ERR_INVALID, "index uses explicit ids");
+  ++idx->generation;
   CU_TRY(cudaSetDevice(S.dev));
   B2F_TRY(ensure_capacity(idx, S, S.n + n));
   const uint32_t k0 = static_cast<uint32_t>(seed) ^ static_cast<uint32_t>(stream);
@@ -1393,6 +1479,7 @@ int b2f_reconstruct_n(b2f_index* idx, int shard, int64_t row0, int64_t n, float*
 int b2f_reset(b2f_index* idx) {
   if (!idx) return fail(B2F_ERR_INVALID, "null index");
   B2F_TRY(settle_pending(idx));
+  ++idx->generation;
   for (Shard& S : idx->shards) {
     CU_TRY(cudaSetDevice(S.dev));
     CU_TRY(cudaStreamSynchronize(S.stream));
@@ -1427,7 +1514,13 @@ int b2f_search_device(b2f_index* idx, const float* q_dev, int64_t nq, int k, flo
 }
 
 int b2f_search_device_async(b2f_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev) {
+  return b2f_search_device_async_sel(idx, nullptr, q_dev, nq, k, D_dev, I_dev);
+}
+
+int b2f_search_device_async_sel(b2f_index* idx, const b2f_selector* sel, const float* q_dev, int64_t nq, int k,
+                                float* D_dev, int64_t* I_dev) {
   B2F_TRY(check_args_search(idx, q_dev, nq, k, D_dev, I_dev));
+  B2F_TRY(check_selector(idx, sel));
   if (idx->shards.size() != 1) return fail(B2F_ERR_INVALID, "b2f_search_device_async needs a single-shard index");
   if (nq == 0) return B2F_OK;
   Shard& S = idx->shards[0];
@@ -1436,8 +1529,8 @@ int b2f_search_device_async(b2f_index* idx, const float* q_dev, int64_t nq, int 
     B2F_TRY(settle_pending(idx));
   B2F_TRY(ensure_query_ws(S, nq, k));
   const int slot = static_cast<int>(idx->pending.size());
-  B2F_TRY(enqueue_search(idx, S, q_dev, nq, k, D_dev, I_dev, slot));
-  idx->pending.push_back(Pending{q_dev, nq, k, D_dev, I_dev, slot});
+  B2F_TRY(enqueue_search(idx, S, q_dev, nq, k, D_dev, I_dev, slot, sel ? &sel->parts[0] : nullptr));
+  idx->pending.push_back(Pending{q_dev, nq, k, D_dev, I_dev, slot, sel});
   return B2F_OK;
 }
 
@@ -1591,7 +1684,13 @@ static int xchg_push_and_merge(b2f_index* idx, int64_t nq, int k, float* D_dev, 
 
 int b2f_search_xchg_async(b2f_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev,
                           int repush_only) {
+  return b2f_search_xchg_async_sel(idx, nullptr, q_dev, nq, k, D_dev, I_dev, repush_only);
+}
+
+int b2f_search_xchg_async_sel(b2f_index* idx, const b2f_selector* sel, const float* q_dev, int64_t nq, int k,
+                              float* D_dev, int64_t* I_dev, int repush_only) {
   B2F_TRY(check_args_search(idx, q_dev, nq, k, D_dev, I_dev));
+  B2F_TRY(check_selector(idx, sel));
   if (!idx->xchg.connected) return fail(B2F_ERR_INVALID, "exchange not connected (b2f_xchg_create / b2f_xchg_connect)");
   if (nq > idx->xchg.max_nq || k > idx->xchg.max_k || nq * static_cast<int64_t>(k) > idx->xchg.max_nq * idx->xchg.max_k)
     return fail(B2F_ERR_INVALID, "batch exceeds the exchange buffers");
@@ -1599,7 +1698,7 @@ int b2f_search_xchg_async(b2f_index* idx, const float* q_dev, int64_t nq, int k,
   auto& X = idx->xchg;
   float* Dl = reinterpret_cast<float*>(X.stage);
   int64_t* Il = reinterpret_cast<int64_t*>(X.stage + round_up(nq * k * 4, 16));
-  if (!repush_only) B2F_TRY(b2f_search_device_async(idx, q_dev, nq, k, Dl, Il));
+  if (!repush_only) B2F_TRY(b2f_search_device_async_sel(idx, sel, q_dev, nq, k, Dl, Il));
   CU_TRY(cudaSetDevice(idx->shards[0].dev));
   return xchg_push_and_merge(idx, nq, k, D_dev, I_dev);
 }
@@ -1618,7 +1717,13 @@ static bool is_pinned_host(const void* p) {
 }
 
 int b2f_search(b2f_index* idx, const float* q_host, int64_t nq, int k, float* D_host, int64_t* I_host) {
+  return b2f_search_sel(idx, nullptr, q_host, nq, k, D_host, I_host);
+}
+
+int b2f_search_sel(b2f_index* idx, const b2f_selector* sel, const float* q_host, int64_t nq, int k, float* D_host,
+                   int64_t* I_host) {
   B2F_TRY(check_args_search(idx, q_host, nq, k, D_host, I_host));
+  B2F_TRY(check_selector(idx, sel));
   if (nq == 0) return B2F_OK;
   B2F_TRY(settle_pending(idx));
   reset_stats(idx);
@@ -1665,16 +1770,16 @@ int b2f_search(b2f_index* idx, const float* q_host, int64_t nq, int k, float* D_
     CU_TRY(cudaSetDevice(S.dev));
     B2F_TRY(ensure_query_ws(S, nq, k));
     CU_TRY(cudaMemcpyAsync(S.ws.q32, q_src, qbytes, cudaMemcpyHostToDevice, S.stream));
-    return enqueue_search(idx, S, S.ws.q32, nq, k, part_D(g), part_I(g));
+    return enqueue_search(idx, S, S.ws.q32, nq, k, part_D(g), part_I(g), 0, sel ? &sel->parts[g] : nullptr);
   }));
   if (G == 1) {
     // ONE synchronisation; only if a candidate list overflowed (rare) the affected queries are re-run,
     // their rows rewritten in place
-    B2F_TRY(finish_search(idx, S0, S0.ws.q32, nq, k, outD, outI, 0, nullptr));
+    B2F_TRY(finish_search(idx, S0, S0.ws.q32, nq, k, outD, outI, 0, nullptr, sel ? &sel->parts[0] : nullptr));
   } else {
     for (int g = 0; g < G; ++g) {
       Shard& S = idx->shards[g];
-      B2F_TRY(finish_search(idx, S, S.ws.q32, nq, k, part_D(g), part_I(g)));
+      B2F_TRY(finish_search(idx, S, S.ws.q32, nq, k, part_D(g), part_I(g), 0, nullptr, sel ? &sel->parts[g] : nullptr));
     }
     CU_TRY(cudaSetDevice(S0.dev));
     Workspace& W = S0.ws;
@@ -1748,6 +1853,119 @@ int b2f_search_xchg_host(b2f_index* idx, const float* q_host, int64_t nq, int k,
   return B2F_OK;
 }
 
+static void free_selector_parts(b2f_selector* sel) {
+  for (SelShard& P : sel->parts) {
+    if (!P.bits && !P.qs_tiles && !P.ts_tiles) continue;
+    cudaSetDevice(P.dev);
+    dev_free(P.bits); dev_free(P.qs_tiles); dev_free(P.ts_tiles);
+  }
+  (void)cudaGetLastError();
+}
+
+// Evaluate the selector on every row of one shard (selector_bits_kernel), then compact the tile flags into the
+// tile lists on the host: the one synchronisation of the build.
+static int build_selector_part(b2f_index* idx, Shard& S, const SelDesc& desc_host, const std::vector<int64_t>& ids,
+                               const uint8_t* bitmap_host, SelShard& P) {
+  P.dev = S.dev;
+  if (S.n == 0) return B2F_OK;
+  CU_TRY(cudaSetDevice(S.dev));
+  B2F_TRY(upload_segs(S));
+  const int64_t n_words = round_up(S.n, kQsTileRows) / 32;
+  const int64_t n_qs = n_words / (kQsTileRows / 32), n_ts = n_words / (kTileRows / 32);
+  B2F_TRY(dev_alloc(&P.bits, static_cast<size_t>(n_words)));
+  // scratch: [count (8 bytes)][QS tile flags][TS tile flags], the sorted ids, the bitmap
+  struct Scratch {
+    unsigned char* flags = nullptr; int64_t* ids = nullptr; uint8_t* bitmap = nullptr;
+    ~Scratch() { dev_free(flags); dev_free(ids); dev_free(bitmap); }
+  } tmp;
+  const size_t flag_bytes = 8 + static_cast<size_t>(n_qs + n_ts);
+  B2F_TRY(dev_alloc(&tmp.flags, flag_bytes));
+  SelDesc d = desc_host;
+  if (d.kind == kSelBatch && !ids.empty()) {
+    B2F_TRY(dev_alloc(&tmp.ids, ids.size()));
+    CU_TRY(cudaMemcpyAsync(tmp.ids, ids.data(), ids.size() * 8, cudaMemcpyHostToDevice, S.stream));
+  }
+  if (d.kind == kSelBitmap && d.n_bytes > 0) {
+    B2F_TRY(dev_alloc(&tmp.bitmap, static_cast<size_t>(d.n_bytes)));
+    CU_TRY(cudaMemcpyAsync(tmp.bitmap, bitmap_host, static_cast<size_t>(d.n_bytes), cudaMemcpyHostToDevice, S.stream));
+  }
+  d.ids = tmp.ids;
+  d.n_ids = static_cast<int64_t>(ids.size());
+  d.bitmap = tmp.bitmap;
+  CU_TRY(cudaMemsetAsync(tmp.flags, 0, flag_bytes, S.stream));
+  const int blocks = static_cast<int>(std::min<int64_t>((n_words + 7) / 8, static_cast<int64_t>(S.sm_count) * 8));
+  selector_bits_kernel<<<blocks, 256, 0, S.stream>>>(d, S.n, n_words, S.segs_d, static_cast<int>(S.segs.size()),
+                                                     S.has_ids ? S.idmap : nullptr, P.bits, tmp.flags + 8,
+                                                     tmp.flags + 8 + n_qs, reinterpret_cast<unsigned long long*>(tmp.flags));
+  CU_TRY(cudaGetLastError());
+  std::vector<unsigned char> flags(flag_bytes);
+  CU_TRY(cudaMemcpyAsync(flags.data(), tmp.flags, flag_bytes, cudaMemcpyDeviceToHost, S.stream));
+  CU_TRY(cudaStreamSynchronize(S.stream));
+  unsigned long long count = 0;
+  std::memcpy(&count, flags.data(), 8);
+  P.count = static_cast<int64_t>(count);
+  std::vector<int> qs;
+  for (int64_t t = 0; t < n_qs; ++t)
+    if (flags[8 + t]) qs.push_back(static_cast<int>(t));
+  for (int64_t t = 0; t < n_ts; ++t)
+    if (flags[8 + n_qs + t]) P.ts_host.push_back(static_cast<int>(t));
+  P.n_qs = static_cast<int>(qs.size());
+  P.n_ts = static_cast<int>(P.ts_host.size());
+  B2F_TRY(dev_alloc(&P.qs_tiles, qs.size()));
+  B2F_TRY(dev_alloc(&P.ts_tiles, P.ts_host.size()));
+  if (!qs.empty()) CU_TRY(cudaMemcpy(P.qs_tiles, qs.data(), qs.size() * 4, cudaMemcpyHostToDevice));
+  if (!P.ts_host.empty()) CU_TRY(cudaMemcpy(P.ts_tiles, P.ts_host.data(), P.ts_host.size() * 4, cudaMemcpyHostToDevice));
+  return B2F_OK;
+}
+
+int b2f_selector_create(b2f_index* idx, int kind, int invert, int64_t imin, int64_t imax, const int64_t* ids_host,
+                        int64_t n_ids, const uint8_t* bitmap_host, int64_t n_bytes, b2f_selector** out) {
+  if (!out) return fail(B2F_ERR_INVALID, "null out pointer");
+  *out = nullptr;
+  if (!idx) return fail(B2F_ERR_INVALID, "null index");
+  if (kind != kSelRange && kind != kSelBatch && kind != kSelBitmap)
+    return fail(B2F_ERR_INVALID, "selector kind must be B2F_SEL_RANGE, B2F_SEL_BATCH or B2F_SEL_BITMAP");
+  if (kind == kSelBatch && (n_ids < 0 || (n_ids > 0 && !ids_host))) return fail(B2F_ERR_INVALID, "bad batch selector ids");
+  if (kind == kSelBitmap && (n_bytes < 0 || (n_bytes > 0 && !bitmap_host)))
+    return fail(B2F_ERR_INVALID, "bad bitmap selector bytes");
+  B2F_TRY(settle_pending(idx));
+  SelDesc d{kind, invert ? 1 : 0, imin, imax, nullptr, 0, nullptr, kind == kSelBitmap ? n_bytes : 0};
+  std::vector<int64_t> ids;
+  if (kind == kSelBatch) {   // any order, duplicates allowed: sorted and unique for the per-row binary search
+    ids.assign(ids_host, ids_host + n_ids);
+    std::sort(ids.begin(), ids.end());
+    ids.erase(std::unique(ids.begin(), ids.end()), ids.end());
+  }
+  std::unique_ptr<b2f_selector> sel(new b2f_selector());
+  sel->idx = idx;
+  sel->generation = idx->generation.load();
+  sel->parts.resize(idx->shards.size());
+  for (size_t g = 0; g < idx->shards.size(); ++g) {
+    const int rc = build_selector_part(idx, idx->shards[g], d, ids, bitmap_host, sel->parts[g]);
+    if (rc != B2F_OK) {
+      const std::string msg = g_err;
+      free_selector_parts(sel.get());
+      return fail(rc, msg);
+    }
+    sel->count += sel->parts[g].count;
+  }
+  *out = sel.release();
+  return B2F_OK;
+}
+
+int b2f_selector_count(const b2f_selector* sel, int64_t* selected_out) {
+  if (!sel || !selected_out) return fail(B2F_ERR_INVALID, "null selector or output pointer");
+  *selected_out = sel->count;
+  return B2F_OK;
+}
+
+void b2f_selector_destroy(b2f_selector* sel) {
+  if (!sel) return;
+  (void)settle_pending(sel->idx);   // searches in flight may still read its bitmap and tile lists
+  free_selector_parts(sel);
+  delete sel;
+}
+
 int b2f_set_option(b2f_index* idx, const char* key, int64_t value) {
   if (!idx || !key) return fail(B2F_ERR_INVALID, "bad option arguments");
   B2F_TRY(settle_pending(idx));
@@ -1760,6 +1978,7 @@ int b2f_set_option(b2f_index* idx, const char* key, int64_t value) {
     if (idx->ntotal > 0) return fail(B2F_ERR_INVALID, "shadow can only be changed on an empty index");
     if (value < 0 || value > 3) return fail(B2F_ERR_INVALID, "shadow must be 0 (none), 1 (bf16), 2 (int8) or 3 (auto)");
     idx->shadow = static_cast<int>(value);
+    ++idx->generation;
     for (Shard& S : idx->shards) {
       cudaSetDevice(S.dev);
       dev_free(S.x32); dev_free(S.x16); dev_free(S.x8); dev_free(S.tscale); dev_free(S.idmap);
@@ -1838,6 +2057,7 @@ int b2f_get_stat(const b2f_index* idx, const char* key, double* out) {
     s.phases = idx->shards[0].stats.phases;
   }
   if (k == "shadow_format") *out = idx->shards.empty() ? 0 : idx->shards[0].fmt;   // 0 none, 1 bf16, 2 int8
+  else if (k == "generation") *out = static_cast<double>(idx->generation.load());   // bumped by every add and reset
   else if (k == "shadow_rho") *out = idx->shards.empty() ? 0 : idx->shards[0].rho;  // AUTO: median 2 eps8 / sigma
   else if (k == "launches") *out = s.launches;
   else if (k == "phases") *out = s.phases;
@@ -1923,6 +2143,7 @@ extern "C" int b2f_add_flat_file(b2f_index* idx, int shard, const char* path, in
   if (gbytes_out) *gbytes_out = 0.0;
   if (n == 0) return B2F_OK;
   if (S.n + n >= 0xfffffff0ll) return fail(B2F_ERR_INVALID, "a shard holds at most 2^32-16 rows");
+  ++idx->generation;
   CU_TRY(cudaSetDevice(S.dev));
   CU_TRY(cudaStreamSynchronize(S.stream));
   if (!S.has_ids) {

@@ -30,6 +30,7 @@ struct ScanArgs {
   const float* tau;        // [nq_pass] approx-mode threshold
   const uint64_t* tauP;    // [nq_pass] exact-mode threshold record
   int* ovf;                // [nq_pass] set when a candidate did not fit
+  const uint32_t* sel_bits;  // SEL instances: the shard's row bitmap (bit r & 31 of word r >> 5: row r is selected)
 };
 
 template <typename T, int V>
@@ -54,7 +55,9 @@ __device__ __forceinline__ T reduce_transpose(T (&a)[V], int lane) {
   return a[0];
 }
 
-template <bool kExact>
+// SEL: filtered search.  Unselected rows never pass; the dense phase stores empty records (0) for them, and outside
+// it a row group without a selected row is not loaded at all.
+template <bool kExact, bool SEL>
 __global__ void __launch_bounds__(kScanThreads, 1) scan_kernel(const ScanArgs a) {
   using acc_t = typename std::conditional<kExact, double, float>::type;
   constexpr int R = kScanRows;
@@ -86,6 +89,13 @@ __global__ void __launch_bounds__(kScanThreads, 1) scan_kernel(const ScanArgs a)
 
   for (int64_t g = gwarp; g < ngroups; g += nwarps) {
     const int64_t r0 = a.row_begin + g * R;
+    if constexpr (SEL) {
+      bool any_sel = false;
+#pragma unroll
+      for (int r = 0; r < R; ++r)
+        any_sel = any_sel || (r0 + r < a.row_end && ((__ldg(a.sel_bits + ((r0 + r) >> 5)) >> ((r0 + r) & 31)) & 1u));
+      if (!any_sel && !a.dense) continue;   // warp-uniform
+    }
     float4 p[R][kF4PerLane];
 #pragma unroll
     for (int r = 0; r < R; ++r) {
@@ -128,11 +138,13 @@ __global__ void __launch_bounds__(kScanThreads, 1) scan_kernel(const ScanArgs a)
       const int64_t row = r0 + my_r;
       const int qi = qb + my_qq;
       if (lane < V && row < a.row_end && qi < a.nq_pass) {
+        bool sel_ok = true;
+        if constexpr (SEL) sel_ok = (__ldg(a.sel_bits + (row >> 5)) >> (row & 31)) & 1u;
         const uint64_t rec = pack_cand(score, static_cast<uint32_t>(row));
         if (a.dense) {
-          a.cand[static_cast<int64_t>(qi) * a.C + (row - a.dense_row0)] = rec;
+          a.cand[static_cast<int64_t>(qi) * a.C + (row - a.dense_row0)] = sel_ok ? rec : 0ull;
         } else {
-          const bool pass = kExact ? (rec > tauP_s[qi]) : (score >= tau_s[qi]);
+          const bool pass = sel_ok && (kExact ? (rec > tauP_s[qi]) : (score >= tau_s[qi]));
           if (pass) {
             const int slot = atomicAdd(a.cnt + qi, 1);
             if (slot < a.C) a.cand[static_cast<int64_t>(qi) * a.C + slot] = rec;

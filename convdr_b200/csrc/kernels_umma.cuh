@@ -101,7 +101,20 @@ struct UmmaArgs {
   const int* hshift;          // [nq] log2(keys per bucket)
   const float* qscale;        // int8 shadow: [nq] query scales sq (q16 then points at the int8 codes)
   const float* tscale;        // int8 shadow: [row tiles of 32] tile scales st
+  // Filtered search (SEL instances only): the launch walks tile_list[tile_begin .. tile_end) (pair tiles that hold
+  // at least one selected row) instead of the tiles themselves; sel_bits is the shard's row bitmap (bit r & 31 of
+  // word r >> 5: row r is selected).
+  const uint32_t* sel_bits;
+  const int* tile_list;
 };
+
+// Tile of iteration i: the listed tile of a filtered launch, i itself otherwise.  Every role that walks tiles calls
+// it with the same i, so they stay in lockstep.
+template <bool SEL>
+__device__ __forceinline__ int tile_at(const int* tile_list, int i) {
+  if constexpr (SEL) return __ldg(tile_list + i);
+  else return i;
+}
 
 // ------------------------------------------------------------------------------------------
 // PTX wrappers
@@ -400,8 +413,11 @@ __device__ __forceinline__ bool any_ge32_s32(const uint32_t* v, int tau) {
 // column, so a K-step of 32 codes is still 8 columns).  Each epilogue thread's 32 rows are one shadow tile: its
 // float threshold becomes ONE integer threshold per tile (i8_threshold), the compare chain stays one instruction
 // per score, and the float score is only formed for a hit.
+// SEL: filtered search.  The roles walk the listed tiles only; the epilogue ANDs the row bitmap word of its 32 rows
+// into the hit mask (and stores empty records for unselected rows in the dense phase), so only selected rows are
+// ever appended or counted in the tightening histogram.
 // ------------------------------------------------------------------------------------------
-template <bool I8>
+template <bool I8, bool SEL>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
     umma_score_select_kernel(const __grid_constant__ CUtensorMap tmap_p, const UmmaArgs a) {
   constexpr int NKB = I8 ? kShadow8KBlocks : kNumKBlocks;        // K-blocks of 128 bytes per row
@@ -459,7 +475,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
   if (warp == 0 && lane == 0) {
     // ===================== TMA producer =====================
     uint32_t stage = 0, phase = 0;
-    for (int tile = a.tile_begin + pair; tile < a.tile_end; tile += npairs) {
+    for (int ti = a.tile_begin + pair; ti < a.tile_end; ti += npairs) {
+      const int tile = tile_at<SEL>(a.tile_list, ti);
       // shadow layout (common.cuh): CTA tile = 2*tile + rank; kKBlocksPerStage consecutive K-blocks
       // of it are 128 consecutive 128-byte rows = one contiguous 16 KB box
       const int row0 = (tile * 2 + static_cast<int>(cta_rank)) * NKB * kTileRowsCta;
@@ -563,7 +580,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
     const uint32_t tempty_leader = mapa_u32(bar_tempty, 0);
     const float sq = I8 ? a.qscale[q_ok ? q : 0] : 0.f;
     int it = 0;
-    for (int tile = a.tile_begin + pair; tile < a.tile_end; tile += npairs, ++it) {
+    for (int ti = a.tile_begin + pair; ti < a.tile_end; ti += npairs, ++it) {
+      const int tile = tile_at<SEL>(a.tile_list, ti);
       const uint32_t as = static_cast<uint32_t>(it) % kAccStages, aph = (static_cast<uint32_t>(it) / kAccStages) & 1u;
       if (it == 1 && live && a.first_wait_cycles > 0) {
         // The first tile of every pair passed unfiltered (thresholds start at -inf): together those rows place
@@ -585,6 +603,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
       tmem_ld_wait();
       const int64_t row0 = static_cast<int64_t>(tile) * kTileRows + kHalfRows * half;
       const int n_valid = static_cast<int>(max(static_cast<int64_t>(0), min(static_cast<int64_t>(kHalfRows), a.n_rows - row0)));
+      uint32_t sel_word = 0xffffffffu;       // this thread's 32 rows are one bitmap word
+      if constexpr (SEL) sel_word = __ldg(a.sel_bits + (row0 >> 5));
       if constexpr (I8) {
         // one integer threshold for this (query, shadow tile); scores as floats only where they are stored
         const float st = n_valid > 0 ? __ldg(a.tscale + (row0 >> 5)) : 0.f;
@@ -594,8 +614,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
 #pragma unroll
             for (int c = 0; c < kHalfRows; c += 2) {
               ulonglong2 o;
-              o.x = (c < n_valid) ? pack_cand(i8_score(static_cast<int>(v[c]), sq, st), static_cast<uint32_t>(row0 + c)) : 0ull;
-              o.y = (c + 1 < n_valid) ? pack_cand(i8_score(static_cast<int>(v[c + 1]), sq, st), static_cast<uint32_t>(row0 + c + 1)) : 0ull;
+              o.x = (c < n_valid && ((sel_word >> c) & 1u)) ? pack_cand(i8_score(static_cast<int>(v[c]), sq, st), static_cast<uint32_t>(row0 + c)) : 0ull;
+              o.y = (c + 1 < n_valid && ((sel_word >> (c + 1)) & 1u)) ? pack_cand(i8_score(static_cast<int>(v[c + 1]), sq, st), static_cast<uint32_t>(row0 + c + 1)) : 0ull;
               *reinterpret_cast<ulonglong2*>(dst + c) = o;
             }
           }
@@ -607,6 +627,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
 #pragma unroll
             for (int c = 0; c < kHalfRows; ++c) m |= (static_cast<int>(v[c]) >= T) ? (1u << c) : 0u;
             if (n_valid < kHalfRows) m &= (n_valid > 0) ? ((1u << n_valid) - 1u) : 0u;   // shard tail
+            if constexpr (SEL) m &= sel_word;
             uint32_t any = __reduce_or_sync(0xffffffffu, m);
             if (__popc(any) > 6) {   // busy word: unrolled predicated stores, v[] stays in registers
               if (m) {
@@ -644,8 +665,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
 #pragma unroll
           for (int c = 0; c < kHalfRows; c += 2) {
             ulonglong2 o;
-            o.x = (c < n_valid) ? pack_cand(__uint_as_float(v[c]), static_cast<uint32_t>(row0 + c)) : 0ull;
-            o.y = (c + 1 < n_valid) ? pack_cand(__uint_as_float(v[c + 1]), static_cast<uint32_t>(row0 + c + 1)) : 0ull;
+            o.x = (c < n_valid && ((sel_word >> c) & 1u)) ? pack_cand(__uint_as_float(v[c]), static_cast<uint32_t>(row0 + c)) : 0ull;
+            o.y = (c + 1 < n_valid && ((sel_word >> (c + 1)) & 1u)) ? pack_cand(__uint_as_float(v[c + 1]), static_cast<uint32_t>(row0 + c + 1)) : 0ull;
             *reinterpret_cast<ulonglong2*>(dst + c) = o;
           }
         }
@@ -658,6 +679,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
 #pragma unroll
         for (int c = 0; c < kHalfRows; ++c) m |= (__uint_as_float(v[c]) >= tau) ? (1u << c) : 0u;
         if (n_valid < kHalfRows) m &= (n_valid > 0) ? ((1u << n_valid) - 1u) : 0u;   // shard tail
+        if constexpr (SEL) m &= sel_word;
         uint32_t any = __reduce_or_sync(0xffffffffu, m);
         if (__popc(any) > 6) {
           if (m) {

@@ -76,6 +76,10 @@ struct UmmaQsArgs {
   int first_wait_cycles;      // the other quarters wait this long at most for every threshold to exist (0: no wait)
   const float* qscale;        // int8 shadow: [n_cols] query scales sq (0 for padded columns)
   const float* tscale;        // int8 shadow: [row tiles of 32] tile scales st
+  // Filtered search (SEL instances only): the launch walks tile_list[tile_begin .. tile_end) (pair tiles of 256 rows
+  // that hold at least one selected row); sel_bits is the shard's row bitmap (bit r & 31 of word r >> 5: row r).
+  const uint32_t* sel_bits;
+  const int* tile_list;
 };
 
 struct QsPlan { int a_stages, q_stages, resident_kb, smem_bytes, half_stage; };
@@ -206,8 +210,10 @@ __device__ __forceinline__ bool any_ge16_s32(const uint32_t (&v)[16], const int 
 // thresholds: once per tile the warp's lanes convert the float thresholds of its query columns for the tile scale
 // (one 32-row shadow tile per warp) into a per-warp shared-memory scratch, which every lane reads per 16-query
 // chunk with 4 LDS.128 — the same cost as the float thresholds of the bf16 path.
+// SEL: filtered search.  Every role walks the listed tiles only (tile_at); an epilogue warp's 32 rows are one word
+// of the row bitmap, ANDed into row_ok, and a warp whose word is 0 skips the threshold snapshot and the chunks.
 // ------------------------------------------------------------------------------------------
-template <bool I8>
+template <bool I8, bool SEL>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
     umma_qs_score_select_kernel(const __grid_constant__ CUtensorMap tmap_p,
                                 const __grid_constant__ CUtensorMap tmap_ph /* 32-column boxes, 64B swizzle */,
@@ -294,7 +300,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
     // ===================== passage producer =====================
     uint32_t stage = 0, phase = 0;
     int prod_it = 0;
-    for (int tile = a.tile_begin + pair; tile < a.tile_end; tile += npairs, ++prod_it) {
+    for (int ti = a.tile_begin + pair; ti < a.tile_end; ti += npairs, ++prod_it) {
+      const int tile = tile_at<SEL>(a.tile_list, ti);
       *prod_it_s = prod_it;       // progress mark for the L2 prefetch warp
       // shadow layout (common.cuh): this CTA's 128 rows are 4 consecutive 32-row tiles; K-block kb of
       // each is a contiguous 4 KB piece -> 4 TMA boxes per 16 KB stage (rows past the end: zero fill)
@@ -354,7 +361,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
     // consecutive 32-row tiles x 12 K-blocks x 4 KB), paced by the producer's progress mark.
     constexpr int64_t kTileBytesCta = static_cast<int64_t>(kQsTileRowsCta) * kD * (I8 ? 1 : 2);     // 196,608 (bf16)
     int it_pf = 0;
-    for (int tile = a.tile_begin + pair; tile < a.tile_end; tile += npairs, ++it_pf) {
+    for (int ti = a.tile_begin + pair; ti < a.tile_end; ti += npairs, ++it_pf) {
+      const int tile = tile_at<SEL>(a.tile_list, ti);
       while (it_pf > *prod_it_s + a.prefetch) __nanosleep(400);
       if (it_pf <= *prod_it_s) continue;          // the producer is already there
       const int64_t off = (static_cast<int64_t>(tile) * 2 + cta_rank) * kTileBytesCta;
@@ -439,7 +447,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
       }
     };
     int it = 0;
-    for (int tile = a.tile_begin + pair; tile < a.tile_end; tile += npairs, ++it) {
+    for (int ti = a.tile_begin + pair; ti < a.tile_end; ti += npairs, ++it) {
+      const int tile = tile_at<SEL>(a.tile_list, ti);
       const uint32_t as = it & 1, aph = (it >> 1) & 1;
       mbar_wait(bar_tfull + 8 * as, aph, a.err);
       tc_fence_after();
@@ -453,87 +462,94 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
         while (*tau_ready_s == 0 && clock64() - t0 < a.first_wait_cycles) __nanosleep(256);
       }
       const int64_t row64 = static_cast<int64_t>(tile) * kQsTileRows + cta_rank * kQsTileRowsCta + ew * 32 + lane;
-      const bool row_ok = row64 < a.n_rows;
+      bool row_ok = row64 < a.n_rows;
+      uint32_t sel_word = 0xffffffffu;
+      if constexpr (SEL) {
+        sel_word = __ldg(a.sel_bits + ((row64 - lane) >> 5));
+        row_ok = row_ok && ((sel_word >> lane) & 1u);
+      }
       const uint32_t row = static_cast<uint32_t>(row64);
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(ew * 32) << 16) + as * kQsAccStride;
       // int8: this warp's 32 rows are one shadow tile with one scale
       const float st = (I8 && row64 - lane < a.n_rows) ? __ldg(a.tscale + ((row64 - lane) >> 5)) : 0.f;
       int* thr_w = thr_s + (warp - 4) * 128;
-      if constexpr (I8) {
-        // this warp's query columns: 16 * half + 32 * i + j (i-th chunk, j < 16); thresholds only rise, so converting
-        // them once per tile (a snapshot) keeps every filter valid
-        const int n_own = 16 * ((a.n_cols - 16 * half + 31) / 32);
-        for (int x = lane; x < n_own; x += 32) {
-          const int col = 16 * half + 32 * (x >> 4) + (x & 15);
-          thr_w[x] = i8_threshold(*reinterpret_cast<volatile float*>(tau_s + col), __ldg(a.qscale + col), st);
-        }
-        __syncwarp();
-      }
-      for (int c0 = 16 * half; c0 < a.n_cols; c0 += 32) {
-        uint32_t v[16];
-        tmem_ld_x16(taddr + c0, v);
+      if (sel_word != 0u) {   // warp-uniform; always true without a filter
         if constexpr (I8) {
-          const int* thr = thr_w + 16 * ((c0 - 16 * half) >> 5);
-          int t[16];
-#pragma unroll
+          // this warp's query columns: 16 * half + 32 * i + j (i-th chunk, j < 16); thresholds only rise, so converting
+          // them once per tile (a snapshot) keeps every filter valid
+          const int n_own = 16 * ((a.n_cols - 16 * half + 31) / 32);
+          for (int x = lane; x < n_own; x += 32) {
+            const int col = 16 * half + 32 * (x >> 4) + (x & 15);
+            thr_w[x] = i8_threshold(*reinterpret_cast<volatile float*>(tau_s + col), __ldg(a.qscale + col), st);
+          }
+          __syncwarp();
+        }
+        for (int c0 = 16 * half; c0 < a.n_cols; c0 += 32) {
+          uint32_t v[16];
+          tmem_ld_x16(taddr + c0, v);
+          if constexpr (I8) {
+            const int* thr = thr_w + 16 * ((c0 - 16 * half) >> 5);
+            int t[16];
+  #pragma unroll
+            for (int u = 0; u < 4; ++u) {
+              const int4 f = *reinterpret_cast<const int4*>(thr + 4 * u);
+              t[4 * u] = f.x; t[4 * u + 1] = f.y; t[4 * u + 2] = f.z; t[4 * u + 3] = f.w;
+            }
+            tmem_ld_wait();
+            const bool mine = row_ok && any_ge16_s32(v, t);
+            if (__any_sync(0xffffffffu, mine)) {
+              uint32_t m = 0;
+  #pragma unroll
+              for (int j = 0; j < 16; ++j) m |= (static_cast<int>(v[j]) >= t[j]) ? (1u << j) : 0u;
+              if (!row_ok) m = 0;
+              uint32_t any = __reduce_or_sync(0xffffffffu, m);
+              if (__popc(any) > 4) {
+                // busy chunk (loose thresholds early in a pass): unrolled, v[] stays in registers
+  #pragma unroll
+                for (int j = 0; j < 16; ++j)
+                  if ((any >> j) & 1u)
+                    hit(c0 + j, (m >> j) & 1u, __float_as_uint(i8_score(static_cast<int>(v[j]), __ldg(a.qscale + c0 + j), st)), row);
+                any = 0;
+              }
+              while (any) {   // the recorded score is formed on this rare path only
+                const int j = __ffs(any) - 1;
+                any &= any - 1;
+                const uint32_t acc = tmem_ld_x1(taddr + c0 + j);
+                tmem_ld_wait();
+                hit(c0 + j, (m >> j) & 1u, __float_as_uint(i8_score(static_cast<int>(acc), __ldg(a.qscale + c0 + j), st)), row);
+              }
+            }
+            continue;
+          }
+          // thresholds of these 16 queries (volatile: the refresher warp rewrites them while we run)
+          float t[16];
+  #pragma unroll
           for (int u = 0; u < 4; ++u) {
-            const int4 f = *reinterpret_cast<const int4*>(thr + 4 * u);
+            const float4 f = lds_volatile_f4(tau_s_addr + 4u * static_cast<uint32_t>(c0 + 4 * u));
             t[4 * u] = f.x; t[4 * u + 1] = f.y; t[4 * u + 2] = f.z; t[4 * u + 3] = f.w;
           }
           tmem_ld_wait();
-          const bool mine = row_ok && any_ge16_s32(v, t);
+          const bool mine = row_ok && any_ge16(v, t);
           if (__any_sync(0xffffffffu, mine)) {
+            // some row of this warp reached a threshold of this chunk: now build the per-lane hit mask
             uint32_t m = 0;
-#pragma unroll
-            for (int j = 0; j < 16; ++j) m |= (static_cast<int>(v[j]) >= t[j]) ? (1u << j) : 0u;
+  #pragma unroll
+            for (int j = 0; j < 16; ++j) m |= (__uint_as_float(v[j]) >= t[j]) ? (1u << j) : 0u;
             if (!row_ok) m = 0;
             uint32_t any = __reduce_or_sync(0xffffffffu, m);
             if (__popc(any) > 4) {
-              // busy chunk (loose thresholds early in a pass): unrolled, v[] stays in registers
-#pragma unroll
+              // busy chunk (loose thresholds, the first tiles of a pass): unrolled, v[] stays in registers
+  #pragma unroll
               for (int j = 0; j < 16; ++j)
-                if ((any >> j) & 1u)
-                  hit(c0 + j, (m >> j) & 1u, __float_as_uint(i8_score(static_cast<int>(v[j]), __ldg(a.qscale + c0 + j), st)), row);
-              any = 0;
-            }
-            while (any) {   // the recorded score is formed on this rare path only
-              const int j = __ffs(any) - 1;
-              any &= any - 1;
-              const uint32_t acc = tmem_ld_x1(taddr + c0 + j);
-              tmem_ld_wait();
-              hit(c0 + j, (m >> j) & 1u, __float_as_uint(i8_score(static_cast<int>(acc), __ldg(a.qscale + c0 + j), st)), row);
-            }
-          }
-          continue;
-        }
-        // thresholds of these 16 queries (volatile: the refresher warp rewrites them while we run)
-        float t[16];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const float4 f = lds_volatile_f4(tau_s_addr + 4u * static_cast<uint32_t>(c0 + 4 * u));
-          t[4 * u] = f.x; t[4 * u + 1] = f.y; t[4 * u + 2] = f.z; t[4 * u + 3] = f.w;
-        }
-        tmem_ld_wait();
-        const bool mine = row_ok && any_ge16(v, t);
-        if (__any_sync(0xffffffffu, mine)) {
-          // some row of this warp reached a threshold of this chunk: now build the per-lane hit mask
-          uint32_t m = 0;
-#pragma unroll
-          for (int j = 0; j < 16; ++j) m |= (__uint_as_float(v[j]) >= t[j]) ? (1u << j) : 0u;
-          if (!row_ok) m = 0;
-          uint32_t any = __reduce_or_sync(0xffffffffu, m);
-          if (__popc(any) > 4) {
-            // busy chunk (loose thresholds, the first tiles of a pass): unrolled, v[] stays in registers
-#pragma unroll
-            for (int j = 0; j < 16; ++j)
-              if ((any >> j) & 1u) hit(c0 + j, (m >> j) & 1u, v[j], row);
-          } else {
-            while (any) {   // rare: re-read the flagged column from TMEM (a dynamic index would spill v[])
-              const int j = __ffs(any) - 1;
-              any &= any - 1;
-              const uint32_t bits = tmem_ld_x1(taddr + c0 + j);
-              tmem_ld_wait();
-              hit(c0 + j, (m >> j) & 1u, bits, row);
+                if ((any >> j) & 1u) hit(c0 + j, (m >> j) & 1u, v[j], row);
+            } else {
+              while (any) {   // rare: re-read the flagged column from TMEM (a dynamic index would spill v[])
+                const int j = __ffs(any) - 1;
+                any &= any - 1;
+                const uint32_t bits = tmem_ld_x1(taddr + c0 + j);
+                tmem_ld_wait();
+                hit(c0 + j, (m >> j) & 1u, bits, row);
+              }
             }
           }
         }

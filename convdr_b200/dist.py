@@ -155,16 +155,23 @@ class ShardedFlatIP:
             self._key = key
         return self._send, self._recv
 
-    def search(self, q: torch.Tensor, k: int):
+    def search(self, q: torch.Tensor, k: int, params=None):
         """q: [nq, 768] float32 on this rank's device (replicated).  Returns the global (D, I).
+        `params=SearchParameters(sel=...)` filters: every rank builds the selector on its own rows from the same
+        description (the labels are global), so the merged result is the filtered global top-k.
 
         GPU ranks: local search, ONE all-gather of the packed (score, id) lists and the merge kernel
         are queued on the engine's stream without a host round trip in between; the host waits once,
         at the end (where the overflow flags of the local search are checked)."""
         nq = q.shape[0]
         if self.index is not None and q.is_cuda:
-            return self._search_cuda(q, k)
-        D, I = self._local_search(q, k)
+            return self._search_cuda(q, k, params)
+        if params is not None:
+            if self.index is None:
+                raise NotImplementedError("filtered search needs a rank that owns a FlatIPIndex")
+            D, I = self.index.search_device(q, k, params=params)
+        else:
+            D, I = self._local_search(q, k)
         if self.world == 1:
             return D, I
         send, recv = self._buffers(nq, k, D.device)
@@ -175,7 +182,7 @@ class ShardedFlatIP:
         Ig = torch.stack([recv[w, self._i_off:].view(torch.int64).view(nq, k) for w in range(self.world)])
         return self._merge(Dg, Ig)
 
-    def search_async(self, q: torch.Tensor, k: int, D: torch.Tensor, I: torch.Tensor) -> None:
+    def search_async(self, q: torch.Tensor, k: int, D: torch.Tensor, I: torch.Tensor, params=None) -> None:
         """Queue local search -> all-gather -> merge on the engine's stream and return; `finish()`
         settles.  q, D, I (CUDA tensors) must stay alive; consecutive calls reuse the exchange buffers
         in stream order."""
@@ -185,17 +192,17 @@ class ShardedFlatIP:
             self._ext = torch.cuda.ExternalStream(idx.stream_ptr(0), device=q.device)
         self._ext.wait_stream(torch.cuda.current_stream(q.device))     # q may have been produced there
         if self.world == 1:
-            idx.search_device_async(q, k, D, I)
+            idx.search_device_async(q, k, D, I, params=params)
             return
         if getattr(self, "_peer", False) and nq * k <= self._peer_cap[0] * self._peer_cap[1] and nq <= self._peer_cap[0] \
                 and k <= self._peer_cap[1]:
-            idx.search_xchg_async(q, k, D, I)     # search -> NVLink push -> wait + merge, all engine kernels
+            idx.search_xchg_async(q, k, D, I, params=params)   # search -> NVLink push -> wait + merge, all engine kernels
             self._last_peer = True
             return
         self._last_peer = False
         send, recv = self._buffers(nq, k, q.device)
         with torch.cuda.stream(self._ext):
-            idx.search_device_async(q, k, self._Dl, self._Il)          # local top-k with global ids
+            idx.search_device_async(q, k, self._Dl, self._Il, params=params)   # local top-k with global ids
             dist.all_gather_into_tensor(recv.view(-1), send, group=self.group)  # the only exchange (NCCL)
             idx.merge_packed_device_async(recv, self.world, self._part, self._i_off, nq, k, D, I)
         self._last = (q, k, D, I)
@@ -206,13 +213,13 @@ class ShardedFlatIP:
         self.index.finish()
         return not (self.world > 1 and self.index.stat("merge_saw_overflow") > 0)
 
-    def _search_cuda(self, q: torch.Tensor, k: int):
+    def _search_cuda(self, q: torch.Tensor, k: int, params=None):
         nq = q.shape[0]
         idx = self.index
         D = torch.empty((nq, k), dtype=torch.float32, device=q.device)
         I = torch.empty((nq, k), dtype=torch.int64, device=q.device)
         q = q.contiguous()
-        self.search_async(q, k, D, I)
+        self.search_async(q, k, D, I, params)
         if self.world == 1:
             idx.finish()
             return D, I

@@ -8,6 +8,8 @@ Reference call sites (drivers/run_convdr_inference.py):
     faiss.GpuResourcesVector() / faiss.Int32Vector() .push_back  :360-364
     faiss.index_cpu_to_gpu_multiple(vres, vdev, cpu_index, co)   :365-367
     index.add / index.search / index.reset    :180, :182, :202
+Beyond the driver: filtered search, `index.search(x, k, params=SearchParameters(sel=IDSelector...(...)))`
+(selectors.py).
 
 Use it either as `import convdr_b200.faiss_compat as faiss` or by putting `convdr_b200/shim`
 on PYTHONPATH, which makes a plain `import faiss` resolve to this module (INTEGRATION.md).
@@ -17,6 +19,8 @@ CPU index behind `IndexFlatIP`.
 from __future__ import annotations
 
 from .index import FlatIPIndex, get_num_gpus  # noqa: F401  (get_num_gpus is part of the surface)
+from .selectors import (IDSelector, IDSelectorAnd, IDSelectorArray, IDSelectorBatch, IDSelectorBitmap,  # noqa: F401
+                        IDSelectorNot, IDSelectorOr, IDSelectorRange, IDSelectorXOr, SearchParameters)
 
 METRIC_INNER_PRODUCT = 0
 METRIC_L2 = 1

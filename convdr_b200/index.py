@@ -18,6 +18,7 @@ import numpy as np
 from . import _lib
 
 PATHS = {"auto": 0, "scan_f32": 1, "scan_exact": 2, "umma_bf16": 3}
+_SELECTOR_CACHE = 8   # compiled selectors kept per index (each holds a row bitmap per shard)
 DIM = 768
 MAX_K = 2048
 
@@ -37,6 +38,7 @@ class FlatIPIndex:
         self._devices = None if devices is None else [int(x) for x in devices]
         self._h = None
         self._options: dict[str, int] = {}
+        self._selectors: dict[int, tuple] = {}   # id(selector) -> (selector, index generation, b2f_selector handle)
         if self.d != DIM:
             raise RuntimeError(f"b2f supports d = {DIM} only (ConvDR hard-codes IndexFlatIP(768)), got {d}")
 
@@ -57,6 +59,9 @@ class FlatIPIndex:
 
     def close(self) -> None:
         if self._h is not None:
+            for _, _, hs in self._selectors.values():   # a selector goes before its index
+                _lib.load().b2f_selector_destroy(hs)
+            self._selectors.clear()
             _lib.load().b2f_destroy(self._h)
             self._h = None
 
@@ -93,8 +98,10 @@ class FlatIPIndex:
         h = self._ensure()
         _lib.check(_lib.load().b2f_add_with_ids(h, x.ctypes.data, ids.ctypes.data, x.shape[0]))
 
-    def search(self, x, k: int):
-        """D, I = index.search(x, k): exact top-k by inner product, sorted descending."""
+    def search(self, x, k: int, params=None):
+        """D, I = index.search(x, k, params=None): exact top-k by inner product, sorted descending.  With
+        `params=SearchParameters(sel=...)` only rows whose label the selector accepts can be returned; fewer than
+        k such rows pad with -FLT_MAX / -1, as faiss does."""
         x = self._as_rows(x, "x")
         k = int(k)
         assert k > 0, "k must be positive"
@@ -102,8 +109,48 @@ class FlatIPIndex:
         D = np.empty((nq, k), dtype=np.float32)
         I = np.empty((nq, k), dtype=np.int64)
         h = self._ensure()
-        _lib.check(_lib.load().b2f_search(h, x.ctypes.data, nq, k, D.ctypes.data, I.ctypes.data))
+        sel = self._selector(params)
+        if sel is None:
+            _lib.check(_lib.load().b2f_search(h, x.ctypes.data, nq, k, D.ctypes.data, I.ctypes.data))
+        else:
+            _lib.check(_lib.load().b2f_search_sel(h, sel, x.ctypes.data, nq, k, D.ctypes.data, I.ctypes.data))
         return D, I
+
+    # -- filtered search ---------------------------------------------------------------------------
+    def _selector(self, params):
+        """The compiled selector of `params` (None: no filter).  Built on the GPU the first time a selector object
+        is used with this index, and again after rows were added or the index was reset."""
+        sel = getattr(params, "sel", None) if params is not None else None
+        if sel is None:
+            return None
+        from .selectors import IDSelector
+        if not isinstance(sel, IDSelector):
+            raise TypeError("params.sel must be an IDSelector of convdr_b200.faiss_compat")
+        lib = _lib.load()
+        h = self._ensure()
+        gen = int(self.stat("generation"))
+        hit = self._selectors.get(id(sel))
+        if hit is not None and hit[0] is sel and hit[1] == gen:
+            return hit[2]
+        for key in [key for key, (s, g, _) in self._selectors.items() if g != gen or key == id(sel)]:
+            lib.b2f_selector_destroy(self._selectors.pop(key)[2])
+        while len(self._selectors) >= _SELECTOR_CACHE:
+            lib.b2f_selector_destroy(self._selectors.pop(next(iter(self._selectors)))[2])
+        kind, invert, imin, imax, ids, bitmap = sel._describe()
+        out = C.c_void_p()
+        _lib.check(lib.b2f_selector_create(
+            h, kind, int(invert), int(imin), int(imax), None if ids is None or ids.size == 0 else ids.ctypes.data,
+            0 if ids is None else ids.size, None if bitmap is None or bitmap.size == 0 else bitmap.ctypes.data,
+            0 if bitmap is None else bitmap.size, C.byref(out)))
+        self._selectors[id(sel)] = (sel, gen, out)
+        return out
+
+    def selected_count(self, sel) -> int:
+        """How many rows of the index the selector accepts (b2f_selector_count)."""
+        from .selectors import SearchParameters
+        out = C.c_int64()
+        _lib.check(_lib.load().b2f_selector_count(self._selector(SearchParameters(sel=sel)), C.byref(out)))
+        return int(out.value)
 
     def reconstruct_n(self, i0: int, ni: int, shard: int = 0) -> np.ndarray:
         """IndexFlat.reconstruct_n: stored rows [i0, i0+ni) of one shard, as float32 [ni, d]."""
@@ -173,16 +220,21 @@ class FlatIPIndex:
         _lib.check(_lib.load().b2f_add_synthetic(self._ensure(), int(shard), int(first_row), int(n), int(seed),
                                                  int(stream), float(norm), int(id_base)))
 
-    def search_device(self, q, k: int):
-        """Search with a CUDA torch tensor of queries; returns CUDA tensors (D, I).  Single shard."""
+    def search_device(self, q, k: int, params=None):
+        """Search with a CUDA torch tensor of queries; returns CUDA tensors (D, I).  Single shard.  `params` as
+        in `search`."""
         import torch
         assert q.is_cuda and q.dim() == 2 and q.shape[1] == self.d
         q = q.contiguous().to(torch.float32)
         nq = q.shape[0]
         D = torch.empty((nq, int(k)), dtype=torch.float32, device=q.device)
         I = torch.empty((nq, int(k)), dtype=torch.int64, device=q.device)
-        _lib.check(_lib.load().b2f_search_device(self._ensure(), q.data_ptr(), nq, int(k), D.data_ptr(),
-                                                 I.data_ptr()))
+        if self._selector(params) is None:
+            _lib.check(_lib.load().b2f_search_device(self._ensure(), q.data_ptr(), nq, int(k), D.data_ptr(),
+                                                     I.data_ptr()))
+        else:
+            self.search_device_async(q, k, D, I, params=params)
+            self.finish()
         return D, I
 
     def search_device_into(self, q, k: int, D, I) -> None:
@@ -190,11 +242,17 @@ class FlatIPIndex:
         _lib.check(_lib.load().b2f_search_device(self._ensure(), q.data_ptr(), q.shape[0], int(k), D.data_ptr(),
                                                  I.data_ptr()))
 
-    def search_device_async(self, q, k: int, D, I) -> None:
+    def search_device_async(self, q, k: int, D, I, params=None) -> None:
         """Enqueue only (b2f_search_device_async): q, D, I are CUDA tensors that must stay alive until
-        `finish()`; later work on the index stream may consume D / I without a host round trip."""
-        _lib.check(_lib.load().b2f_search_device_async(self._ensure(), q.data_ptr(), q.shape[0], int(k),
-                                                       D.data_ptr(), I.data_ptr()))
+        `finish()`; later work on the index stream may consume D / I without a host round trip.  `params` as in
+        `search`; searches with different selectors may be in flight together."""
+        sel = self._selector(params)
+        if sel is None:
+            _lib.check(_lib.load().b2f_search_device_async(self._ensure(), q.data_ptr(), q.shape[0], int(k),
+                                                           D.data_ptr(), I.data_ptr()))
+        else:
+            _lib.check(_lib.load().b2f_search_device_async_sel(self._ensure(), sel, q.data_ptr(), q.shape[0], int(k),
+                                                               D.data_ptr(), I.data_ptr()))
 
     def finish(self) -> None:
         """Wait for every search enqueued with `search_device_async` (re-running overflowed queries)."""
@@ -219,10 +277,12 @@ class FlatIPIndex:
         blob = b"".join(handles)
         _lib.check(_lib.load().b2f_xchg_connect(self._ensure(), blob))
 
-    def search_xchg_async(self, q, k: int, D, I, repush_only: bool = False) -> None:
-        """Collective: local search -> NVLink push of the packed part to every rank -> wait + merge."""
-        _lib.check(_lib.load().b2f_search_xchg_async(self._ensure(), q.data_ptr(), q.shape[0], int(k), D.data_ptr(),
-                                                     I.data_ptr(), 1 if repush_only else 0))
+    def search_xchg_async(self, q, k: int, D, I, repush_only: bool = False, params=None) -> None:
+        """Collective: local search -> NVLink push of the packed part to every rank -> wait + merge.  With
+        `params`, every rank filters its own rows with the same selector description."""
+        _lib.check(_lib.load().b2f_search_xchg_async_sel(self._ensure(), self._selector(params), q.data_ptr(),
+                                                         q.shape[0], int(k), D.data_ptr(), I.data_ptr(),
+                                                         1 if repush_only else 0))
 
     def search_xchg_host(self, x, k: int, D=None, I=None):
         """Collective end-to-end search with host buffers (b2f_search_xchg_host): numpy in, numpy out; pass

@@ -111,6 +111,33 @@ int b2f_add_synthetic(b2f_index* idx, int shard, int64_t first_row, int64_t n, u
 int b2f_search(b2f_index* idx, const float* q_host, int64_t nq, int k, float* D_host,
                int64_t* I_host);
 
+/* Filtered search: faiss index.search(x, k, params=faiss.SearchParameters(sel=...)).
+ * A selector is built once against one index and reused for many searches.  It is
+ * evaluated on the labels search returns (explicit ids, or the implicit positions):
+ *   B2F_SEL_RANGE   imin <= id < imax                            (IDSelectorRange)
+ *   B2F_SEL_BATCH   id in ids_host[0 .. n_ids), any order, duplicates allowed
+ *                                                                (IDSelectorBatch / IDSelectorArray)
+ *   B2F_SEL_BITMAP  (bitmap_host[id >> 3] >> (id & 7)) & 1; ids >= 8 n_bytes are not
+ *                   selected                                     (IDSelectorBitmap)
+ * invert != 0 selects the complement (IDSelectorNot).  Per shard the selector keeps a
+ * row bitmap and the lists of the row tiles that hold a selected row: a filtered search
+ * streams only those tiles and only selected rows can enter the results, which stay
+ * exact; fewer than k selected rows pad with D = -FLT_MAX, I = -1 like faiss.
+ * Adding rows or resetting the index makes a selector stale: searching with it then
+ * fails with B2F_ERR_INVALID.  Destroy a selector before its index;
+ * b2f_selector_destroy first settles the searches still in flight.
+ * A NULL selector in the *_sel entry points means no filter.                   */
+typedef struct b2f_selector b2f_selector;
+enum { B2F_SEL_RANGE = 1, B2F_SEL_BATCH = 2, B2F_SEL_BITMAP = 3 };
+int b2f_selector_create(b2f_index* idx, int kind, int invert, int64_t imin, int64_t imax,
+                        const int64_t* ids_host, int64_t n_ids, const uint8_t* bitmap_host,
+                        int64_t n_bytes, b2f_selector** out);
+/* Number of selected rows over all shards. */
+int b2f_selector_count(const b2f_selector* sel, int64_t* selected_out);
+void b2f_selector_destroy(b2f_selector* sel);
+int b2f_search_sel(b2f_index* idx, const b2f_selector* sel, const float* q_host, int64_t nq, int k,
+                   float* D_host, int64_t* I_host);
+
 /* Device-resident variant (single-shard indexes): q_dev / D_dev / I_dev live on
  * the shard's device; work is enqueued on the index stream (b2f_stream) and the
  * stream is synchronised before returning (the candidate-overflow flags are
@@ -130,6 +157,8 @@ int b2f_search_device(b2f_index* idx, const float* q_dev, int64_t nq, int k, flo
 int b2f_search_device_async(b2f_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev,
                             int64_t* I_dev);
 int b2f_search_finish(b2f_index* idx);
+int b2f_search_device_async_sel(b2f_index* idx, const b2f_selector* sel, const float* q_dev, int64_t nq,
+                                int k, float* D_dev, int64_t* I_dev);
 
 /* Merge `n_parts` per-shard results [n_parts, nq, k] (device memory, each part
  * sorted descending, padded with -FLT_MAX / -1) into the global top-k
@@ -180,6 +209,10 @@ int b2f_xchg_create(b2f_index* idx, int rank, int world, int64_t max_nq, int max
 int b2f_xchg_connect(b2f_index* idx, const void* handles);
 int b2f_search_xchg_async(b2f_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev,
                           int64_t* I_dev, int repush_only);
+/* Same collective, filtered: every rank passes a selector built from the same
+ * description on its own index.                                                */
+int b2f_search_xchg_async_sel(b2f_index* idx, const b2f_selector* sel, const float* q_dev, int64_t nq,
+                              int k, float* D_dev, int64_t* I_dev, int repush_only);
 /* The same collective as ONE host-buffer call (the end-to-end path of the
  * one-process-per-GPU layout): upload of q_host (straight from the caller's buffer
  * when it is page-locked), local search, push, wait + merge — whose result rows are
@@ -249,7 +282,8 @@ int b2f_set_option(b2f_index* idx, const char* key, int64_t value);
  * than the survivor buffer holds); "path", "passes", "qs_passes"; with "profile" on also "score_ms",
  * "score_launches", "score_rows" (scoring kernels: device time, launches, rows
  * streamed) and "select_ms" (refresh + final kernels); "shadow_format" (first shard: 0 none,
- * 1 bf16, 2 int8) and "shadow_rho" (AUTO: median 2 eps8 / sigma of the probe, 0 if not measured). */
+ * 1 bf16, 2 int8) and "shadow_rho" (AUTO: median 2 eps8 / sigma of the probe, 0 if not measured);
+ * "generation" (bumped by every add and reset: a selector built at another generation is stale). */
 int b2f_get_stat(const b2f_index* idx, const char* key, double* out);
 
 void b2f_destroy(b2f_index* idx);
