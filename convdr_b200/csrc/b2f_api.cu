@@ -620,6 +620,18 @@ int ensure_pin(Shard& S, size_t bytes) {
 //     s~ (i8_threshold), the recorded score fl(fl(acc) fl(sq st)) is within 2^-23 |s~| of it, and
 //     |s~| <= ||q^|| ||p^|| <= (||q|| + e_q)(P + E8): the term 2^-21 (||q|| + e_q)(P + E8) covers it 4x over.
 // Every factor is an upper bound and every operation rounds up; `scale` (margin_ppm) multiplies the result.
+// Outside the normal fp32 range (DESIGN.md section 4):
+//   - a product of bounds with a zero factor is an exactly-zero term (bound_mul): a zero bound means a zero vector,
+//     so 0 * inf must not turn the margin into NaN;
+//   - the relative bounds above assume normal arithmetic.  With subnormal values each fp32 rounding (scan FMA
+//     chain, tensor-core accumulation) may add up to 2^-126 of absolute error, a flushed tensor-core product less
+//     than 2^-126, and the recorded int8 score fl(acc) fl(sq st) less than 2^24 * 2^-150 + 2^-150 when the scale
+//     product is subnormal.  At most 768 products and 768 additions: < 1536 * 2^-126 < 2^-115, added in every mode;
+//   - a query whose margin or histogram top R is not finite (a norm bound overflowed) is flagged here and re-run
+//     by the exact engine, like an overflowed list; it is never filtered with a NaN threshold.
+__device__ __forceinline__ float bound_mul(float a, float b) { return (a == 0.f || b == 0.f) ? 0.f : __fmul_ru(a, b); }
+constexpr float kSubnormalAbs = 0x1p-115f;
+
 __global__ void pass_init_kernel(const float* __restrict__ qnorm, const float* __restrict__ qerr,
                                  const unsigned int* __restrict__ maxnorm2_bits, int mode, float scale, float u_scan,
                                  float* __restrict__ margin, int* __restrict__ cnt,
@@ -627,13 +639,15 @@ __global__ void pass_init_kernel(const float* __restrict__ qnorm, const float* _
                                  unsigned int* __restrict__ hist, uint32_t* __restrict__ hkey0, int* __restrict__ hshift,
                                  float* __restrict__ tau) {
   const int q = blockIdx.x;
+  bool finite = true;
   if (hist != nullptr) {
     // TS engine without a bootstrap launch: empty tightening histogram of 64 buckets per binade over
     // the eight binades below R = (1 + 2^-6) * ||q|| * max||p|| >= |any prefilter score of q|; tau = -inf.
     for (int b = threadIdx.x; b < kHistStride; b += blockDim.x) hist[static_cast<int64_t>(q) * kHistStride + b] = 0u;
     if (threadIdx.x == 0) {
-      const float R = __fmul_ru(__fmul_ru(qnorm[q], __fsqrt_ru(__uint_as_float(maxnorm2_bits[2]))), 1.015625f);
-      const uint32_t top = fkey(R) >> 17;
+      const float R = __fmul_ru(bound_mul(qnorm[q], __fsqrt_ru(__uint_as_float(maxnorm2_bits[2]))), 1.015625f);
+      finite = isfinite(R);
+      const uint32_t top = fkey(finite ? R : FLT_MAX) >> 17;
       hkey0[q] = (top >= static_cast<uint32_t>(kHistBuckets - 1) ? top - (kHistBuckets - 1) : 0u) << 17;
       hshift[q] = 17;
     }
@@ -645,30 +659,34 @@ __global__ void pass_init_kernel(const float* __restrict__ qnorm, const float* _
     // tensor engine: scores are taken against the CENTRED rows p - mu (constant shift q.mu per query), so its
     // bounds use Pc = max ||p - mu||; the fp32 scan reads the rows themselves: P = max ||p||
     const float P = __fsqrt_ru(__uint_as_float(maxnorm2_bits[mode == 1 ? 0 : 2]));
+    const float qn = qnorm[q], qe = qerr[q];
     float eps = 0.f;
     if (mode == 1) {
-      eps = __fmul_ru(__fmul_ru(qnorm[q], P), u_scan);
+      eps = bound_mul(bound_mul(qn, P), u_scan);
     } else if (mode == 3) {   // data-independent worst case (A/B reference for mode 2): bf16 round-to-nearest has
       // unit roundoff 2^-8, so E <= 2^-8 P, ||q^|| <= (1 + 2^-8) ||q||, e_q <= 2^-8 ||q||:
       // 2^-8 (1 + 2^-8) + 2^-8 + 1.1e-4 < 0.007954
-      eps = __fmul_ru(__fmul_ru(qnorm[q], P), 0.007954f);
+      eps = bound_mul(bound_mul(qn, P), 0.007954f);
     } else if (mode == 2) {
       const float E = __fsqrt_ru(__uint_as_float(maxnorm2_bits[1]));
-      const float a = __fmul_ru(__fmul_ru(qnorm[q], E), 1.00390625f);   // ||bf16(q)|| <= (1 + 2^-8) ||q||
-      const float b = __fmul_ru(qerr[q], P);
-      const float c = __fmul_ru(__fmul_ru(qnorm[q], P), 1.1e-4f);
+      const float a = bound_mul(bound_mul(qn, E), 1.00390625f);   // ||bf16(q)|| <= (1 + 2^-8) ||q||
+      const float b = bound_mul(qe, P);
+      const float c = bound_mul(bound_mul(qn, P), 1.1e-4f);
       eps = __fadd_ru(__fadd_ru(a, b), c);
     } else if (mode == 4) {
       const float E = __fsqrt_ru(__uint_as_float(maxnorm2_bits[1]));
-      const float qh = __fadd_ru(qnorm[q], qerr[q]);
-      const float a = __fmul_ru(qh, E);
-      const float b = __fmul_ru(qerr[q], P);
-      const float c = __fmul_ru(__fmul_ru(qh, __fadd_ru(P, E)), 4.76837158203125e-7f);   // 2^-21
+      const float qh = __fadd_ru(qn, qe);
+      const float a = bound_mul(qh, E);
+      const float b = bound_mul(qe, P);
+      const float c = bound_mul(bound_mul(qh, __fadd_ru(P, E)), 4.76837158203125e-7f);   // 2^-21
       eps = __fadd_ru(__fadd_ru(a, b), c);
     }
-    margin[q] = __fmul_ru(__fmul_ru(eps, 2.0f), scale);
+    if (mode != 0) eps = __fadd_ru(eps, kSubnormalAbs);
+    const float m = __fmul_ru(__fmul_ru(eps, 2.0f), scale);
+    const bool fallback = mode != 0 && !(finite && isfinite(m));
+    margin[q] = fallback ? FLT_MAX : m;
     cnt[q] = 0;
-    ovf[q] = 0;
+    ovf[q] = fallback ? 1 : 0;
   }
   if (cnt2 != nullptr)
     for (int p = threadIdx.x; p < max_pairs; p += blockDim.x) cnt2[q * max_pairs + p] = 0;

@@ -5,18 +5,45 @@
 
 namespace b2f {
 
-// Upper bound of a row norm^2 computed in fp32 (any summation order): inflate by 2^-12 so the
-// stored value is >= the true sum of squares.
-__device__ __forceinline__ float norm2_upper(float ss) { return ss * (1.0f + 2.44140625e-4f); }
+// Sums of squares are accumulated in fp64 and turned into an fp32 upper bound here, so that every bound is one
+// for all finite inputs (DESIGN.md section 4): the square of an fp32 value is exact and normal in fp64 (the
+// smallest, (2^-149)^2 = 2^-298, is far above 2^-1022), so only the additions round.  768 non-negative terms in any
+// order are then within 767 * 2^-53 < 2^-43 of their sum, relative; 1 + 2^-40 covers that and the conversion
+// rounds up.  The result is 0 only for an all-zero vector and +inf above FLT_MAX.  An fp32 sum instead flushes
+// squares below 2^-149 to zero and overflows at FLT_MAX, where no relative factor can recover the bound.
+__device__ __forceinline__ float sumsq_upper(double s) { return __double2float_ru(__dmul_ru(s, 1.0 + 0x1p-40)); }
+__device__ __forceinline__ double sumsq4(double acc, float4 v) {
+  acc = fma(static_cast<double>(v.x), static_cast<double>(v.x), acc);
+  acc = fma(static_cast<double>(v.y), static_cast<double>(v.y), acc);
+  acc = fma(static_cast<double>(v.z), static_cast<double>(v.z), acc);
+  return fma(static_cast<double>(v.w), static_cast<double>(v.w), acc);
+}
+// An fp32 operation (subtraction, fma) rounds to within 2^-24 of its result, or to within 2^-150 of it when the
+// result is subnormal.  Over 768 components the absolute part is at most sqrt(768) * 2^-150 < 2^-145 in norm.
+constexpr float kSubnormalNorm = 0x1p-145f;
+// Upper bound of ||(x - mu) - shadow|| from the computed error vector e~ (sum of its squares s) and the computed
+// centred row d (norm bound cn): the error components may carry one rounding each (rel_round: the fma of the
+// int8 shadow) and d carries the rounding of the fp32 subtraction x - mu, each 2^-24 relative + 2^-145 in norm.
+__device__ __forceinline__ float shadow_err_upper(double s, float cn, bool rel_round) {
+  float e = __fsqrt_ru(sumsq_upper(s));
+  if (rel_round) e = __fadd_ru(__fmul_ru(e, 1.0000001f), kSubnormalNorm);
+  return __fadd_ru(__fadd_ru(e, __fmul_ru(cn, 6.0e-8f)), kSubnormalNorm);
+}
+// Upper bound of ||x - mu||^2 from cn >= ||d||, d = fl32(x - mu): ||x - mu|| <= (1 + 2^-24) ||d|| + 2^-145.
+__device__ __forceinline__ float centred_norm2_upper(float cn) {
+  const float c = __fadd_ru(__fmul_ru(cn, 1.0000001f), kSubnormalNorm);
+  return __fmul_ru(c, c);
+}
 
-// Squared bf16 rounding error of four components: (x - bf16_rn(x)) is exact in fp32 (the difference
-// of two floats within half a bf16 ulp of each other), so only the squares and the sum round.
-__device__ __forceinline__ float bf16_err2(float4 v) {
-  const float dx = v.x - __bfloat162float(__float2bfloat16_rn(v.x));
-  const float dy = v.y - __bfloat162float(__float2bfloat16_rn(v.y));
-  const float dz = v.z - __bfloat162float(__float2bfloat16_rn(v.z));
-  const float dw = v.w - __bfloat162float(__float2bfloat16_rn(v.w));
-  return dx * dx + dy * dy + dz * dz + dw * dw;
+// acc + the squared bf16 rounding error of four components: (x - bf16_rn(x)) is exact in fp32 (the difference
+// of two floats within half a bf16 ulp of each other), and so are its squares in fp64.
+__device__ __forceinline__ double bf16_err2(double acc, float4 v) {
+  float4 d;
+  d.x = v.x - __bfloat162float(__float2bfloat16_rn(v.x));
+  d.y = v.y - __bfloat162float(__float2bfloat16_rn(v.y));
+  d.z = v.z - __bfloat162float(__float2bfloat16_rn(v.z));
+  d.w = v.w - __bfloat162float(__float2bfloat16_rn(v.w));
+  return sumsq4(acc, d);
 }
 
 __device__ __forceinline__ uint2 pack_bf16x4(float4 v) {
@@ -76,15 +103,15 @@ __global__ void __launch_bounds__(256) convert_rows_kernel(const float* __restri
   float wmax = 0.f, emax = 0.f, cmax = 0.f;
   for (int64_t r = warp; r < n_rows; r += nwarps) {
     const float4* src = reinterpret_cast<const float4*>(x32 + (row0 + r) * kD);
-    float ss = 0.f, es = 0.f, cs = 0.f;
+    double ss = 0.0, es = 0.0, cs = 0.0;
 #pragma unroll
     for (int i = 0; i < kF4PerLane; ++i) {
       const float4 v = ldg_stream_f4(src + lane + 32 * i);
-      ss += v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w;
+      ss = sumsq4(ss, v);
       float4 d;
       d.x = __fsub_rn(v.x, m4[i].x); d.y = __fsub_rn(v.y, m4[i].y); d.z = __fsub_rn(v.z, m4[i].z); d.w = __fsub_rn(v.w, m4[i].w);
-      cs += d.x * d.x + d.y * d.y + d.z * d.z + d.w * d.w;
-      es += bf16_err2(d);
+      cs = sumsq4(cs, d);
+      es = bf16_err2(es, d);
       if (x16) *reinterpret_cast<uint2*>(x16 + shadow_index(row0 + r, 4 * (lane + 32 * i))) = pack_bf16x4(d);
     }
 #pragma unroll
@@ -93,11 +120,11 @@ __global__ void __launch_bounds__(256) convert_rows_kernel(const float* __restri
       es += __shfl_xor_sync(0xffffffffu, es, s);
       cs += __shfl_xor_sync(0xffffffffu, cs, s);
     }
-    const float cn = __fsqrt_ru(norm2_upper(cs));                         // >= ||d||
-    const float e = __fadd_ru(__fsqrt_ru(norm2_upper(es)), __fmul_ru(cn, 6.0e-8f));   // + 2^-24 ||d|| (subtraction rounding)
-    wmax = fmaxf(wmax, norm2_upper(ss));
+    const float cn = __fsqrt_ru(sumsq_upper(cs));                        // >= ||d||
+    const float e = shadow_err_upper(es, cn, false);
+    wmax = fmaxf(wmax, sumsq_upper(ss));
     emax = fmaxf(emax, __fmul_ru(e, e));
-    cmax = fmaxf(cmax, __fmul_ru(__fmul_ru(cn, cn), 1.0000002f));         // ||x - mu|| <= (1 + 2^-24) ||d||
+    cmax = fmaxf(cmax, centred_norm2_upper(cn));
   }
   if (lane == 0 && wmax > 0.f) atomicMax(maxnorm2_bits, __float_as_uint(wmax));
   if (lane == 0 && emax > 0.f) atomicMax(maxnorm2_bits + 1, __float_as_uint(emax));
@@ -108,13 +135,22 @@ __global__ void __launch_bounds__(256) convert_rows_kernel(const float* __restri
 __device__ __forceinline__ int quant8(float v, float inv) {
   return max(-127, min(127, __float2int_rn(v * inv)));
 }
+// fl(v - sq * q8(v)) per component (one fma rounding each) and the upper bound of ||q - sq q8|| built from the
+// sum of their squares: 2^-24 relative + 2^-145 in norm for the fma roundings.
+__device__ __forceinline__ float4 i8_residual(float4 v, float sq, float inv) {
+  return make_float4(fmaf(-sq, static_cast<float>(quant8(v.x, inv)), v.x), fmaf(-sq, static_cast<float>(quant8(v.y, inv)), v.y),
+                     fmaf(-sq, static_cast<float>(quant8(v.z, inv)), v.z), fmaf(-sq, static_cast<float>(quant8(v.w, inv)), v.w));
+}
+__device__ __forceinline__ float i8_query_err_upper(double s) {
+  return __fadd_ru(__fmul_ru(__fsqrt_ru(sumsq_upper(s)), 1.0000001f), kSubnormalNorm);
+}
 
 // int8 shadow (DESIGN.md section 4): one warp per 32-row tile of rows [tile_row0, row0 + n_rows), where tile_row0 is
 // row0 rounded down to the tile — a tile that an earlier add left partly filled is re-quantised with the scale of
 // all its rows.  Pass 1: st = max|d| / 127 over the tile (d = fl32(x - mu)); pass 2: p8 = rint(d / st), the
 // K-block-major int8 row (common.cuh shadow8_index) and the same three bounds as convert_rows_kernel, with slot [1]
-// an upper bound of max ||(x - mu) - st * p8||^2: fma(-st, p8, d) rounds the exact difference once (relative 2^-24,
-// covered by norm2_upper), plus 2^-24 ||d|| for the rounding of the fp32 subtraction.  Any p8 is valid — the bound
+// an upper bound of max ||(x - mu) - st * p8||^2: fma(-st, p8, d) rounds the exact difference once, plus the
+// rounding of the fp32 subtraction (shadow_err_upper).  Any p8 is valid — the bound
 // measures the error that was made.  x8 == nullptr: bounds only (used by the format choice).
 __global__ void __launch_bounds__(256) convert_rows_i8_kernel(const float* __restrict__ x32, int8_t* __restrict__ x8,
                                                               float* __restrict__ tscale, int64_t row0, int64_t n_rows,
@@ -148,18 +184,17 @@ __global__ void __launch_bounds__(256) convert_rows_i8_kernel(const float* __res
     if (x8 && lane == 0) tscale[t] = st;
     for (int64_t r = r0; r < r1; ++r) {
       const float4* src = reinterpret_cast<const float4*>(x32 + r * kD);
-      float ss = 0.f, es = 0.f, cs = 0.f;
+      double ss = 0.0, es = 0.0, cs = 0.0;
 #pragma unroll
       for (int i = 0; i < kF4PerLane; ++i) {
         const float4 v = __ldg(src + lane + 32 * i);
-        ss += v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w;
+        ss = sumsq4(ss, v);
         float4 d;
         d.x = __fsub_rn(v.x, m4[i].x); d.y = __fsub_rn(v.y, m4[i].y); d.z = __fsub_rn(v.z, m4[i].z); d.w = __fsub_rn(v.w, m4[i].w);
-        cs += d.x * d.x + d.y * d.y + d.z * d.z + d.w * d.w;
+        cs = sumsq4(cs, d);
         const int a = quant8(d.x, inv), b = quant8(d.y, inv), c = quant8(d.z, inv), e = quant8(d.w, inv);
-        const float ex = fmaf(-st, static_cast<float>(a), d.x), ey = fmaf(-st, static_cast<float>(b), d.y);
-        const float ez = fmaf(-st, static_cast<float>(c), d.z), ew = fmaf(-st, static_cast<float>(e), d.w);
-        es += ex * ex + ey * ey + ez * ez + ew * ew;
+        es = sumsq4(es, make_float4(fmaf(-st, static_cast<float>(a), d.x), fmaf(-st, static_cast<float>(b), d.y),
+                                    fmaf(-st, static_cast<float>(c), d.z), fmaf(-st, static_cast<float>(e), d.w)));
         if (x8) {
           const uint32_t packed = (static_cast<uint32_t>(a) & 0xffu) | ((static_cast<uint32_t>(b) & 0xffu) << 8) |
                                   ((static_cast<uint32_t>(c) & 0xffu) << 16) | (static_cast<uint32_t>(e) << 24);
@@ -172,11 +207,11 @@ __global__ void __launch_bounds__(256) convert_rows_i8_kernel(const float* __res
         es += __shfl_xor_sync(0xffffffffu, es, s);
         cs += __shfl_xor_sync(0xffffffffu, cs, s);
       }
-      const float cn = __fsqrt_ru(norm2_upper(cs));
-      const float e = __fadd_ru(__fsqrt_ru(norm2_upper(es)), __fmul_ru(cn, 6.0e-8f));
-      wmax = fmaxf(wmax, norm2_upper(ss));
+      const float cn = __fsqrt_ru(sumsq_upper(cs));
+      const float e = shadow_err_upper(es, cn, true);
+      wmax = fmaxf(wmax, sumsq_upper(ss));
       emax = fmaxf(emax, __fmul_ru(e, e));
-      cmax = fmaxf(cmax, __fmul_ru(__fmul_ru(cn, cn), 1.0000002f));
+      cmax = fmaxf(cmax, centred_norm2_upper(cn));
     }
   }
   if (lane == 0 && wmax > 0.f) atomicMax(maxnorm2_bits, __float_as_uint(wmax));
@@ -195,12 +230,13 @@ __global__ void __launch_bounds__(256) shadow_probe_kernel(const float* __restri
   const int j = blockIdx.y;
   const float4* q4 = reinterpret_cast<const float4*>(x32 + (m * j / 64) * kD);
   float4 q[kF4PerLane];
-  float amax = 0.f, qq = 0.f;
+  float amax = 0.f;
+  double qq = 0.0;
 #pragma unroll
   for (int i = 0; i < kF4PerLane; ++i) {
     q[i] = __ldg(q4 + lane + 32 * i);
     amax = fmaxf(amax, fmaxf(fmaxf(fabsf(q[i].x), fabsf(q[i].y)), fmaxf(fabsf(q[i].z), fabsf(q[i].w))));
-    qq += q[i].x * q[i].x + q[i].y * q[i].y + q[i].z * q[i].z + q[i].w * q[i].w;
+    qq = sumsq4(qq, q[i]);
   }
   double s1 = 0.0, s2 = 0.0;
   for (int r = blockIdx.x * 8 + w; r < n_s; r += gridDim.x * 8) {
@@ -225,23 +261,18 @@ __global__ void __launch_bounds__(256) shadow_probe_kernel(const float* __restri
 #pragma unroll
     for (int s = 16; s >= 1; s >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, s));
     const float sq = amax / 127.f, inv = amax > 0.f ? 127.f / amax : 0.f;
-    float es = 0.f;
+    double es = 0.0;
 #pragma unroll
-    for (int i = 0; i < kF4PerLane; ++i) {
-      const float ex = fmaf(-sq, static_cast<float>(quant8(q[i].x, inv)), q[i].x);
-      const float ey = fmaf(-sq, static_cast<float>(quant8(q[i].y, inv)), q[i].y);
-      const float ez = fmaf(-sq, static_cast<float>(quant8(q[i].z, inv)), q[i].z);
-      const float ew = fmaf(-sq, static_cast<float>(quant8(q[i].w, inv)), q[i].w);
-      es += ex * ex + ey * ey + ez * ez + ew * ew;
-    }
+    for (int i = 0; i < kF4PerLane; ++i)
+      es = sumsq4(es, i8_residual(q[i], sq, inv));
 #pragma unroll
     for (int s = 16; s >= 1; s >>= 1) {
       es += __shfl_xor_sync(0xffffffffu, es, s);
       qq += __shfl_xor_sync(0xffffffffu, qq, s);
     }
     if (lane == 0) {
-      qstat[2 * j] = __fsqrt_ru(norm2_upper(qq));
-      qstat[2 * j + 1] = __fsqrt_ru(norm2_upper(es));
+      qstat[2 * j] = __fsqrt_ru(sumsq_upper(qq));
+      qstat[2 * j + 1] = amax > 0.f ? i8_query_err_upper(es) : 0.f;
     }
   }
 }
@@ -330,12 +361,12 @@ __global__ void __launch_bounds__(128) prep_queries_kernel(const float* __restri
     return;
   }
   const float4* src = reinterpret_cast<const float4*>(q32 + static_cast<int64_t>(q) * kD);
-  float ss = 0.f, es = 0.f;
+  double ss = 0.0, es = 0.0;
 #pragma unroll
   for (int i = 0; i < kF4PerLane; ++i) {
     float4 v = __ldg(src + lane + 32 * i);
-    ss += v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w;
-    es += bf16_err2(v);
+    ss = sumsq4(ss, v);
+    es = bf16_err2(es, v);
     dst[lane + 32 * i] = pack_bf16x4(v);
   }
 #pragma unroll
@@ -344,8 +375,8 @@ __global__ void __launch_bounds__(128) prep_queries_kernel(const float* __restri
     es += __shfl_xor_sync(0xffffffffu, es, s);
   }
   if (lane == 0) {
-    qnorm[q] = __fsqrt_ru(norm2_upper(ss));
-    qerr[q] = __fsqrt_ru(norm2_upper(es));
+    qnorm[q] = __fsqrt_ru(sumsq_upper(ss));
+    qerr[q] = __fsqrt_ru(sumsq_upper(es));   // the bf16 errors are exact: only their sum rounds
   }
 }
 
@@ -366,12 +397,13 @@ __global__ void __launch_bounds__(128) prep_queries_i8_kernel(const float* __res
   }
   const float4* src = reinterpret_cast<const float4*>(q32 + static_cast<int64_t>(q) * kD);
   float4 v[kF4PerLane];
-  float amax = 0.f, ss = 0.f, es = 0.f;
+  float amax = 0.f;
+  double ss = 0.0, es = 0.0;
 #pragma unroll
   for (int i = 0; i < kF4PerLane; ++i) {
     v[i] = __ldg(src + lane + 32 * i);
     amax = fmaxf(amax, fmaxf(fmaxf(fabsf(v[i].x), fabsf(v[i].y)), fmaxf(fabsf(v[i].z), fabsf(v[i].w))));
-    ss += v[i].x * v[i].x + v[i].y * v[i].y + v[i].z * v[i].z + v[i].w * v[i].w;
+    ss = sumsq4(ss, v[i]);
   }
 #pragma unroll
   for (int s = 16; s >= 1; s >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, s));
@@ -379,9 +411,7 @@ __global__ void __launch_bounds__(128) prep_queries_i8_kernel(const float* __res
 #pragma unroll
   for (int i = 0; i < kF4PerLane; ++i) {
     const int a = quant8(v[i].x, inv), b = quant8(v[i].y, inv), c = quant8(v[i].z, inv), e = quant8(v[i].w, inv);
-    const float ex = fmaf(-sq, static_cast<float>(a), v[i].x), ey = fmaf(-sq, static_cast<float>(b), v[i].y);
-    const float ez = fmaf(-sq, static_cast<float>(c), v[i].z), ew = fmaf(-sq, static_cast<float>(e), v[i].w);
-    es += ex * ex + ey * ey + ez * ez + ew * ew;
+    es = sumsq4(es, i8_residual(v[i], sq, inv));
     dst[lane + 32 * i] = (static_cast<uint32_t>(a) & 0xffu) | ((static_cast<uint32_t>(b) & 0xffu) << 8) |
                          ((static_cast<uint32_t>(c) & 0xffu) << 16) | (static_cast<uint32_t>(e) << 24);
   }
@@ -392,8 +422,8 @@ __global__ void __launch_bounds__(128) prep_queries_i8_kernel(const float* __res
   }
   if (lane == 0) {
     qscale[q] = sq;
-    qnorm[q] = __fsqrt_ru(norm2_upper(ss));
-    qerr[q] = __fsqrt_ru(norm2_upper(es));
+    qnorm[q] = __fsqrt_ru(sumsq_upper(ss));
+    qerr[q] = amax > 0.f ? i8_query_err_upper(es) : 0.f;   // a zero query is coded exactly
   }
 }
 
