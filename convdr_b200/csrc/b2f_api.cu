@@ -185,7 +185,7 @@ struct Shard {
   float* x32 = nullptr;
   __nv_bfloat16* x16 = nullptr;     // bf16 shadow (format 1)
   int8_t* x8 = nullptr;              // int8 shadow (format 2) ...
-  float* tscale = nullptr;           // ... and its per-32-row-tile scales
+  float4* tscale = nullptr;          // ... and its per-32-row-tile scales {st, RD(1/st), RU(1/st), 0} (i8_tile_scale)
   int fmt = 0;                       // shadow format of the buffers: 0 none / not chosen yet, 1 bf16, 2 int8
   double rho = 0;                    // AUTO: median 2 eps8 / sigma of the probe (0: not measured)
   int64_t n = 0, cap = 0;
@@ -377,7 +377,7 @@ int ensure_capacity(b2f_index* idx, Shard& S, int64_t need) {
   float* n32 = nullptr;
   __nv_bfloat16* n16 = nullptr;
   int8_t* n8 = nullptr;
-  float* nts = nullptr;
+  float4* nts = nullptr;
   int64_t* nid = nullptr;
   B2F_TRY(dev_alloc(&n32, static_cast<size_t>(ncap) * kD));
   // the shadow in the shard's format; under AUTO an empty shard has none yet (ingest_rows allocates it once the
@@ -397,7 +397,7 @@ int ensure_capacity(b2f_index* idx, Shard& S, int64_t need) {
                              cudaMemcpyDeviceToDevice, S.stream));  // tiles are stored in row order
     if (n8 && S.x8) {
       CU_TRY(cudaMemcpyAsync(n8, S.x8, static_cast<size_t>(shadow_rows_padded(S.n)) * kD, cudaMemcpyDeviceToDevice, S.stream));
-      CU_TRY(cudaMemcpyAsync(nts, S.tscale, static_cast<size_t>(shadow_rows_padded(S.n) / kShadowTileRows) * 4,
+      CU_TRY(cudaMemcpyAsync(nts, S.tscale, static_cast<size_t>(shadow_rows_padded(S.n) / kShadowTileRows) * sizeof(float4),
                              cudaMemcpyDeviceToDevice, S.stream));
     }
     if (nid && S.idmap)
@@ -616,8 +616,8 @@ int ensure_pin(Shard& S, size_t bytes) {
 //     core sums the 768 code products exactly in int32, so s~ = q^ . p^ exactly and
 //       |s~ - s| <= |q^ . (p^ - p)| + |(q^ - q) . p| <= (||q|| + e_q) E8 + e_q P,
 //     with E8 = max ||p - p^|| (slot [1] of an int8 shard, kept at add time), e_q = ||q - q^||, ||q^|| <= ||q|| + e_q.
-//     No accumulation term.  What is compared and recorded are fp32 images of s~: the threshold test is exact on
-//     s~ (i8_threshold), the recorded score fl(fl(acc) fl(sq st)) is within 2^-23 |s~| of it, and
+//     No accumulation term.  What is compared and recorded are fp32 images of s~: the threshold test never rejects
+//     a row with s~ >= tau (i8_threshold), the recorded score fl(fl(acc) fl(sq st)) is within 2^-23 |s~| of s~, and
 //     |s~| <= ||q^|| ||p^|| <= (||q|| + e_q)(P + E8): the term 2^-21 (||q|| + e_q)(P + E8) covers it 4x over.
 // Every factor is an upper bound and every operation rounds up; `scale` (margin_ppm) multiplies the result.
 // Outside the normal fp32 range (DESIGN.md section 4):

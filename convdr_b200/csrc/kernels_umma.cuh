@@ -100,7 +100,7 @@ struct UmmaArgs {
   const uint32_t* hkey0;      // [nq] key of the bootstrap's k-th best approximate score (0xffffffff: none yet)
   const int* hshift;          // [nq] log2(keys per bucket)
   const float* qscale;        // int8 shadow: [nq] query scales sq (q16 then points at the int8 codes)
-  const float* tscale;        // int8 shadow: [row tiles of 32] tile scales st
+  const float4* tscale;       // int8 shadow: [row tiles of 32] tile scales {st, RD(1/st), RU(1/st), 0}
   // Filtered search (SEL instances only): the launch walks tile_list[tile_begin .. tile_end) (pair tiles that hold
   // at least one selected row) instead of the tiles themselves; sel_bits is the shard's row bitmap (bit r & 31 of
   // word r >> 5: row r is selected).
@@ -411,7 +411,8 @@ __device__ __forceinline__ bool any_ge32_s32(const uint32_t* v, int tau) {
 // I8: int8 shadow and queries (kind::i8, s32 accumulators).  A 32-row tile is 6 K-blocks of 128 bytes, walked in 2
 // stages of 3 K-blocks (12 KB boxes, 18 of them in the ring); the queries take 192 TMEM columns (4 codes per
 // column, so a K-step of 32 codes is still 8 columns).  Each epilogue thread's 32 rows are one shadow tile: its
-// float threshold becomes ONE integer threshold per tile (i8_threshold), the compare chain stays one instruction
+// float threshold becomes ONE integer threshold per tile (i8_threshold: one product of the thread's tau / sq and
+// the tile's reciprocal scale), the compare chain stays one instruction
 // per score, and the float score is only formed for a hit.
 // SEL: filtered search.  The roles walk the listed tiles only; the epilogue ANDs the row bitmap word of its 32 rows
 // into the hit mask (and stores empty records for unselected rows in the dense phase), so only selected rows are
@@ -579,6 +580,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
     };
     const uint32_t tempty_leader = mapa_u32(bar_tempty, 0);
     const float sq = I8 ? a.qscale[q_ok ? q : 0] : 0.f;
+    float u = I8 ? i8_tau_over_sq(tau, sq) : 0.f;   // query factor of the integer threshold, redone when tau rises
     int it = 0;
     for (int ti = a.tile_begin + pair; ti < a.tile_end; ti += npairs, ++it) {
       const int tile = tile_at<SEL>(a.tile_list, ti);
@@ -595,6 +597,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
       if (live) tau_new = *tau_g;            // issued before the wait: the L2 latency hides behind it
       mbar_wait(bar_tfull + 8 * as, aph, a.err);
       tc_fence_after();
+      if (I8 && tau_new > tau) u = i8_tau_over_sq(tau_new, sq);
       tau = fmaxf(tau, tau_new);             // thresholds only rise
       constexpr int kHalfRows = kTileRows / 2;   // 32: this thread's rows of the tile
       uint32_t v[kHalfRows];
@@ -607,7 +610,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
       if constexpr (SEL) sel_word = __ldg(a.sel_bits + (row0 >> 5));
       if constexpr (I8) {
         // one integer threshold for this (query, shadow tile); scores as floats only where they are stored
-        const float st = n_valid > 0 ? __ldg(a.tscale + (row0 >> 5)) : 0.f;
+        const float4 ts = n_valid > 0 ? __ldg(a.tscale + (row0 >> 5)) : make_float4(0.f, INFINITY, INFINITY, 0.f);
+        const float st = ts.x;
         if (a.dense) {
           if (q_ok && n_mine + kHalfRows <= a.cap_p) {
             uint64_t* dst = my_list + n_mine;
@@ -621,7 +625,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
           }
           n_mine += kHalfRows;
         } else {
-          const int T = i8_threshold(tau, sq, st);
+          const int T = i8_threshold(u, ts);
           if (__any_sync(0xffffffffu, any_ge32_s32(v, T))) {
             uint32_t m = 0;
 #pragma unroll

@@ -41,7 +41,7 @@ constexpr int kQsSmemLimit = 232448;
 constexpr int kQsThreads = 416;                  // 4 service warps + 8 epilogue warps (two per TMEM lane quarter) + refresher
 constexpr int kQsEpiWarps = 8;
 constexpr int kQsEpiWarpsI8Scratch = 8 * 128 * 4;   // [8 epilogue warps][<= 128 query columns] int thresholds
-constexpr int kQsTailBytesI8 = kQsTailBytes + kQsEpiWarpsI8Scratch;   // int8 shadow: tail + that scratch
+constexpr int kQsTailBytesI8 = kQsTailBytes + kQsEpiWarpsI8Scratch + kQsMaxCols * 4;   // int8: tail + that scratch + u_s
 constexpr int kQsRefresherWarp = 12;             // the highest warp id: the scheduler prefers it over the epilogue
                                                  // warps of its quarter, so thresholds never wait behind appends
 
@@ -75,7 +75,7 @@ struct UmmaQsArgs {
   int dense_quarters;         // first tile of a CTA: lane quarters [0, dense_quarters) pass unfiltered
   int first_wait_cycles;      // the other quarters wait this long at most for every threshold to exist (0: no wait)
   const float* qscale;        // int8 shadow: [n_cols] query scales sq (0 for padded columns)
-  const float* tscale;        // int8 shadow: [row tiles of 32] tile scales st
+  const float4* tscale;       // int8 shadow: [row tiles of 32] tile scales {st, RD(1/st), RU(1/st), 0}
   // Filtered search (SEL instances only): the launch walks tile_list[tile_begin .. tile_end) (pair tiles of 256 rows
   // that hold at least one selected row); sel_bits is the shard's row bitmap (bit r & 31 of word r >> 5: row r).
   const uint32_t* sel_bits;
@@ -207,9 +207,10 @@ __device__ __forceinline__ bool any_ge16_s32(const uint32_t (&v)[16], const int 
 //                   CTA's shared-memory copy of all thresholds
 // I8: int8 shadow and queries (kind::i8, s32 accumulators, 6 K-blocks of 128 bytes; the byte geometry of every
 // stage, box and K-step is the bf16 one).  The epilogue compares the raw int32 accumulators with integer
-// thresholds: once per tile the warp's lanes convert the float thresholds of its query columns for the tile scale
-// (one 32-row shadow tile per warp) into a per-warp shared-memory scratch, which every lane reads per 16-query
-// chunk with 4 LDS.128 — the same cost as the float thresholds of the bf16 path.
+// thresholds (i8_threshold): the refresher keeps u = RD(tau / sq) of every query in shared memory next to tau, and
+// once per tile, before the accumulator is ready, the warp's lanes multiply the u of its query columns by the
+// reciprocal tile scale (one 32-row shadow tile per warp; no division) into a per-warp shared-memory scratch, which
+// every lane reads per 16-query chunk with 4 LDS.128 — the same cost as the float thresholds of the bf16 path.
 // SEL: filtered search.  Every role walks the listed tiles only (tile_at); an epilogue warp's 32 rows are one word
 // of the row bitmap, ANDed into row_ok, and a warp whose word is 0 skips the threshold snapshot and the chunks.
 // ------------------------------------------------------------------------------------------
@@ -250,6 +251,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
   uint32_t* hkey0_s = reinterpret_cast<uint32_t*>(tail_ptr + 512 + 2048);  // [kQsMaxCols]
   const uint32_t tau_s_addr = tail + 512;
   int* thr_s = reinterpret_cast<int*>(tail_ptr + kQsTailBytes);          // int8: [kQsEpiWarps][128] integer thresholds
+  float* u_s = reinterpret_cast<float*>(tail_ptr + kQsTailBytes + kQsEpiWarpsI8Scratch);   // int8: [kQsMaxCols] tau / sq
   constexpr int NKB = I8 ? kShadow8KBlocks : kNumKBlocks;                 // K-blocks of 128 bytes per row
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -287,6 +289,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
   if (threadIdx.x == 0) { *epi_done_s = 0; *tau_ready_s = 0; *prod_it_s = 0; }
   for (int i = threadIdx.x; i < kQsMaxCols; i += kQsThreads) {
     tau_s[i] = (i < a.nq) ? a.tau[i] : INFINITY;     // padded query columns never hit
+    if constexpr (I8) u_s[i] = (i < a.nq) ? i8_tau_over_sq(tau_s[i], __ldg(a.qscale + i)) : INFINITY;
     cnt_s[i] = 0;
     hkey0_s[i] = (i < a.nq) ? a.hkey0[i] : 0xffffffffu;
   }
@@ -446,10 +449,35 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
         }
       }
     };
+    // int8: this warp's query columns are 16 * half + 32 * i + j (i-th chunk, j < 16); their integer thresholds for
+    // the warp's shadow tile (one scale: the warp's 32 rows are one shadow tile) go to the warp's scratch.  Thresholds
+    // only rise, so a snapshot taken before the accumulator is ready keeps every filter valid.
+    auto snap_thresholds = [&](float4 ts, int* thr_w) {
+      const int n_own = 16 * ((a.n_cols - 16 * half + 31) / 32);
+      for (int x = lane; x < n_own; x += 32) {
+        const int col = 16 * half + 32 * (x >> 4) + (x & 15);
+        thr_w[x] = i8_threshold(*reinterpret_cast<volatile float*>(u_s + col), ts);
+      }
+      __syncwarp();
+    };
     int it = 0;
     for (int ti = a.tile_begin + pair; ti < a.tile_end; ti += npairs, ++it) {
       const int tile = tile_at<SEL>(a.tile_list, ti);
       const uint32_t as = it & 1, aph = (it >> 1) & 1;
+      const int64_t row64 = static_cast<int64_t>(tile) * kQsTileRows + cta_rank * kQsTileRowsCta + ew * 32 + lane;
+      bool row_ok = row64 < a.n_rows;
+      uint32_t sel_word = 0xffffffffu;
+      if constexpr (SEL) {
+        sel_word = __ldg(a.sel_bits + ((row64 - lane) >> 5));
+        row_ok = row_ok && ((sel_word >> lane) & 1u);
+      }
+      const uint32_t row = static_cast<uint32_t>(row64);
+      const float4 ts = (I8 && row64 - lane < a.n_rows) ? __ldg(a.tscale + ((row64 - lane) >> 5))
+                                                         : make_float4(0.f, INFINITY, INFINITY, 0.f);
+      const float st = ts.x;
+      int* thr_w = thr_s + (warp - 4) * 128;
+      // the conversion overlaps the MMA of this tile; the first tile converts after the wait for the first thresholds
+      if (I8 && it > 0 && sel_word != 0u) snap_thresholds(ts, thr_w);
       mbar_wait(bar_tfull + 8 * as, aph, a.err);
       tc_fence_after();
       if (it == 0 && ew >= a.dense_quarters && a.first_wait_cycles > 0) {
@@ -461,29 +489,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
         const long long t0 = clock64();
         while (*tau_ready_s == 0 && clock64() - t0 < a.first_wait_cycles) __nanosleep(256);
       }
-      const int64_t row64 = static_cast<int64_t>(tile) * kQsTileRows + cta_rank * kQsTileRowsCta + ew * 32 + lane;
-      bool row_ok = row64 < a.n_rows;
-      uint32_t sel_word = 0xffffffffu;
-      if constexpr (SEL) {
-        sel_word = __ldg(a.sel_bits + ((row64 - lane) >> 5));
-        row_ok = row_ok && ((sel_word >> lane) & 1u);
-      }
-      const uint32_t row = static_cast<uint32_t>(row64);
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(ew * 32) << 16) + as * kQsAccStride;
-      // int8: this warp's 32 rows are one shadow tile with one scale
-      const float st = (I8 && row64 - lane < a.n_rows) ? __ldg(a.tscale + ((row64 - lane) >> 5)) : 0.f;
-      int* thr_w = thr_s + (warp - 4) * 128;
       if (sel_word != 0u) {   // warp-uniform; always true without a filter
-        if constexpr (I8) {
-          // this warp's query columns: 16 * half + 32 * i + j (i-th chunk, j < 16); thresholds only rise, so converting
-          // them once per tile (a snapshot) keeps every filter valid
-          const int n_own = 16 * ((a.n_cols - 16 * half + 31) / 32);
-          for (int x = lane; x < n_own; x += 32) {
-            const int col = 16 * half + 32 * (x >> 4) + (x & 15);
-            thr_w[x] = i8_threshold(*reinterpret_cast<volatile float*>(tau_s + col), __ldg(a.qscale + col), st);
-          }
-          __syncwarp();
-        }
+        if (I8 && it == 0) snap_thresholds(ts, thr_w);
         for (int c0 = 16 * half; c0 < a.n_cols; c0 += 32) {
           uint32_t v[16];
           tmem_ld_x16(taddr + c0, v);
@@ -627,7 +635,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
       bool all_finite = true;
       for (int i = lane; i < a.nq; i += 32) {
         const float t = *reinterpret_cast<volatile float*>(a.tau + i);
-        if (t > tau_s[i]) *reinterpret_cast<volatile float*>(tau_s + i) = t;
+        if (t > tau_s[i]) {
+          *reinterpret_cast<volatile float*>(tau_s + i) = t;
+          // int8: the query factor of the integer thresholds; the divisions stay off the epilogue warps
+          if constexpr (I8) *reinterpret_cast<volatile float*>(u_s + i) = i8_tau_over_sq(t, __ldg(a.qscale + i));
+        }
         all_finite = all_finite && (t > -INFINITY);
       }
       if (__all_sync(0xffffffffu, all_finite) && lane == 0) *tau_ready_s = 1;

@@ -141,6 +141,11 @@ __device__ __forceinline__ float4 i8_residual(float4 v, float sq, float inv) {
   return make_float4(fmaf(-sq, static_cast<float>(quant8(v.x, inv)), v.x), fmaf(-sq, static_cast<float>(quant8(v.y, inv)), v.y),
                      fmaf(-sq, static_cast<float>(quant8(v.z, inv)), v.z), fmaf(-sq, static_cast<float>(quant8(v.w, inv)), v.w));
 }
+// Entry of the int8 shard's per-tile scale array: {st, RD(1/st), RU(1/st), 0}; the reciprocals are the tile
+// factors of the integer threshold (i8_threshold).
+__device__ __forceinline__ float4 i8_tile_scale(float st) {
+  return make_float4(st, __frcp_rd(st), __frcp_ru(st), 0.f);
+}
 __device__ __forceinline__ float i8_query_err_upper(double s) {
   return __fadd_ru(__fmul_ru(__fsqrt_ru(sumsq_upper(s)), 1.0000001f), kSubnormalNorm);
 }
@@ -153,7 +158,7 @@ __device__ __forceinline__ float i8_query_err_upper(double s) {
 // rounding of the fp32 subtraction (shadow_err_upper).  Any p8 is valid — the bound
 // measures the error that was made.  x8 == nullptr: bounds only (used by the format choice).
 __global__ void __launch_bounds__(256) convert_rows_i8_kernel(const float* __restrict__ x32, int8_t* __restrict__ x8,
-                                                              float* __restrict__ tscale, int64_t row0, int64_t n_rows,
+                                                              float4* __restrict__ tscale, int64_t row0, int64_t n_rows,
                                                               unsigned int* __restrict__ maxnorm2_bits,
                                                               const float* __restrict__ mu) {
   const int lane = threadIdx.x & 31;
@@ -181,7 +186,7 @@ __global__ void __launch_bounds__(256) convert_rows_i8_kernel(const float* __res
     for (int s = 16; s >= 1; s >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, s));
     const float st = amax / 127.f;
     const float inv = amax > 0.f ? 127.f / amax : 0.f;
-    if (x8 && lane == 0) tscale[t] = st;
+    if (x8 && lane == 0) tscale[t] = i8_tile_scale(st);
     for (int64_t r = r0; r < r1; ++r) {
       const float4* src = reinterpret_cast<const float4*>(x32 + r * kD);
       double ss = 0.0, es = 0.0, cs = 0.0;
@@ -427,17 +432,23 @@ __global__ void __launch_bounds__(128) prep_queries_i8_kernel(const float* __res
   }
 }
 
-// Integer threshold of the int8 tensor engine.  A prefilter score is s~ = acc * c with acc the exact int32 dot
-// product of the codes and c = sq * st (real product of the query and tile scales).  Returns T with
-// "acc * c >= tau  =>  acc >= T" for every integer acc: T = floor of a value <= tau / c (c rounded towards the side
-// that makes the quotient smaller for the sign of tau, the division rounded down); -inf and NaN pass everything.
-__device__ __forceinline__ int i8_threshold(float tau, float sq, float st) {
-  if (!(tau > -INFINITY)) return INT_MIN;
-  const float c = tau >= 0.f ? __fmul_ru(sq, st) : __fmul_rd(sq, st);
-  if (c == 0.f) return tau > 0.f ? INT_MAX : INT_MIN;   // tau > 0: c is exactly 0, every score is 0 < tau
-  const float x = __fdiv_rd(tau, c);
+// Integer threshold of the int8 tensor engine (DESIGN.md section 4).  A prefilter score is s~ = acc * sq * st with
+// acc the exact int32 dot product of the codes, sq the query scale and st the tile scale.  The threshold T satisfies
+// "acc * sq * st >= tau  =>  acc >= T" for every integer acc, and is formed from two factors so that the per-tile
+// step needs no division:
+//   per query (on a threshold change):  u = RD(tau / sq)                               (i8_tau_over_sq)
+//   per tile (at ingest):               r_lo = RD(1 / st), r_hi = RU(1 / st)            (i8_tile_scale)
+//   per (query, tile):                  x = RD(u * (u >= 0 ? r_lo : r_hi)),  T = floor(x), saturated; NaN -> INT_MIN
+// u <= tau/sq and r_lo <= 1/st <= r_hi, so x <= tau / (sq st) in every sign case, and acc >= tau/(sq st) >= x gives
+// acc >= floor(x).  The zero and infinite cases are what the IEEE operations give: st = 0 -> r = +inf (x = +-inf, or
+// NaN for u = 0: every row passes, and every score of a zero tile is 0); sq = 0 -> u = +-inf for tau != 0 (NaN for
+// tau = 0); tau = -inf -> u = -inf; a padded query column (tau = +inf, sq = 0) -> u = +inf; a subnormal st whose
+// reciprocal overflows -> r_lo = FLT_MAX, r_hi = +inf.  Saturation: |acc| <= 768 * 127^2 < 2^24.
+__device__ __forceinline__ float i8_tau_over_sq(float tau, float sq) { return __fdiv_rd(tau, sq); }
+__device__ __forceinline__ int i8_threshold(float u, float4 ts) {
+  const float x = __fmul_rd(u, u >= 0.f ? ts.y : ts.z);
   if (x >= 2147483520.f) return INT_MAX;
-  if (x < -2147483520.f) return INT_MIN;
+  if (!(x >= -2147483520.f)) return INT_MIN;   // and NaN
   return static_cast<int>(floorf(x));
 }
 // The score recorded for a hit: fl(fl(acc) * fl(sq * st)); |acc| <= 768 * 127^2 < 2^24, so fl(acc) is exact and the
