@@ -140,10 +140,11 @@ struct Workspace {
   int64_t out_cap = 0;
   float* D = nullptr;
   int64_t* I = nullptr;
-  // merge staging (shard 0 only)
-  int64_t parts_cap = 0;
-  float* Dp = nullptr;
-  int64_t* Ip = nullptr;
+  // merge staging (shard 0 only): the parts [G][nq][k] of a multi-shard search, one area per pending slot (a
+  // search owns its slot's parts until it is settled: a re-run shard's part is merged again then)
+  int64_t parts_cap[kMaxPending] = {};
+  float* Dp[kMaxPending] = {};
+  int64_t* Ip[kMaxPending] = {};
   // fallback staging
   float* fbq = nullptr;   // [kScanMaxQ, 768]
   float* fbD = nullptr;   // [kScanMaxQ, B2F_MAX_K]
@@ -1156,13 +1157,14 @@ int finish_search(b2f_index* idx, Shard& S, const float* q_d, int64_t nq, int k,
   cudaStream_t s = S.stream;
   for (size_t b0 = 0; b0 < bad.size(); b0 += kScanMaxQ) {
     const int nb = static_cast<int>(std::min<size_t>(kScanMaxQ, bad.size() - b0));
-    for (int i = 0; i < nb; ++i)
+    for (int i = 0; i < nb; ++i)   // cudaMemcpyDefault: a multi-shard search re-runs from the first device's queries
       CU_TRY(cudaMemcpyAsync(W.fbq + static_cast<size_t>(i) * kD, q_d + bad[b0 + i] * kD, kD * 4,
-                             cudaMemcpyDeviceToDevice, s));
+                             cudaMemcpyDefault, s));
     B2F_TRY(enqueue_pass(idx, S, plan, W.fbq, nullptr, W.qnorm /*unused: exact*/, W.qerr, nb, k, W.fbD, W.fbI, k, nullptr,
                          nullptr, sel));
     for (int i = 0; i < nb; ++i) {
       // cudaMemcpyDefault: D_d / I_d may be mapped pinned host memory (b2f_search writes results there directly)
+      // or a part on the first device
       CU_TRY(cudaMemcpyAsync(D_d + bad[b0 + i] * k, W.fbD + static_cast<size_t>(i) * k, sizeof(float) * k,
                              cudaMemcpyDefault, s));
       CU_TRY(cudaMemcpyAsync(I_d + bad[b0 + i] * k, W.fbI + static_cast<size_t>(i) * k, sizeof(int64_t) * k,
@@ -1197,6 +1199,103 @@ int run_on_shards(b2f_index* idx, const std::function<int(int)>& fn) {
   return rc;
 }
 
+// The parts area of one slot on the first device.  Only the search that takes the slot uses it, so it can grow while
+// the searches of lower slots are still in flight.
+int ensure_parts(Shard& S0, int slot, int64_t need) {
+  Workspace& W = S0.ws;
+  if (need <= W.parts_cap[slot]) return B2F_OK;
+  CU_TRY(cudaSetDevice(S0.dev));
+  dev_free(W.Dp[slot]); dev_free(W.Ip[slot]);
+  W.parts_cap[slot] = 0;
+  B2F_TRY(dev_alloc(&W.Dp[slot], static_cast<size_t>(need)));
+  B2F_TRY(dev_alloc(&W.Ip[slot], static_cast<size_t>(need)));
+  W.parts_cap[slot] = need;
+  return B2F_OK;
+}
+
+// Merge the parts of the slot's multi-shard search into D / I on shard 0's stream.
+int enqueue_merge(b2f_index* idx, int slot, int64_t nq, int k, float* D, int64_t* I, bool mark_pending) {
+  Shard& S0 = idx->shards[0];
+  const int G = static_cast<int>(idx->shards.size());
+  const int64_t per = nq * k;
+  CU_TRY(cudaSetDevice(S0.dev));
+  merge_kernel<<<static_cast<int>(nq), merge_threads(G, k), merge_stage_bytes(G, k), S0.stream>>>(
+      S0.ws.Dp[slot], S0.ws.Ip[slot], G, nq, k, D, I, per, per, nullptr, merge_mode(G, k), mark_pending ? 1 : 0);
+  CU_TRY(cudaGetLastError());
+  idx->stats.launches += 1;
+  return B2F_OK;
+}
+
+// Enqueue one search of a multi-shard index, without a host wait: every shard searches (each device enqueued by its
+// own host thread) into its part of the slot's parts area, and shard 0's stream merges the parts into D / I (on the
+// first device, or mapped host memory) once every part is there.
+//   q_host: host queries, uploaded by every shard.  Else q_dev, on the first device: shard 0 reads it in place, every
+//   other shard copies it once shard 0's stream has reached this call (the caller orders q's producer before that).
+//   A shard whose device can store into the first device's memory writes its part there directly (the last kernel of
+//   its search pushes the rows over NVLink); any other searches into its own buffer and copies the part over on its
+//   own stream, so that its next search cannot overwrite the buffer before the copy.
+//   mark_pending: a merged row whose part overflowed on some shard carries id -2 in its slot 0 until finish_sharded.
+int enqueue_sharded(b2f_index* idx, const b2f_selector* sel, const float* q_host, const float* q_dev, int64_t nq, int k,
+                    float* D, int64_t* I, int slot, bool mark_pending) {
+  const int G = static_cast<int>(idx->shards.size());
+  Shard& S0 = idx->shards[0];
+  const int64_t per = nq * k;
+  const size_t qbytes = static_cast<size_t>(nq) * kD * 4;
+  B2F_TRY(ensure_parts(S0, slot, per * G));
+  float* Dp = S0.ws.Dp[slot];
+  int64_t* Ip = S0.ws.Ip[slot];
+  if (q_dev) CU_TRY(cudaEventRecord(S0.ev, S0.stream));
+  B2F_TRY(run_on_shards(idx, [&](int g) -> int {
+    Shard& S = idx->shards[g];
+    CU_TRY(cudaSetDevice(S.dev));
+    B2F_TRY(ensure_query_ws(S, nq, k));
+    const float* q = S.ws.q32;
+    if (!q_dev) {
+      CU_TRY(cudaMemcpyAsync(S.ws.q32, q_host, qbytes, cudaMemcpyHostToDevice, S.stream));
+    } else if (g == 0) {
+      q = q_dev;
+    } else {
+      CU_TRY(cudaStreamWaitEvent(S.stream, S0.ev, 0));
+      if (S.dev == S0.dev) CU_TRY(cudaMemcpyAsync(S.ws.q32, q_dev, qbytes, cudaMemcpyDeviceToDevice, S.stream));
+      else CU_TRY(cudaMemcpyPeerAsync(S.ws.q32, S.dev, q_dev, S0.dev, qbytes, S.stream));
+    }
+    const bool direct = g == 0 || S.peer_to_first;
+    B2F_TRY(enqueue_search(idx, S, q, nq, k, direct ? Dp + per * g : S.ws.D, direct ? Ip + per * g : S.ws.I, slot,
+                           sel ? &sel->parts[g] : nullptr));
+    if (g == 0) return B2F_OK;
+    if (!direct) {
+      CU_TRY(cudaMemcpyPeerAsync(Dp + per * g, S0.dev, S.ws.D, S.dev, sizeof(float) * per, S.stream));
+      CU_TRY(cudaMemcpyPeerAsync(Ip + per * g, S0.dev, S.ws.I, S.dev, sizeof(int64_t) * per, S.stream));
+    }
+    CU_TRY(cudaEventRecord(S.ev, S.stream));
+    return B2F_OK;
+  }));
+  CU_TRY(cudaSetDevice(S0.dev));
+  for (int g = 1; g < G; ++g) CU_TRY(cudaStreamWaitEvent(S0.stream, idx->shards[g].ev, 0));
+  return enqueue_merge(idx, slot, nq, k, D, I, mark_pending);
+}
+
+// Settle a search of enqueue_sharded: every shard waits for its stream and re-runs its overflowed queries (reading
+// them from q0, on the first device) straight into its part of the slot; if any shard re-ran, the parts are merged
+// again.  One host wait per shard, and one more only after a re-run.
+int finish_sharded(b2f_index* idx, const b2f_selector* sel, const float* q0, int64_t nq, int k, float* D, int64_t* I,
+                   int slot) {
+  const int G = static_cast<int>(idx->shards.size());
+  Shard& S0 = idx->shards[0];
+  const int64_t per = nq * k;
+  bool any = false;
+  for (int g = 0; g < G; ++g) {
+    bool reran = false;
+    B2F_TRY(finish_search(idx, idx->shards[g], q0, nq, k, S0.ws.Dp[slot] + per * g, S0.ws.Ip[slot] + per * g, slot,
+                          &reran, sel ? &sel->parts[g] : nullptr));
+    any = any || reran;
+  }
+  if (!any) return B2F_OK;
+  B2F_TRY(enqueue_merge(idx, slot, nq, k, D, I, false));
+  CU_TRY(cudaStreamSynchronize(S0.stream));
+  return B2F_OK;
+}
+
 // Settle every search enqueued by b2f_search_device_async: wait for the stream, then re-run (on the
 // exact engine) the queries whose candidate lists overflowed.  Normally just the synchronisation.
 int settle_pending(b2f_index* idx) {
@@ -1205,18 +1304,25 @@ int settle_pending(b2f_index* idx) {
   Shard& S = idx->shards[0];
   std::vector<Pending> todo;
   todo.swap(idx->pending);
-  for (const Pending& p : todo)
-    B2F_TRY(finish_search(idx, S, p.q, p.nq, p.k, p.D, p.I, p.slot, nullptr, p.sel ? &p.sel->parts[0] : nullptr));
+  for (const Pending& p : todo) {
+    if (idx->shards.size() > 1)
+      B2F_TRY(finish_sharded(idx, p.sel, p.q, p.nq, p.k, p.D, p.I, p.slot));
+    else
+      B2F_TRY(finish_search(idx, S, p.q, p.nq, p.k, p.D, p.I, p.slot, nullptr, p.sel ? &p.sel->parts[0] : nullptr));
+  }
   return B2F_OK;
 }
 
-// True when enqueueing this search would (re)allocate a workspace that searches in flight still use.
-bool search_would_realloc(const b2f_index* idx, const Shard& S, int64_t nq, int k) {
-  const Workspace& W = S.ws;
-  if (nq > W.nq_cap || nq * k > W.out_cap || !W.fbq) return true;
-  if (S.n == 0) return false;
-  const PassPlan plan = make_plan(idx, S, resolve_path(idx, S, nq), k, nq);
-  return plan.qp > W.qp_cap || plan.C > W.C;
+// True when enqueueing this search would (re)allocate a workspace of some shard that searches in flight still use.
+bool search_would_realloc(const b2f_index* idx, int64_t nq, int k) {
+  for (const Shard& S : idx->shards) {
+    const Workspace& W = S.ws;
+    if (nq > W.nq_cap || nq * k > W.out_cap || !W.fbq) return true;
+    if (S.n == 0) continue;
+    const PassPlan plan = make_plan(idx, S, resolve_path(idx, S, nq), k, nq);
+    if (plan.qp > W.qp_cap || plan.C > W.C) return true;
+  }
+  return false;
 }
 
 // A selector filters only the index it was built for, and only while no row was added or removed since.
@@ -1350,7 +1456,8 @@ void b2f_destroy(b2f_index* idx) {
     dev_free(W.cand[0]); dev_free(W.cand[1]); dev_free(W.cnt); dev_free(W.tau); dev_free(W.tauP);
     dev_free(W.ovf); dev_free(W.margin); dev_free(W.err); dev_free(W.q32); dev_free(W.q16);
     dev_free(W.gath); dev_free(W.cnt2); dev_free(W.hist); dev_free(W.hkey0); dev_free(W.hshift);
-    dev_free(W.qnorm); dev_free(W.qerr); dev_free(W.D); dev_free(W.I); dev_free(W.Dp); dev_free(W.Ip);
+    dev_free(W.qnorm); dev_free(W.qerr); dev_free(W.D); dev_free(W.I);
+    for (int s = 0; s < kMaxPending; ++s) { dev_free(W.Dp[s]); dev_free(W.Ip[s]); }
     dev_free(W.fbq); dev_free(W.fbD); dev_free(W.fbI);
     if (W.ovf_host) cudaFreeHost(W.ovf_host);
     if (W.pin) cudaFreeHost(W.pin);
@@ -1519,12 +1626,15 @@ int b2f_reset(b2f_index* idx) {
 
 int b2f_search_device(b2f_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev) {
   B2F_TRY(check_args_search(idx, q_dev, nq, k, D_dev, I_dev));
-  if (idx->shards.size() != 1) return fail(B2F_ERR_INVALID, "b2f_search_device needs a single-shard index");
   if (nq == 0) return B2F_OK;
   B2F_TRY(settle_pending(idx));
   reset_stats(idx);
   Shard& S = idx->shards[0];
   CU_TRY(cudaSetDevice(S.dev));
+  if (idx->shards.size() > 1) {
+    B2F_TRY(enqueue_sharded(idx, nullptr, nullptr, q_dev, nq, k, D_dev, I_dev, 0, false));
+    return finish_sharded(idx, nullptr, q_dev, nq, k, D_dev, I_dev, 0);
+  }
   B2F_TRY(ensure_query_ws(S, nq, k));
   B2F_TRY(enqueue_search(idx, S, q_dev, nq, k, D_dev, I_dev));
   B2F_TRY(finish_search(idx, S, q_dev, nq, k, D_dev, I_dev));
@@ -1539,15 +1649,18 @@ int b2f_search_device_async_sel(b2f_index* idx, const b2f_selector* sel, const f
                                 float* D_dev, int64_t* I_dev) {
   B2F_TRY(check_args_search(idx, q_dev, nq, k, D_dev, I_dev));
   B2F_TRY(check_selector(idx, sel));
-  if (idx->shards.size() != 1) return fail(B2F_ERR_INVALID, "b2f_search_device_async needs a single-shard index");
   if (nq == 0) return B2F_OK;
   Shard& S = idx->shards[0];
   CU_TRY(cudaSetDevice(S.dev));
-  if (static_cast<int>(idx->pending.size()) >= kMaxPending || search_would_realloc(idx, S, nq, k))
+  if (static_cast<int>(idx->pending.size()) >= kMaxPending || search_would_realloc(idx, nq, k))
     B2F_TRY(settle_pending(idx));
-  B2F_TRY(ensure_query_ws(S, nq, k));
   const int slot = static_cast<int>(idx->pending.size());
-  B2F_TRY(enqueue_search(idx, S, q_dev, nq, k, D_dev, I_dev, slot, sel ? &sel->parts[0] : nullptr));
+  if (idx->shards.size() > 1) {
+    B2F_TRY(enqueue_sharded(idx, sel, nullptr, q_dev, nq, k, D_dev, I_dev, slot, true));
+  } else {
+    B2F_TRY(ensure_query_ws(S, nq, k));
+    B2F_TRY(enqueue_search(idx, S, q_dev, nq, k, D_dev, I_dev, slot, sel ? &sel->parts[0] : nullptr));
+  }
   idx->pending.push_back(Pending{q_dev, nq, k, D_dev, I_dev, slot, sel});
   return B2F_OK;
 }
@@ -1572,7 +1685,7 @@ int b2f_merge_device(b2f_index* idx, const float* D_parts_dev, const int64_t* I_
   CU_TRY(cudaSetDevice(S.dev));
   const int msb = merge_stage_bytes(n_parts, k);
   merge_kernel<<<static_cast<int>(nq), merge_threads(n_parts, k), msb, S.stream>>>(D_parts_dev, I_parts_dev, n_parts, nq, k, D_dev, I_dev,
-                                                             nq * k, nq * k, nullptr, merge_mode(n_parts, k));
+                                                             nq * k, nq * k, nullptr, merge_mode(n_parts, k), 0);
   CU_TRY(cudaGetLastError());
   idx->stats.launches += 1;
   CU_TRY(cudaStreamSynchronize(S.stream));
@@ -1591,7 +1704,7 @@ int b2f_merge_packed_device_async(b2f_index* idx, const void* parts_dev, int n_p
   const int msb = merge_stage_bytes(n_parts, k);
   merge_kernel<<<static_cast<int>(nq), merge_threads(n_parts, k), msb, S.stream>>>(
       reinterpret_cast<const float*>(base), reinterpret_cast<const int64_t*>(base + i_offset_bytes), n_parts, nq, k,
-      D_dev, I_dev, part_bytes / 4, part_bytes / 8, idx->merge_flag_dev, merge_mode(n_parts, k));
+      D_dev, I_dev, part_bytes / 4, part_bytes / 8, idx->merge_flag_dev, merge_mode(n_parts, k), 0);
   CU_TRY(cudaGetLastError());
   idx->stats.launches += 1;
   return B2F_OK;
@@ -1768,50 +1881,17 @@ int b2f_search_sel(b2f_index* idx, const b2f_selector* sel, const float* q_host,
   char* out_base = pin + round_up(static_cast<int64_t>(qbytes), 64);
   float* outD = out_pinned ? D_host : reinterpret_cast<float*>(out_base);
   int64_t* outI = out_pinned ? I_host : reinterpret_cast<int64_t*>(out_base + d_off);
-  const int64_t per = nq * k;
-  if (G > 1) {   // gather area on the first device: parts [G][nq][k]
-    Workspace& W = S0.ws;
-    if (per * G > W.parts_cap) {
-      dev_free(W.Dp); dev_free(W.Ip);
-      B2F_TRY(dev_alloc(&W.Dp, static_cast<size_t>(per) * G));
-      B2F_TRY(dev_alloc(&W.Ip, static_cast<size_t>(per) * G));
-      W.parts_cap = per * G;
-    }
-  }
-  // Where shard g leaves its [nq,k] lists.  One shard: the host buffer itself.  Several: a shard whose device
-  // can store into the first device's memory writes its part of the gather area directly (the last kernel of
-  // the search pushes the rows over NVLink as it produces them); otherwise its own buffer + a peer copy below.
-  auto part_D = [&](int g) { return G == 1 ? outD : ((g == 0 || idx->shards[g].peer_to_first) ? S0.ws.Dp + per * g : idx->shards[g].ws.D); };
-  auto part_I = [&](int g) { return G == 1 ? outI : ((g == 0 || idx->shards[g].peer_to_first) ? S0.ws.Ip + per * g : idx->shards[g].ws.I); };
-  B2F_TRY(run_on_shards(idx, [&](int g) -> int {   // every device is enqueued by its own host thread
-    Shard& S = idx->shards[g];
-    CU_TRY(cudaSetDevice(S.dev));
-    B2F_TRY(ensure_query_ws(S, nq, k));
-    CU_TRY(cudaMemcpyAsync(S.ws.q32, q_src, qbytes, cudaMemcpyHostToDevice, S.stream));
-    return enqueue_search(idx, S, S.ws.q32, nq, k, part_D(g), part_I(g), 0, sel ? &sel->parts[g] : nullptr);
-  }));
   if (G == 1) {
+    B2F_TRY(ensure_query_ws(S0, nq, k));
+    CU_TRY(cudaMemcpyAsync(S0.ws.q32, q_src, qbytes, cudaMemcpyHostToDevice, S0.stream));
+    B2F_TRY(enqueue_search(idx, S0, S0.ws.q32, nq, k, outD, outI, 0, sel ? &sel->parts[0] : nullptr));
     // ONE synchronisation; only if a candidate list overflowed (rare) the affected queries are re-run,
     // their rows rewritten in place
     B2F_TRY(finish_search(idx, S0, S0.ws.q32, nq, k, outD, outI, 0, nullptr, sel ? &sel->parts[0] : nullptr));
   } else {
-    for (int g = 0; g < G; ++g) {
-      Shard& S = idx->shards[g];
-      B2F_TRY(finish_search(idx, S, S.ws.q32, nq, k, part_D(g), part_I(g), 0, nullptr, sel ? &sel->parts[g] : nullptr));
-    }
-    CU_TRY(cudaSetDevice(S0.dev));
-    Workspace& W = S0.ws;
-    for (int g = 1; g < G; ++g) {
-      Shard& S = idx->shards[g];
-      if (S.peer_to_first) continue;
-      CU_TRY(cudaMemcpyPeerAsync(W.Dp + per * g, S0.dev, S.ws.D, S.dev, sizeof(float) * per, S0.stream));
-      CU_TRY(cudaMemcpyPeerAsync(W.Ip + per * g, S0.dev, S.ws.I, S.dev, sizeof(int64_t) * per, S0.stream));
-    }
-    const int msb = merge_stage_bytes(G, k);
-    merge_kernel<<<static_cast<int>(nq), merge_threads(G, k), msb, S0.stream>>>(W.Dp, W.Ip, G, nq, k, outD, outI, per, per, nullptr, merge_mode(G, k));
-    CU_TRY(cudaGetLastError());
-    idx->stats.launches += 1;
-    CU_TRY(cudaStreamSynchronize(S0.stream));
+    // every device is enqueued by its own host thread; the merge stores the result rows into the output
+    B2F_TRY(enqueue_sharded(idx, sel, q_src, nullptr, nq, k, outD, outI, 0, false));
+    B2F_TRY(finish_sharded(idx, sel, S0.ws.q32, nq, k, outD, outI, 0));
   }
   if (!out_pinned) {
     std::memcpy(D_host, outD, sizeof(float) * nq * k);

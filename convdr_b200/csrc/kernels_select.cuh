@@ -717,6 +717,18 @@ __global__ void __launch_bounds__(kFinThreads, 2) finalize_kernel(
   }
 }
 
+// Marker mode of the merges (the asynchronous search of a multi-shard index): when some part's list overflowed
+// (id -2 in its slot 0, see finalize_kernel) the merged row is not final either, so it carries -2 in its slot 0 too,
+// exactly like the row of a single-shard search, until the re-run shard's parts are merged again.
+__device__ __forceinline__ void mark_pending_row(const int64_t* Ip, int G, int64_t q, int k, int64_t strideI,
+                                                 int64_t* __restrict__ I) {
+  for (int g = 0; g < G; ++g)
+    if (__ldcg(Ip + static_cast<int64_t>(g) * strideI + q * k) == -2) {
+      I[q * k] = -2;
+      return;
+    }
+}
+
 // Cross-shard merge: parts [G][nq][k] (each sorted by score desc, padded with id = -1) -> [nq][k].
 // Rank-by-counting: an element's output position is its position in its own list plus, for every
 // other list, the number of elements that precede it; ties go to the earlier part, then the earlier
@@ -734,7 +746,8 @@ __global__ void __launch_bounds__(kFinThreads, 2) finalize_kernel(
 // per record (measured 41 -> 18 us per launch at G = 8, k = 100; two lists stay on rank-by-counting: 7 vs 8 us).
 __device__ __forceinline__ void merge_sort_body(const float* Dp, const int64_t* Ip, int G, int64_t q, int k,
                                                 float* __restrict__ D, int64_t* __restrict__ I, int64_t strideD,
-                                                int64_t strideI, int* saw_overflow, unsigned char* stage_smem) {
+                                                int64_t strideI, int* saw_overflow, int mark_pending,
+                                                unsigned char* stage_smem) {
   uint64_t* keys = reinterpret_cast<uint64_t*>(stage_smem);
   const int E = G * k;
   int P2 = 32;
@@ -778,12 +791,13 @@ __device__ __forceinline__ void merge_sort_body(const float* Dp, const int64_t* 
     D[q * k + i] = sc;
     I[q * k + i] = id;
   }
+  if (mark_pending && threadIdx.x == 0) mark_pending_row(Ip, G, q, k, strideI, I);   // after this thread's slot-0 store
 }
 
 __device__ __forceinline__ void merge_body(const float* Dp, const int64_t* Ip, int G, int64_t q,
                                            int k, float* __restrict__ D, int64_t* __restrict__ I,
                                            int64_t strideD, int64_t strideI, int* saw_overflow, int* total_valid_s,
-                                           int staged, unsigned char* stage_smem) {
+                                           int staged, int mark_pending, unsigned char* stage_smem) {
   const int E = G * k;
   int64_t* sI = reinterpret_cast<int64_t*>(stage_smem);            // [G][k]
   float* sD = reinterpret_cast<float*>(stage_smem + static_cast<size_t>(E) * sizeof(int64_t));   // [G][k]
@@ -846,6 +860,8 @@ __device__ __forceinline__ void merge_body(const float* Dp, const int64_t* Ip, i
     D[q * k + i] = -3.402823466e+38f;
     I[q * k + i] = -1;
   }
+  // the ranked stores are behind the barrier above; the padding store of slot 0, if any, is this thread's own
+  if (mark_pending && threadIdx.x == 0) mark_pending_row(Ip, G, q, k, strideI, I);
 }
 
 constexpr int kMergeStageMaxBytes = 96 * 1024;
@@ -873,11 +889,11 @@ __global__ void __launch_bounds__(1024) merge_kernel(const float* Dp, const int6
                                                     int k, float* __restrict__ D, int64_t* __restrict__ I,
                                                     int64_t strideD, int64_t strideI,
                                                     int* __restrict__ saw_overflow /* mapped host int or null */,
-                                                    int staged) {
+                                                    int staged, int mark_pending) {
   extern __shared__ __align__(16) unsigned char merge_smem[];
   __shared__ int total_valid;
-  if (staged == 2) merge_sort_body(Dp, Ip, G, blockIdx.x, k, D, I, strideD, strideI, saw_overflow, merge_smem);
-  else merge_body(Dp, Ip, G, blockIdx.x, k, D, I, strideD, strideI, saw_overflow, &total_valid, staged, merge_smem);
+  if (staged == 2) merge_sort_body(Dp, Ip, G, blockIdx.x, k, D, I, strideD, strideI, saw_overflow, mark_pending, merge_smem);
+  else merge_body(Dp, Ip, G, blockIdx.x, k, D, I, strideD, strideI, saw_overflow, &total_valid, staged, mark_pending, merge_smem);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -948,10 +964,10 @@ __global__ void __launch_bounds__(1024) xchg_merge_kernel(const char* __restrict
   __syncthreads();
   if (staged == 2)
     merge_sort_body(reinterpret_cast<const float*>(parts), reinterpret_cast<const int64_t*>(parts + i_off), world, blockIdx.x,
-                    k, D, I, part_cap / 4, part_cap / 8, saw_overflow, merge_smem);
+                    k, D, I, part_cap / 4, part_cap / 8, saw_overflow, 0, merge_smem);
   else
     merge_body(reinterpret_cast<const float*>(parts), reinterpret_cast<const int64_t*>(parts + i_off), world, blockIdx.x, k,
-               D, I, part_cap / 4, part_cap / 8, saw_overflow, &total_valid, staged, merge_smem);
+               D, I, part_cap / 4, part_cap / 8, saw_overflow, &total_valid, staged, 0, merge_smem);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -39,6 +39,7 @@ class FlatIPIndex:
         self._h = None
         self._options: dict[str, int] = {}
         self._selectors: dict[int, tuple] = {}   # id(selector) -> (selector, index generation, b2f_selector handle)
+        self._ext = None   # the first shard's index stream, as a torch stream
         if self.d != DIM:
             raise RuntimeError(f"b2f supports d = {DIM} only (ConvDR hard-codes IndexFlatIP(768)), got {d}")
 
@@ -64,6 +65,7 @@ class FlatIPIndex:
             self._selectors.clear()
             _lib.load().b2f_destroy(self._h)
             self._h = None
+            self._ext = None
 
     def __del__(self):
         try:
@@ -220,9 +222,28 @@ class FlatIPIndex:
         _lib.check(_lib.load().b2f_add_synthetic(self._ensure(), int(shard), int(first_row), int(n), int(seed),
                                                  int(stream), float(norm), int(id_base)))
 
+    def _first_device(self) -> int:
+        """The device of the first shard: device-resident queries and results live there."""
+        return self._devices[0] if self._devices else 0
+
+    def _device_call(self, q, *out):
+        """Checks that q and the outputs live on the first shard's device (outputs may also be page-locked host
+        tensors, which the last kernel writes directly), then orders the index stream after the caller's current
+        stream there: q may have just been produced by work queued on it (an encoder)."""
+        import torch
+        dev = self._first_device()
+        for t in (q,) + out:
+            assert (t.is_cuda and t.device.index == dev) or (t is not q and not t.is_cuda and t.is_pinned()), \
+                f"device search tensors must be on cuda:{dev}, the first shard's device; got {t.device}"
+        h = self._ensure()
+        if self._ext is None:
+            self._ext = torch.cuda.ExternalStream(self.stream_ptr(0), device=q.device)
+        self._ext.wait_stream(torch.cuda.current_stream(q.device))
+        return h
+
     def search_device(self, q, k: int, params=None):
-        """Search with a CUDA torch tensor of queries; returns CUDA tensors (D, I).  Single shard.  `params` as
-        in `search`."""
+        """Search with a CUDA torch tensor of queries on the first shard's device (any number of shards); returns
+        CUDA tensors (D, I) on that device.  `params` as in `search`."""
         import torch
         assert q.is_cuda and q.dim() == 2 and q.shape[1] == self.d
         q = q.contiguous().to(torch.float32)
@@ -230,8 +251,8 @@ class FlatIPIndex:
         D = torch.empty((nq, int(k)), dtype=torch.float32, device=q.device)
         I = torch.empty((nq, int(k)), dtype=torch.int64, device=q.device)
         if self._selector(params) is None:
-            _lib.check(_lib.load().b2f_search_device(self._ensure(), q.data_ptr(), nq, int(k), D.data_ptr(),
-                                                     I.data_ptr()))
+            _lib.check(_lib.load().b2f_search_device(self._device_call(q, D, I), q.data_ptr(), nq, int(k),
+                                                     D.data_ptr(), I.data_ptr()))
         else:
             self.search_device_async(q, k, D, I, params=params)
             self.finish()
@@ -239,20 +260,22 @@ class FlatIPIndex:
 
     def search_device_into(self, q, k: int, D, I) -> None:
         """Same, into caller-provided CUDA tensors (no allocation inside a timed loop)."""
-        _lib.check(_lib.load().b2f_search_device(self._ensure(), q.data_ptr(), q.shape[0], int(k), D.data_ptr(),
-                                                 I.data_ptr()))
+        _lib.check(_lib.load().b2f_search_device(self._device_call(q, D, I), q.data_ptr(), q.shape[0], int(k),
+                                                 D.data_ptr(), I.data_ptr()))
 
     def search_device_async(self, q, k: int, D, I, params=None) -> None:
-        """Enqueue only (b2f_search_device_async): q, D, I are CUDA tensors that must stay alive until
-        `finish()`; later work on the index stream may consume D / I without a host round trip.  `params` as in
-        `search`; searches with different selectors may be in flight together."""
+        """Enqueue only (b2f_search_device_async): q, D, I are CUDA tensors on the first shard's device that must
+        stay alive until `finish()`; later work on the index stream (`stream_ptr(0)`) may consume D / I without a
+        host round trip.  Until then, a row whose candidate list overflowed carries id -2 in its first slot.
+        `params` as in `search`; searches with different selectors may be in flight together."""
         sel = self._selector(params)
+        h = self._device_call(q, D, I)
         if sel is None:
-            _lib.check(_lib.load().b2f_search_device_async(self._ensure(), q.data_ptr(), q.shape[0], int(k),
-                                                           D.data_ptr(), I.data_ptr()))
+            _lib.check(_lib.load().b2f_search_device_async(h, q.data_ptr(), q.shape[0], int(k), D.data_ptr(),
+                                                           I.data_ptr()))
         else:
-            _lib.check(_lib.load().b2f_search_device_async_sel(self._ensure(), sel, q.data_ptr(), q.shape[0], int(k),
-                                                               D.data_ptr(), I.data_ptr()))
+            _lib.check(_lib.load().b2f_search_device_async_sel(h, sel, q.data_ptr(), q.shape[0], int(k), D.data_ptr(),
+                                                               I.data_ptr()))
 
     def finish(self) -> None:
         """Wait for every search enqueued with `search_device_async` (re-running overflowed queries)."""

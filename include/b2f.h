@@ -16,7 +16,7 @@
  *   - every function returns 0 on success, a B2F_ERR_* code otherwise, and never
  *     throws; b2f_last_error() returns a thread-local description;
  *   - "host" pointers are ordinary (pageable or pinned) host memory, "dev"
- *     pointers are CUDA device memory on the index's (first) device;
+ *     pointers are CUDA device memory on the index's (first shard's) device;
  *   - vectors are row-major float32 [n, d], d fixed at 768 (reference :353);
  *   - there is NO CPU fallback: without a CUDA device every compute entry point
  *     fails with B2F_ERR_NO_DEVICE.
@@ -138,22 +138,28 @@ void b2f_selector_destroy(b2f_selector* sel);
 int b2f_search_sel(b2f_index* idx, const b2f_selector* sel, const float* q_host, int64_t nq, int k,
                    float* D_host, int64_t* I_host);
 
-/* Device-resident variant (single-shard indexes): q_dev / D_dev / I_dev live on
- * the shard's device; work is enqueued on the index stream (b2f_stream) and the
- * stream is synchronised before returning (the candidate-overflow flags are
- * checked on the host).                                                        */
+/* Device-resident variant, for any number of shards: q_dev / D_dev / I_dev live on
+ * the first shard's device.  The search starts on that shard's index stream
+ * (b2f_stream(idx, 0)), so the caller orders q_dev's producer before it; the other
+ * shards copy the queries from there, and the merge of their results runs on that
+ * stream.  Every stream is synchronised before returning (the candidate-overflow
+ * flags are checked on the host, overflowed queries re-run and merged again).  */
 int b2f_search_device(b2f_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev,
                       int64_t* I_dev);
 
-/* Asynchronous form of b2f_search_device: only enqueues on the index stream and
- * returns; up to 16 searches may be in flight.  Results (and q_dev, which must
- * stay valid) may be consumed by later work on the same stream; the host may read
- * them after b2f_search_finish(), which waits for the stream and re-runs, on
- * the exact engine, any query whose candidate list overflowed (flags are written
- * by the last kernel of a pass straight into mapped host memory).  Every other
- * entry point settles pending searches first.  This is what lets a caller (the
- * NCCL layout in convdr_b200/dist.py, bench.py) queue search -> all-gather ->
- * merge, or several batches, without a host round trip in between.             */
+/* Asynchronous form of b2f_search_device, for any number of shards (q_dev, D_dev,
+ * I_dev on the first shard's device): only enqueues and returns; up to 16 searches
+ * may be in flight.  Results are ordered on the first shard's index stream
+ * (b2f_stream(idx, 0)): later work on that stream may consume them (q_dev must stay
+ * valid); the host may read them after b2f_search_finish(), which waits for the
+ * streams and re-runs, on the exact engine, any query whose candidate list
+ * overflowed (flags are written by the last kernel of a pass straight into mapped
+ * host memory) and, with several shards, merges that search again.  Until then such
+ * a row carries id -2 in its first slot, the merged row of a multi-shard search
+ * too; every other row is final once the stream has passed it.  Every other entry
+ * point settles pending searches first.  This is what lets a caller (the NCCL
+ * layout in convdr_b200/dist.py, bench.py) queue search -> all-gather -> merge, or
+ * several batches, without a host round trip in between.                       */
 int b2f_search_device_async(b2f_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev,
                             int64_t* I_dev);
 int b2f_search_finish(b2f_index* idx);
