@@ -45,6 +45,11 @@ SYMBOLS = {
     "b2f_merge_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int,
                                    C.c_void_p, C.c_void_p]),
     "b2f_reconstruct_n": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_void_p]),
+    "b2f_reconstruct_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "b2f_search_and_reconstruct_sel": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p,
+                                                 C.c_void_p, C.c_void_p]),
+    "b2f_search_and_reconstruct_device_sel": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int,
+                                                        C.c_void_p, C.c_void_p, C.c_void_p]),
     "b2f_reset": (C.c_int, [C.c_void_p]),
     "b2f_ntotal": (C.c_int64, [C.c_void_p]),
     "b2f_shard_rows": (C.c_int64, [C.c_void_p, C.c_int]),

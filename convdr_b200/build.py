@@ -14,7 +14,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(ROOT, "convdr_b200", "csrc")
 LIB = os.path.join(CSRC, "libb2f.so")
 SOURCES = ["b2f_api.cu"]
-HEADERS = ["common.cuh", "kernels_scan.cuh", "kernels_select.cuh", "kernels_selector.cuh", "kernels_umma.cuh", "kernels_umma_qs.cuh", "kernels_util.cuh",
+HEADERS = ["common.cuh", "kernels_gather.cuh", "kernels_scan.cuh", "kernels_select.cuh", "kernels_selector.cuh", "kernels_umma.cuh", "kernels_umma_qs.cuh", "kernels_util.cuh",
            os.path.join("..", "..", "include", "b2f.h")]
 
 NVCC_FLAGS = [

@@ -34,7 +34,10 @@
 #include <unistd.h>
 #include <vector>
 
+#include <cub/device/device_radix_sort.cuh>
+
 #include "common.cuh"
+#include "kernels_gather.cuh"
 #include "kernels_scan.cuh"
 #include "kernels_select.cuh"
 #include "kernels_selector.cuh"
@@ -206,6 +209,27 @@ struct Shard {
   Prof prof;
   Stats stats;
   bool peer_to_first = false;   // this device can store into shard 0's device memory (in-process result gather)
+  // label -> row lookup (kernels_gather.cuh), built by the first lookup of an index generation
+  struct Labels {
+    bool valid = false;
+    uint64_t generation = 0;
+    Seg* segs = nullptr;             // form 1: the segments sorted by global_start ...
+    int64_t* end_max = nullptr;      // ... and the prefix maximum of their ends
+    int nseg = 0;
+    bool ascending = false;          // form 2: idmap is searched in place
+    int64_t* keys = nullptr;         // form 3: sorted copy of idmap ...
+    uint32_t* rows = nullptr;        // ... and the row of each key
+  } lab;
+  // row gather (b2f_reconstruct_batch, b2f_search_and_reconstruct*)
+  struct GatherWs {
+    int64_t* keys = nullptr; int64_t keys_cap = 0;     // first shard: labels of a host call; other shards: a chunk's labels
+    int* found = nullptr; int64_t found_cap = 0;       // first shard: per label, the rows that hold it
+    float* out = nullptr; int64_t out_cap = 0;         // first shard: output rows of a host call
+    float* rows = nullptr; int64_t rows_cap = 0;       // staging shard: its found rows; first shard: those received
+    uint32_t* pos = nullptr; int64_t pos_cap = 0;      // output position of each of those rows
+    int* parts = nullptr; int64_t parts_cap = 0;       // staging shard: its per-label counts; first shard: all received
+    unsigned int* count = nullptr;                     // staging shard: rows staged
+  } gws;
 };
 
 }  // namespace
@@ -1347,6 +1371,232 @@ void reset_stats(b2f_index* idx) {
   for (Shard& S : idx->shards) S.stats = Stats();
 }
 
+// ---------------------------------------------------------------------------------------------------------
+// Rows by label (kernels_gather.cuh).
+// ---------------------------------------------------------------------------------------------------------
+void drop_label_index(Shard& S) {
+  if (S.lab.segs || S.lab.end_max || S.lab.keys || S.lab.rows) {
+    cudaSetDevice(S.dev);
+    dev_free(S.lab.segs); dev_free(S.lab.end_max); dev_free(S.lab.keys); dev_free(S.lab.rows);
+  }
+  S.lab = Shard::Labels();
+}
+
+// Every add and reset changes the labels: later lookups rebuild what they need.  Sorted copies are freed at once.
+void invalidate_labels(b2f_index* idx) {
+  ++idx->generation;
+  for (Shard& S : idx->shards) drop_label_index(S);
+}
+
+int64_t label_index_bytes(const Shard& S) {
+  return S.lab.keys ? S.n * static_cast<int64_t>(sizeof(int64_t) + sizeof(uint32_t)) : 0;
+}
+
+// The lookup structure of one shard for the current generation (on the shard's device; may wait for its stream).
+int ensure_label_index(b2f_index* idx, Shard& S) {
+  const uint64_t gen = idx->generation.load();
+  if (S.lab.valid && S.lab.generation == gen) return B2F_OK;
+  drop_label_index(S);
+  CU_TRY(cudaSetDevice(S.dev));
+  if (!S.has_ids) {   // form 1
+    std::vector<Seg> segs = S.segs;
+    std::stable_sort(segs.begin(), segs.end(), [](const Seg& a, const Seg& b) { return a.global_start < b.global_start; });
+    std::vector<int64_t> end_max(segs.size());
+    for (size_t i = 0; i < segs.size(); ++i)
+      end_max[i] = std::max(i ? end_max[i - 1] : INT64_MIN, segs[i].global_start + segs[i].count);
+    if (!segs.empty()) {
+      B2F_TRY(dev_alloc(&S.lab.segs, segs.size()));
+      B2F_TRY(dev_alloc(&S.lab.end_max, segs.size()));
+      CU_TRY(cudaMemcpyAsync(S.lab.segs, segs.data(), sizeof(Seg) * segs.size(), cudaMemcpyHostToDevice, S.stream));
+      CU_TRY(cudaMemcpyAsync(S.lab.end_max, end_max.data(), 8 * segs.size(), cudaMemcpyHostToDevice, S.stream));
+      CU_TRY(cudaStreamSynchronize(S.stream));   // the host vectors are local
+    }
+    S.lab.nseg = static_cast<int>(segs.size());
+  } else if (S.n > 0) {
+    const int blocks = static_cast<int>(std::min<int64_t>((S.n + 255) / 256, static_cast<int64_t>(S.sm_count) * 8));
+    struct Tmp {
+      int* flag = nullptr; uint32_t* rows_in = nullptr; void* cub = nullptr;
+      ~Tmp() { dev_free(flag); dev_free(rows_in); if (cub) cudaFree(cub); }
+    } tmp;
+    B2F_TRY(dev_alloc(&tmp.flag, 1));
+    CU_TRY(cudaMemsetAsync(tmp.flag, 0, sizeof(int), S.stream));
+    labels_descend_kernel<<<blocks, 256, 0, S.stream>>>(S.idmap, S.n, tmp.flag);
+    CU_TRY(cudaGetLastError());
+    int descending = 0;
+    CU_TRY(cudaMemcpyAsync(&descending, tmp.flag, sizeof(int), cudaMemcpyDeviceToHost, S.stream));
+    CU_TRY(cudaStreamSynchronize(S.stream));
+    if (!descending) {   // form 2
+      S.lab.ascending = true;
+    } else {             // form 3: (label, row) pairs sorted by label
+      B2F_TRY(dev_alloc(&S.lab.keys, static_cast<size_t>(S.n)));
+      B2F_TRY(dev_alloc(&S.lab.rows, static_cast<size_t>(S.n)));
+      B2F_TRY(dev_alloc(&tmp.rows_in, static_cast<size_t>(S.n)));
+      iota_rows_kernel<<<blocks, 256, 0, S.stream>>>(tmp.rows_in, S.n);
+      CU_TRY(cudaGetLastError());
+      size_t temp_bytes = 0;
+      CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, S.idmap, S.lab.keys, tmp.rows_in, S.lab.rows, S.n,
+                                             0, 64, S.stream));
+      if (cudaMalloc(&tmp.cub, temp_bytes) != cudaSuccess) {
+        (void)cudaGetLastError();
+        tmp.cub = nullptr;
+        return fail(B2F_ERR_OOM, "cudaMalloc of " + std::to_string(temp_bytes) + " bytes for the label sort failed");
+      }
+      CU_TRY(cub::DeviceRadixSort::SortPairs(tmp.cub, temp_bytes, S.idmap, S.lab.keys, tmp.rows_in, S.lab.rows, S.n,
+                                             0, 64, S.stream));
+      CU_TRY(cudaStreamSynchronize(S.stream));   // before the temporaries are freed
+    }
+  }
+  S.lab.generation = gen;
+  S.lab.valid = true;
+  return B2F_OK;
+}
+
+LabelIndex label_index_of(const Shard& S) {
+  LabelIndex L{};
+  if (!S.has_ids) {
+    L.segs = S.lab.segs;
+    L.end_max = S.lab.end_max;
+    L.nseg = S.lab.nseg;
+  } else {
+    L.keys = S.lab.ascending ? S.idmap : S.lab.keys;
+    L.rows = S.lab.ascending ? nullptr : S.lab.rows;
+    L.n = S.lab.keys || S.lab.ascending ? S.n : 0;
+  }
+  return L;
+}
+
+template <typename T>
+int ensure_buf(T*& p, int64_t& cap, int64_t need) {
+  if (need <= cap) return B2F_OK;
+  dev_free(p);
+  cap = 0;
+  B2F_TRY(dev_alloc(&p, static_cast<size_t>(need)));
+  cap = need;
+  return B2F_OK;
+}
+
+int gather_grid(const Shard& S, int64_t warps) {
+  return static_cast<int>(std::min<int64_t>(std::max<int64_t>((warps + 7) / 8, 1), static_cast<int64_t>(S.sm_count) * 8));
+}
+
+// Labels per gather step: bounds the staging and receive buffers and the output buffer of a host call (768 MB).
+constexpr int64_t kGatherChunk = int64_t(1) << 18;
+
+// Copy the stored row of every label labels[0..n) (settled labels, device memory on the first device) to out [n][768]:
+// device memory on the first device, or host memory (out_host; through the first shard's output buffer, one copy
+// per chunk).  A negative label gives a row of 0xFF bytes.  Per chunk, shard 0's stream records an event once the
+// labels are final there; every other shard waits for it, copies the chunk's labels and looks them up in its own
+// label index.  A shard that can store into the first device writes its rows into place; any other stages them with
+// their positions, and copies only those rows (and its per-label counts) over to the first device, where a scatter
+// kernel on shard 0's stream places them after every shard's event.  One int per label counts the rows that hold
+// it: after the single wait for shard 0's stream, 0 means "not in the index" and more than 1 "ambiguous".
+int gather_labels(b2f_index* idx, const int64_t* labels, int64_t n, float* out, bool out_host) {
+  if (n == 0) return B2F_OK;
+  const int G = static_cast<int>(idx->shards.size());
+  Shard& S0 = idx->shards[0];
+  B2F_TRY(run_on_shards(idx, [&](int g) { return ensure_label_index(idx, idx->shards[g]); }));
+  bool staging = false;
+  for (int g = 1; g < G; ++g) staging = staging || !idx->shards[g].peer_to_first;
+  const int64_t chunk = std::min(n, kGatherChunk);
+  CU_TRY(cudaSetDevice(S0.dev));
+  Shard::GatherWs& W0 = S0.gws;
+  B2F_TRY(ensure_buf(W0.found, W0.found_cap, n));
+  if (out_host) B2F_TRY(ensure_buf(W0.out, W0.out_cap, chunk * kD));
+  if (staging) {
+    B2F_TRY(ensure_buf(W0.rows, W0.rows_cap, chunk * kD));
+    B2F_TRY(ensure_buf(W0.pos, W0.pos_cap, chunk));
+    B2F_TRY(ensure_buf(W0.parts, W0.parts_cap, chunk * (G - 1)));
+  }
+  CU_TRY(cudaMemsetAsync(W0.found, 0, sizeof(int) * n, S0.stream));
+  for (int64_t c0 = 0; c0 < n; c0 += chunk) {
+    const int64_t m = std::min(chunk, n - c0);
+    float* dst = out_host ? W0.out : out + c0 * kD;
+    int* found = W0.found + c0;
+    if (staging) CU_TRY(cudaMemsetAsync(W0.parts, 0, sizeof(int) * m * (G - 1), S0.stream));
+    CU_TRY(cudaEventRecord(S0.ev, S0.stream));   // the labels are final here; the previous chunk has been placed
+    std::atomic<int64_t> received{0};
+    B2F_TRY(run_on_shards(idx, [&](int g) -> int {
+      Shard& S = idx->shards[g];
+      CU_TRY(cudaSetDevice(S.dev));
+      const LabelIndex L = label_index_of(S);
+      if (g == 0) {
+        gather_rows_kernel<<<gather_grid(S, m), kGatherThreads, 0, S.stream>>>(L, S.x32, labels + c0, m, 1, dst, found,
+                                                                               nullptr, nullptr, nullptr);
+        CU_TRY(cudaGetLastError());
+        return B2F_OK;
+      }
+      Shard::GatherWs& W = S.gws;
+      CU_TRY(cudaStreamWaitEvent(S.stream, S0.ev, 0));
+      if (S.n > 0) {
+        B2F_TRY(ensure_buf(W.keys, W.keys_cap, chunk));
+        if (S.dev == S0.dev) CU_TRY(cudaMemcpyAsync(W.keys, labels + c0, 8 * m, cudaMemcpyDeviceToDevice, S.stream));
+        else CU_TRY(cudaMemcpyPeerAsync(W.keys, S.dev, labels + c0, S0.dev, 8 * m, S.stream));
+        if (S.peer_to_first) {
+          gather_rows_kernel<<<gather_grid(S, m), kGatherThreads, 0, S.stream>>>(L, S.x32, W.keys, m, 0, dst, found,
+                                                                                 nullptr, nullptr, nullptr);
+          CU_TRY(cudaGetLastError());
+        } else {
+          B2F_TRY(ensure_buf(W.rows, W.rows_cap, chunk * kD));
+          B2F_TRY(ensure_buf(W.pos, W.pos_cap, chunk));
+          B2F_TRY(ensure_buf(W.parts, W.parts_cap, chunk));
+          if (!W.count) B2F_TRY(dev_alloc(&W.count, 1));
+          CU_TRY(cudaMemsetAsync(W.parts, 0, sizeof(int) * m, S.stream));
+          CU_TRY(cudaMemsetAsync(W.count, 0, sizeof(unsigned int), S.stream));
+          gather_rows_kernel<<<gather_grid(S, m), kGatherThreads, 0, S.stream>>>(L, S.x32, W.keys, m, 0, nullptr, W.parts,
+                                                                                 W.rows, W.pos, W.count);
+          CU_TRY(cudaGetLastError());
+          unsigned int staged = 0;
+          CU_TRY(cudaMemcpyAsync(&staged, W.count, sizeof(staged), cudaMemcpyDeviceToHost, S.stream));
+          CU_TRY(cudaStreamSynchronize(S.stream));
+          // a receive slot per label suffices unless labels are held by several shards; those are reported from the
+          // counts below, which always travel whole
+          const int64_t off = received.fetch_add(staged);
+          const int64_t take = std::max<int64_t>(0, std::min<int64_t>(staged, m - off));
+          if (take > 0) {
+            CU_TRY(cudaMemcpyPeerAsync(W0.rows + off * kD, S0.dev, W.rows, S.dev, sizeof(float) * kD * take, S.stream));
+            CU_TRY(cudaMemcpyPeerAsync(W0.pos + off, S0.dev, W.pos, S.dev, sizeof(uint32_t) * take, S.stream));
+          }
+          CU_TRY(cudaMemcpyPeerAsync(W0.parts + (g - 1) * m, S0.dev, W.parts, S.dev, sizeof(int) * m, S.stream));
+        }
+      }
+      CU_TRY(cudaEventRecord(S.ev, S.stream));
+      return B2F_OK;
+    }));
+    CU_TRY(cudaSetDevice(S0.dev));
+    for (int g = 1; g < G; ++g) CU_TRY(cudaStreamWaitEvent(S0.stream, idx->shards[g].ev, 0));
+    if (staging) {
+      const int64_t rows = std::min<int64_t>(received.load(), m);
+      scatter_rows_kernel<<<gather_grid(S0, std::max(rows, (m + 31) / 32)), kGatherThreads, 0, S0.stream>>>(
+          W0.rows, W0.pos, rows, dst, W0.parts, G - 1, m, found);
+      CU_TRY(cudaGetLastError());
+    }
+    if (out_host)
+      CU_TRY(cudaMemcpyAsync(out + c0 * kD, W0.out, sizeof(float) * kD * m, cudaMemcpyDeviceToHost, S0.stream));
+  }
+  std::vector<int> counts(static_cast<size_t>(n));
+  CU_TRY(cudaMemcpyAsync(counts.data(), W0.found, sizeof(int) * n, cudaMemcpyDeviceToHost, S0.stream));
+  CU_TRY(cudaStreamSynchronize(S0.stream));
+  if (std::all_of(counts.begin(), counts.end(), [](int c) { return c == 1; })) return B2F_OK;
+  std::vector<int64_t> keys(static_cast<size_t>(n));   // padding (negative labels) counts 0 too
+  CU_TRY(cudaMemcpy(keys.data(), labels, sizeof(int64_t) * n, cudaMemcpyDeviceToHost));
+  for (int64_t i = 0; i < n; ++i) {
+    if (counts[i] == 1 || keys[i] < 0) continue;
+    if (counts[i] == 0) return fail(B2F_ERR_INVALID, "label " + std::to_string(keys[i]) + " is not in the index");
+    return fail(B2F_ERR_INVALID, "label " + std::to_string(keys[i]) +
+                                     " is held by more than one row: the lookup is ambiguous");
+  }
+  return B2F_OK;
+}
+
+// Labels of a host call into the first shard's label buffer (negative keys were refused or are padding).
+int upload_labels(b2f_index* idx, const int64_t* keys_host, int64_t n) {
+  Shard& S0 = idx->shards[0];
+  CU_TRY(cudaSetDevice(S0.dev));
+  B2F_TRY(ensure_buf(S0.gws.keys, S0.gws.keys_cap, n));
+  CU_TRY(cudaMemcpyAsync(S0.gws.keys, keys_host, 8 * n, cudaMemcpyHostToDevice, S0.stream));
+  return B2F_OK;
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -1459,6 +1709,10 @@ void b2f_destroy(b2f_index* idx) {
     dev_free(W.qnorm); dev_free(W.qerr); dev_free(W.D); dev_free(W.I);
     for (int s = 0; s < kMaxPending; ++s) { dev_free(W.Dp[s]); dev_free(W.Ip[s]); }
     dev_free(W.fbq); dev_free(W.fbD); dev_free(W.fbI);
+    drop_label_index(S);
+    Shard::GatherWs& GW = S.gws;
+    dev_free(GW.keys); dev_free(GW.found); dev_free(GW.out); dev_free(GW.rows); dev_free(GW.pos); dev_free(GW.parts);
+    dev_free(GW.count);
     if (W.ovf_host) cudaFreeHost(W.ovf_host);
     if (W.pin) cudaFreeHost(W.pin);
     for (cudaEvent_t ev : S.prof.pool) cudaEventDestroy(ev);
@@ -1502,7 +1756,7 @@ static int add_impl(b2f_index* idx, const float* x_host, const int64_t* ids_host
   if (n < 0 || (n > 0 && !x_host)) return fail(B2F_ERR_INVALID, "bad add arguments");
   if (n == 0) return B2F_OK;
   B2F_TRY(settle_pending(idx));
-  ++idx->generation;
+  invalidate_labels(idx);
   const int G = static_cast<int>(idx->shards.size());
   if (ids_host) {
     for (Shard& S : idx->shards)
@@ -1552,7 +1806,7 @@ int b2f_add_device(b2f_index* idx, int shard, const float* x_dev, int64_t n) {
   B2F_TRY(settle_pending(idx));
   Shard& S = idx->shards[shard];
   if (S.has_ids && S.n > 0) return fail(B2F_ERR_INVALID, "index uses explicit ids");
-  ++idx->generation;
+  invalidate_labels(idx);
   CU_TRY(cudaSetDevice(S.dev));
   B2F_TRY(ensure_capacity(idx, S, S.n + n));
   CU_TRY(cudaMemcpyAsync(S.x32 + S.n * kD, x_dev, static_cast<size_t>(n) * kD * 4, cudaMemcpyDeviceToDevice, S.stream));
@@ -1572,7 +1826,7 @@ int b2f_add_synthetic(b2f_index* idx, int shard, int64_t first_row, int64_t n, u
   B2F_TRY(settle_pending(idx));
   Shard& S = idx->shards[shard];
   if (S.has_ids && S.n > 0) return fail(B2F_ERR_INVALID, "index uses explicit ids");
-  ++idx->generation;
+  invalidate_labels(idx);
   CU_TRY(cudaSetDevice(S.dev));
   B2F_TRY(ensure_capacity(idx, S, S.n + n));
   const uint32_t k0 = static_cast<uint32_t>(seed) ^ static_cast<uint32_t>(stream);
@@ -1604,7 +1858,7 @@ int b2f_reconstruct_n(b2f_index* idx, int shard, int64_t row0, int64_t n, float*
 int b2f_reset(b2f_index* idx) {
   if (!idx) return fail(B2F_ERR_INVALID, "null index");
   B2F_TRY(settle_pending(idx));
-  ++idx->generation;
+  invalidate_labels(idx);
   for (Shard& S : idx->shards) {
     CU_TRY(cudaSetDevice(S.dev));
     CU_TRY(cudaStreamSynchronize(S.stream));
@@ -1900,6 +2154,43 @@ int b2f_search_sel(b2f_index* idx, const b2f_selector* sel, const float* q_host,
   return B2F_OK;
 }
 
+int b2f_reconstruct_batch(b2f_index* idx, const int64_t* keys_host, int64_t n, float* out_host) {
+  if (!idx || n < 0 || (n > 0 && (!keys_host || !out_host))) return fail(B2F_ERR_INVALID, "bad reconstruct_batch arguments");
+  for (int64_t i = 0; i < n; ++i)
+    if (keys_host[i] < 0) return fail(B2F_ERR_INVALID, "label " + std::to_string(keys_host[i]) + " is negative");
+  if (n == 0) return B2F_OK;
+  B2F_TRY(settle_pending(idx));
+  B2F_TRY(upload_labels(idx, keys_host, n));
+  return gather_labels(idx, idx->shards[0].gws.keys, n, out_host, true);
+}
+
+int b2f_search_and_reconstruct_sel(b2f_index* idx, const b2f_selector* sel, const float* q_host, int64_t nq, int k,
+                                   float* D_host, int64_t* I_host, float* R_host) {
+  B2F_TRY(check_args_search(idx, q_host, nq, k, D_host, I_host));
+  if (nq > 0 && !R_host) return fail(B2F_ERR_INVALID, "null output pointer");
+  B2F_TRY(b2f_search_sel(idx, sel, q_host, nq, k, D_host, I_host));
+  if (nq == 0) return B2F_OK;
+  B2F_TRY(upload_labels(idx, I_host, nq * k));
+  return gather_labels(idx, idx->shards[0].gws.keys, nq * k, R_host, true);
+}
+
+int b2f_search_and_reconstruct_device_sel(b2f_index* idx, const b2f_selector* sel, const float* q_dev, int64_t nq,
+                                          int k, float* D_dev, int64_t* I_dev, float* R_dev) {
+  B2F_TRY(check_args_search(idx, q_dev, nq, k, D_dev, I_dev));
+  B2F_TRY(check_selector(idx, sel));
+  if (nq > 0 && !R_dev) return fail(B2F_ERR_INVALID, "null output pointer");
+  if (nq == 0) return B2F_OK;
+  if (sel) {   // the queued form takes a selector; settled right away, labels never carry the -2 marker here
+    B2F_TRY(settle_pending(idx));
+    reset_stats(idx);
+    B2F_TRY(b2f_search_device_async_sel(idx, sel, q_dev, nq, k, D_dev, I_dev));
+    B2F_TRY(settle_pending(idx));
+  } else {
+    B2F_TRY(b2f_search_device(idx, q_dev, nq, k, D_dev, I_dev));
+  }
+  return gather_labels(idx, I_dev, nq * k, R_dev, false);
+}
+
 // The whole end-to-end call of the one-process-per-GPU layout in ONE entry point: stage / upload the queries,
 // local search, NVLink push, wait + merge (storing the result straight into page-locked host memory), one
 // host wait, overflow protocol.  Collective: every rank calls it with the same nq, k.  (The Python layer
@@ -2076,7 +2367,7 @@ int b2f_set_option(b2f_index* idx, const char* key, int64_t value) {
     if (idx->ntotal > 0) return fail(B2F_ERR_INVALID, "shadow can only be changed on an empty index");
     if (value < 0 || value > 3) return fail(B2F_ERR_INVALID, "shadow must be 0 (none), 1 (bf16), 2 (int8) or 3 (auto)");
     idx->shadow = static_cast<int>(value);
-    ++idx->generation;
+    invalidate_labels(idx);
     for (Shard& S : idx->shards) {
       cudaSetDevice(S.dev);
       dev_free(S.x32); dev_free(S.x16); dev_free(S.x8); dev_free(S.tscale); dev_free(S.idmap);
@@ -2157,6 +2448,10 @@ int b2f_get_stat(const b2f_index* idx, const char* key, double* out) {
   if (k == "shadow_format") *out = idx->shards.empty() ? 0 : idx->shards[0].fmt;   // 0 none, 1 bf16, 2 int8
   else if (k == "generation") *out = static_cast<double>(idx->generation.load());   // bumped by every add and reset
   else if (k == "shadow_rho") *out = idx->shards.empty() ? 0 : idx->shards[0].rho;  // AUTO: median 2 eps8 / sigma
+  else if (k == "label_index_bytes") {   // sorted (label, row) copies held by the shards
+    *out = 0;
+    for (const Shard& S : idx->shards) *out += static_cast<double>(label_index_bytes(S));
+  }
   else if (k == "launches") *out = s.launches;
   else if (k == "phases") *out = s.phases;
   else if (k == "candidates") *out = s.candidates;
@@ -2242,6 +2537,7 @@ extern "C" int b2f_add_flat_file(b2f_index* idx, int shard, const char* path, in
   if (n == 0) return B2F_OK;
   if (S.n + n >= 0xfffffff0ll) return fail(B2F_ERR_INVALID, "a shard holds at most 2^32-16 rows");
   ++idx->generation;
+  drop_label_index(S);   // loads of other shards may run concurrently: each drops its own label index
   CU_TRY(cudaSetDevice(S.dev));
   CU_TRY(cudaStreamSynchronize(S.stream));
   if (!S.has_ids) {

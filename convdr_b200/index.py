@@ -160,6 +160,34 @@ class FlatIPIndex:
         _lib.check(_lib.load().b2f_reconstruct_n(self._ensure(), int(shard), int(i0), int(ni), out.ctypes.data))
         return out
 
+    def reconstruct(self, key: int) -> np.ndarray:
+        """index.reconstruct(key): the stored row of the label `key` (what `search` returns), float32 [d]."""
+        return self.reconstruct_batch(np.array([key], dtype=np.int64))[0]
+
+    def reconstruct_batch(self, keys) -> np.ndarray:
+        """index.reconstruct_batch(keys): the stored rows of the labels `keys` (any order, repeats allowed), float32
+        [n, d], gathered on the GPU.  RuntimeError naming the label when one is not in the index, is negative, or is
+        held by more than one row."""
+        keys = np.ascontiguousarray(keys, dtype=np.int64).reshape(-1)
+        out = np.empty((keys.size, self.d), dtype=np.float32)
+        _lib.check(_lib.load().b2f_reconstruct_batch(self._ensure(), keys.ctypes.data, keys.size, out.ctypes.data))
+        return out
+
+    def search_and_reconstruct(self, x, k: int, params=None):
+        """D, I, R = index.search_and_reconstruct(x, k, params=None): `search`, plus R float32 [nq, k, d], the stored
+        row of every result label; a -1 label (padding) gets a row of 0xFF bytes (NaN), as in faiss."""
+        x = self._as_rows(x, "x")
+        k = int(k)
+        assert k > 0, "k must be positive"
+        nq = x.shape[0]
+        D = np.empty((nq, k), dtype=np.float32)
+        I = np.empty((nq, k), dtype=np.int64)
+        R = np.empty((nq, k, self.d), dtype=np.float32)
+        h = self._ensure()
+        _lib.check(_lib.load().b2f_search_and_reconstruct_sel(h, self._selector(params), x.ctypes.data, nq, k,
+                                                              D.ctypes.data, I.ctypes.data, R.ctypes.data))
+        return D, I, R
+
     def reset(self) -> None:
         """index.reset(): drop all rows (device buffers are kept for the next block by default)."""
         if self._h is not None:
@@ -257,6 +285,22 @@ class FlatIPIndex:
             self.search_device_async(q, k, D, I, params=params)
             self.finish()
         return D, I
+
+    def search_and_reconstruct_device(self, q, k: int, params=None):
+        """`search_and_reconstruct` with a CUDA torch tensor of queries on the first shard's device (any number of
+        shards): returns CUDA tensors (D, I, R) there, R float32 [nq, k, d].  The rows are gathered on the GPUs that
+        hold them, next to the resident index."""
+        import torch
+        assert q.is_cuda and q.dim() == 2 and q.shape[1] == self.d
+        q = q.contiguous().to(torch.float32)
+        nq, k = q.shape[0], int(k)
+        D = torch.empty((nq, k), dtype=torch.float32, device=q.device)
+        I = torch.empty((nq, k), dtype=torch.int64, device=q.device)
+        R = torch.empty((nq, k, self.d), dtype=torch.float32, device=q.device)
+        sel = self._selector(params)
+        _lib.check(_lib.load().b2f_search_and_reconstruct_device_sel(self._device_call(q, D, I, R), sel, q.data_ptr(),
+                                                                     nq, k, D.data_ptr(), I.data_ptr(), R.data_ptr()))
+        return D, I, R
 
     def search_device_into(self, q, k: int, D, I) -> None:
         """Same, into caller-provided CUDA tensors (no allocation inside a timed loop)."""

@@ -238,6 +238,32 @@ int b2f_xchg_flush(b2f_index* idx);
  * `shard` (shard-local positions) back to host memory — inspection / tests.    */
 int b2f_reconstruct_n(b2f_index* idx, int shard, int64_t row0, int64_t n, float* out_host);
 
+/* Rows by label: faiss index.reconstruct(key) / reconstruct_batch(keys) / search_and_reconstruct(x, k).
+ * A label is what search returns: the explicit id (b2f_add_with_ids, flat files) or the position given by the
+ * shard's segments (b2f_add, b2f_add_device; b2f_add_synthetic with its id_base).  Each shard finds a label's
+ * row on the GPU through a label index built by its first lookup after an add or reset:
+ *   - segment labels: the segments themselves (nothing is built);
+ *   - explicit labels stored in ascending order (e.g. one ConvDR block per shard): the label map, in place;
+ *   - any other explicit labels: a sorted (label, row) copy, 12 bytes per row (stat "label_index_bytes"),
+ *     freed by the next add or reset.
+ * The rows are gathered on the GPU, across shards, and returned bit for bit as stored (what b2f_reconstruct_n
+ * returns).  A lookup fails with B2F_ERR_INVALID, naming the label, when a label is not in the index, is negative
+ * (b2f_reconstruct_batch), or is held by more than one row, within a shard or across shards (duplicate labels
+ * stay legal for search; only their lookup is ambiguous).
+ *
+ * b2f_reconstruct_batch: keys_host [n] in any order, repeats allowed -> out_host float32 [n, d].
+ * b2f_search_and_reconstruct_sel: b2f_search_sel (sel may be NULL: no filter), then the rows of the result labels:
+ *   R_host float32 [nq, k, d].  D and I are exactly those of b2f_search_sel.  A -1 label (padding: fewer than k
+ *   rows, or fewer than k selected rows) gets a row of 0xFF bytes (NaN in every component), as faiss's
+ *   Index::search_and_reconstruct does.
+ * b2f_search_and_reconstruct_device_sel: the same with q_dev, D_dev, I_dev and R_dev on the first shard's
+ *   device; ordered on b2f_stream(idx, 0) like b2f_search_device, synchronised before returning.           */
+int b2f_reconstruct_batch(b2f_index* idx, const int64_t* keys_host, int64_t n, float* out_host);
+int b2f_search_and_reconstruct_sel(b2f_index* idx, const b2f_selector* sel, const float* q_host, int64_t nq, int k,
+                                   float* D_host, int64_t* I_host, float* R_host);
+int b2f_search_and_reconstruct_device_sel(b2f_index* idx, const b2f_selector* sel, const float* q_dev, int64_t nq,
+                                          int k, float* D_dev, int64_t* I_dev, float* R_dev);
+
 /* index.reset()                                         reference :202 */
 int b2f_reset(b2f_index* idx);
 
@@ -289,7 +315,9 @@ int b2f_set_option(b2f_index* idx, const char* key, int64_t value);
  * "score_launches", "score_rows" (scoring kernels: device time, launches, rows
  * streamed) and "select_ms" (refresh + final kernels); "shadow_format" (first shard: 0 none,
  * 1 bf16, 2 int8) and "shadow_rho" (AUTO: median 2 eps8 / sigma of the probe, 0 if not measured);
- * "generation" (bumped by every add and reset: a selector built at another generation is stale). */
+ * "generation" (bumped by every add and reset: a selector built at another generation is stale);
+ * "label_index_bytes" (sorted label copies held for b2f_reconstruct_batch and b2f_search_and_reconstruct*, all
+ * shards). */
 int b2f_get_stat(const b2f_index* idx, const char* key, double* out);
 
 void b2f_destroy(b2f_index* idx);
