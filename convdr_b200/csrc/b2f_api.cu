@@ -7,9 +7,9 @@
 //   prep_queries -> per pass of <= 256 queries: pass_init -> score+select (ONE launch) -> finalize
 //
 // where score+select is umma_qs_score_select_kernel (<= 208 queries) or umma_score_select_kernel
-// (tcgen05, both), with the phased schedules (dense bootstrap / refresh between phases) kept for the
-// SIMT scan_kernel and as A/B options.  There is no CPU arithmetic anywhere on this path; without a
-// CUDA device every entry point fails.
+// (tcgen05, both).  The SIMT scan_kernel keeps a phased schedule (dense first phase, refresh_kernel
+// between phases).  There is no CPU arithmetic anywhere on this path; without a CUDA device every
+// entry point fails.
 #include "../../include/b2f.h"
 
 #include <cuda.h>
@@ -124,8 +124,7 @@ struct Workspace {
   int* ovf = nullptr;
   float* margin = nullptr;
   int* err = nullptr;
-  bool areas_clean = false;   // tensor-engine invariant: private areas of both cand buffers are all-zero
-  uint64_t* gath = nullptr;   // refresh scratch: dense copy of a segmented list
+  uint64_t* gath = nullptr;   // finalize scratch: gathered lists too long for shared memory
   int* cnt2 = nullptr;        // [qp][max_pairs] per-pair append counts of the tensor engine
   unsigned int* hist = nullptr;   // [qp][kHistBuckets] tightening histogram of the tensor engine
   uint32_t* hkey0 = nullptr;      // [qp] its base key
@@ -297,7 +296,6 @@ struct SelShard {
   int* qs_tiles = nullptr;           // QS tiles (kQsTileRows rows)
   int* ts_tiles = nullptr;           // TS tiles (kTileRows rows)
   int n_qs = 0, n_ts = 0;
-  std::vector<int> ts_host;          // host copy: the phased TS schedules walk a sub-range per phase
 };
 }  // namespace
 
@@ -360,11 +358,8 @@ struct b2f_index {
   int l2_prefetch = 0;    // QS: distance (tiles) of the optional L2 prefetch warp; 0 = off (default: measured slower)
   int worst_case_margin = 0;  // 1: bf16 margin from the data-independent worst case (A/B only)
   int tighten_adaptive = 1;  // refresher pause grows with the elapsed kernel time (see UmmaArgs)
-  int bootstrap = 0;      // TS engine with tightening: 1 = dense bootstrap launch + bootstrap_select_kernel before the
-                          // main launch, 0 = none (thresholds start at -inf inside the single launch)
-  int tighten = 2000;      // TS engine: in-kernel threshold tightening through a global hit histogram (one
-                          // launch after the bootstrap); pause of the refresher between rounds in ns,
-                          // 0 = off (geometric phases with a refresh kernel between them).
+  int tighten = 2000;      // tensor engine: minimum pause in ns of the refresher warp, which tightens the thresholds
+                          // inside the scoring launch through a global hit histogram
   Stats stats;
 };
 
@@ -612,7 +607,6 @@ int ensure_pass_ws(Shard& S, int qp, int C) {
   }
   W.qp_cap = qp;
   W.C = C;
-  W.areas_clean = false;
   return B2F_OK;
 }
 
@@ -666,8 +660,8 @@ __global__ void pass_init_kernel(const float* __restrict__ qnorm, const float* _
   const int q = blockIdx.x;
   bool finite = true;
   if (hist != nullptr) {
-    // TS engine without a bootstrap launch: empty tightening histogram of 64 buckets per binade over
-    // the eight binades below R = (1 + 2^-6) * ||q|| * max||p|| >= |any prefilter score of q|; tau = -inf.
+    // tensor engine: empty tightening histogram of 64 buckets per binade over the eight binades below
+    // R = (1 + 2^-6) * ||q|| * max||p|| >= |any prefilter score of q|; tau = -inf.
     for (int b = threadIdx.x; b < kHistStride; b += blockDim.x) hist[static_cast<int64_t>(q) * kHistStride + b] = 0u;
     if (threadIdx.x == 0) {
       const float R = __fmul_ru(bound_mul(qnorm[q], __fsqrt_ru(__uint_as_float(maxnorm2_bits[2]))), 1.015625f);
@@ -678,8 +672,8 @@ __global__ void pass_init_kernel(const float* __restrict__ qnorm, const float* _
     }
   }
   if (threadIdx.x == 0) {
-    // Every pass starts without a threshold: finalize_kernel filters on tau[q] whenever tightening is on,
-    // and a pass that ends inside the dense phase (shard smaller than the bootstrap) never writes it.
+    // Every pass starts without a threshold: the tensor kernels and finalize_kernel read tau[q] from the
+    // start, so nothing an earlier search or an earlier collection left there may filter this pass.
     tau[q] = -INFINITY;
     // tensor engine: scores are taken against the CENTRED rows p - mu (constant shift q.mu per query), so its
     // bounds use Pc = max ||p - mu||; the fp32 scan reads the rows themselves: P = max ||p||
@@ -762,7 +756,7 @@ struct PassPlan {
   bool exact;   // total-order keys, zero margin, bounded phases
   int qp;       // max queries per pass
   int C;        // candidate capacity per query
-  int64_t n0;   // rows of the dense (bootstrap) phase
+  int64_t n0;   // SIMT scans: rows of the dense first phase
   int S;        // tensor engine: survivor area [0, S) of a list
   int cap_p;    // TS variant: private slots per (query, CTA pair) and launch
   int cap_a;    // QS variant: private slots per (query, CTA)
@@ -773,6 +767,7 @@ PassPlan make_plan(const b2f_index* idx, const Shard& S, int path, int k, int64_
   PassPlan p;
   p.path = path;
   p.exact = (path == B2F_PATH_SCAN_EXACT);
+  p.n0 = 0;
   p.S = 0;
   p.cap_p = 0;
   p.cap_a = 0;
@@ -786,10 +781,6 @@ PassPlan make_plan(const b2f_index* idx, const Shard& S, int path, int k, int64_
     // tensor cycles), TS for (nearly) full passes.
     p.variant = idx->umma_variant == 1 ? 3 : idx->umma_variant;
     p.qp = kUmmaMaxQ;
-    // bootstrap (dense) phase of the phased TS schedules: whole tiles per CTA pair, at least 8k rows
-    const int64_t wave = static_cast<int64_t>(S.max_pairs) * kTileRows;
-    const int64_t t0 = (std::max<int64_t>(4096, 8ll * k) + wave - 1) / wave;
-    p.n0 = t0 * wave;
     // survivors within the margin of the k-th score: ~k * (e^(z * 2eps / sigma) - 1) with z ~ 5 the tail slope
     // at rank 100 of 4e7: ~200 for isotropic unit rows, ~700 for LayerNorm-like rows with a common mean after
     // centring (DESIGN.md section 4) — 4096 leaves a factor of 5
@@ -801,7 +792,7 @@ PassPlan make_plan(const b2f_index* idx, const Shard& S, int path, int k, int64_
     // expected appends per (query, area) in a phase: 2 (margin) * (growth-1) * k / areas; x2 safety
     // (with in-kernel tightening the pass rate follows k/rows_seen, far fewer appends; keep the bound)
     const int64_t expect = 4ll * (std::max(2, idx->growth) - 1) * k / S.max_pairs;
-    p.cap_p = static_cast<int>(round_up(std::max<int64_t>(std::max<int64_t>(512, t0 * kTileRows), expect), 64));   // per pair; half per (pair, half tile)
+    p.cap_p = static_cast<int>(round_up(std::max<int64_t>(512, expect), 64));   // per pair; half per (pair, half tile)
     p.cap_a = static_cast<int>(round_up(std::max<int64_t>(512, kQsTileRowsCta + expect / 2), 32));
     p.C = p.S + std::max(S.max_pairs * p.cap_p, 2 * S.max_pairs * p.cap_a);
   } else {
@@ -816,8 +807,27 @@ PassPlan make_plan(const b2f_index* idx, const Shard& S, int path, int k, int64_
 // Which tensor kernel runs a pass of nqp queries.
 int pass_variant(const b2f_index* idx, const PassPlan& plan, int nqp) {
   if (plan.variant == 2 || plan.variant == 3) return plan.variant;
-  if (!idx->tighten || idx->bootstrap) return 2;      // the phased schedules exist for TS only
   return nqp <= idx->qs_max_q ? 3 : 2;
+}
+
+// The fused last step of a tensor-engine pass (both variants): gather the private areas of `cap` slots per
+// (query, area), select, rescore exactly, sort, write the pass's rows of D_out/I_out.
+int enqueue_finalize(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q32p, int nqp, int k, int cap,
+                     float* D_out, int64_t* I_out, int64_t out_stride, int* ovf_dst) {
+  Workspace& W = S.ws;
+  ProfScope ps(idx, S, 1);
+  int PS = 1024;                       // survivors (bufB): >= S
+  while (PS < plan.S) PS <<= 1;
+  int P = 8192;                        // gathered list (bufA); longer lists go through global memory
+  while (P < PS) P <<= 1;
+  finalize_kernel<<<nqp, kFinThreads, static_cast<size_t>(P + PS) * sizeof(uint64_t), S.stream>>>(
+      W.cand[0], W.gath, W.cnt, W.C, k, W.margin, plan.S, cap, 2 * S.max_pairs, W.cnt2, W.ovf, ovf_dst, q32p,
+      S.x32, S.segs_d, static_cast<int>(S.segs.size()), S.has_ids ? S.idmap : nullptr, D_out, I_out, out_stride, P,
+      W.tau, S.mu);
+  CU_TRY(cudaGetLastError());
+  S.stats.launches += 1;
+  S.stats.passes += 1;
+  return B2F_OK;
 }
 
 // Enqueue one pass (<= plan.qp queries) on the shard stream.  q32p: the pass's fp32 queries
@@ -834,24 +844,13 @@ int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q3
   const int variant = plan.path == B2F_PATH_UMMA_BF16 ? pass_variant(idx, plan, nqp) : 0;
   const bool tensor = variant == 2;      // TS: queries in TMEM, areas per CTA pair
   const bool tensor_qs = variant == 3;   // QS: queries streamed on the N side, areas per CTA
-  const bool one_launch = tensor_qs || (tensor && idx->tighten && !idx->bootstrap);   // ONE scoring launch per pass
-  if (tensor && !one_launch) {
-    if (!W.areas_clean) {   // phased TS schedules gather whole areas: they must be all-zero between launches
-      CU_TRY(cudaMemsetAsync(W.cand[0], 0, sizeof(uint64_t) * static_cast<size_t>(W.qp_cap) * W.C, s));
-      CU_TRY(cudaMemsetAsync(W.cand[1], 0, sizeof(uint64_t) * static_cast<size_t>(W.qp_cap) * W.C, s));
-      W.areas_clean = true;
-    }
-  } else {
-    W.areas_clean = false;  // flat lists / one-launch passes leave records behind in the areas
-  }
   const int n_areas = 2 * S.max_pairs;   // TS: two per CTA pair (one per half tile); QS: one per CTA
-  const int cap_h = plan.cap_p / 2;       // TS: slots per (query, pair, half tile)
   const bool i8 = S.fmt == kShadowInt8;
   const int margin_mode = plan.exact ? 0 : (plan.path == B2F_PATH_UMMA_BF16 ? (i8 ? 4 : (idx->worst_case_margin ? 3 : 2)) : 1);
   pass_init_kernel<<<nqp, 128, 0, s>>>(qnormp, qerrp, S.maxnorm2, margin_mode,
                                        static_cast<float>(idx->margin_ppm * 1e-6 * 1.0000001), static_cast<float>(kUScan),
                                        W.margin, W.cnt, W.ovf, (tensor || tensor_qs) ? W.cnt2 : nullptr, n_areas,
-                                       one_launch ? W.hist : nullptr, W.hkey0, W.hshift, W.tau);
+                                       (tensor || tensor_qs) ? W.hist : nullptr, W.hkey0, W.hshift, W.tau);
   st.launches += 1;
 
   if (tensor_qs) {
@@ -888,12 +887,12 @@ int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q3
     a.prefetch = sel ? 0 : idx->l2_prefetch;
     if (!sel) {
       a.dense_quarters = std::min(4, std::max(1, (4 * k + 2 * pairs * 32 - 1) / (2 * pairs * 32)));
-      a.first_wait_cycles = (idx->tighten && N >= 4ll * pairs * kQsTileRows && a.dense_quarters < 4) ? 100000 : 0;
+      a.first_wait_cycles = (N >= 4ll * pairs * kQsTileRows && a.dense_quarters < 4) ? 100000 : 0;
     } else {
       // the same protocol on the selected rows: a quarter of the first listed tiles holds about `density` x 32 of them
       const double rows_q = 2.0 * pairs * 32 * static_cast<double>(sel->count) / (static_cast<double>(te) * kQsTileRows);
       a.dense_quarters = static_cast<int>(std::min(4.0, std::max(1.0, std::ceil(4.0 * k / rows_q))));
-      a.first_wait_cycles = (idx->tighten && te >= 4 * pairs && a.dense_quarters < 4) ? 100000 : 0;
+      a.first_wait_cycles = (te >= 4 * pairs && a.dense_quarters < 4) ? 100000 : 0;
     }
     {
       ProfScope ps(idx, S, 0);
@@ -911,150 +910,95 @@ int enqueue_pass(b2f_index* idx, Shard& S, const PassPlan& plan, const float* q3
     st.launches += 1;
     st.phases += 1;
     st.qs_passes += 1;
-    ProfScope ps(idx, S, 1);
-    int PS = 1024;
-    while (PS < plan.S) PS <<= 1;
-    int P = 8192;
-    while (P < PS) P <<= 1;
-    finalize_kernel<<<nqp, kFinThreads, static_cast<size_t>(P + PS) * sizeof(uint64_t), s>>>(
-        W.cand[0], W.gath, W.cnt, C, k, W.margin, plan.S, plan.cap_a, n_areas, W.cnt2, W.ovf, ovf_dst, q32p,
-        S.x32, S.segs_d, static_cast<int>(S.segs.size()), S.has_ids ? S.idmap : nullptr, D_out, I_out, out_stride, P,
-        W.tau, S.mu);
-    CU_TRY(cudaGetLastError());
-    st.launches += 1;
-    st.passes += 1;
-    return B2F_OK;
+    return enqueue_finalize(idx, S, plan, q32p, nqp, k, plan.cap_a, D_out, I_out, out_stride, ovf_dst);
   }
 
-  int cur = 0;
-  CUtensorMap tmap_p;
   if (tensor) {
+    // ---- TS: one launch over the whole shard, then the fused last step ----
     // shadow = [row tiles x 12 K-blocks x tile rows, 64 columns] bf16; box = 128 x 128 B = 16 KB
     // (int8: 6 K-blocks of 128 bytes per tile, boxes of 3 K-blocks = 12 KB)
+    CUtensorMap tmap_p;
     if (i8) B2F_TRY(make_tmap_bf16(&tmap_p, S.x8, static_cast<uint64_t>(shadow_rows_padded(N)) * kShadow8KBlocks, kBlockK,
                                    3 * kTileRowsCta));
     else B2F_TRY(make_tmap_bf16(&tmap_p, S.x16, static_cast<uint64_t>(shadow_rows_padded(N)) * kNumKBlocks, kBlockK,
                                 kKBlocksPerStage * kTileRowsCta));
-  }
-
-  // Phase boundaries in rows.  Dense phase first, then geometric growth (or, in exact mode,
-  // fixed-size phases that cannot overflow the candidate capacity even if every row passes).
-  int64_t begin = 0;
-  int phase = 0;
-  while (begin < N) {
-    int64_t end;
-    const bool dense = (phase == 0) && !one_launch;
-    if (one_launch) end = N;
-    else if (dense) end = std::min<int64_t>(N, plan.n0);
-    else if (plan.exact) end = std::min<int64_t>(N, begin + (C - k));
-    else if (tensor && idx->tighten) end = N;   // thresholds are tightened inside the kernel
-    else end = std::min<int64_t>(N, begin * std::max(2, idx->growth));
-    int n_override = -1;
-    if (tensor) {
-      const int tb = static_cast<int>(begin / kTileRows);
-      const int te = static_cast<int>((end + kTileRows - 1) / kTileRows);
-      if (end < N) end = static_cast<int64_t>(te) * kTileRows;  // phases end on tile boundaries
-      // filtered: the listed tiles of [tb, te)
-      int lb = tb, le = te;
+    // filtered: the launch walks the listed tiles only
+    const int te = sel ? sel->n_ts : static_cast<int>((N + kTileRows - 1) / kTileRows);
+    const int cap_h = plan.cap_p / 2;   // slots per (query, pair, half tile)
+    UmmaArgs a;
+    a.n_rows = N; a.tile_begin = 0; a.tile_end = te; a.nq = nqp; a.q16 = q16p;
+    a.sel_bits = sel ? sel->bits : nullptr; a.tile_list = sel ? sel->ts_tiles : nullptr;
+    a.qscale = qscalep; a.tscale = S.tscale;
+    a.cand = W.cand[0]; a.C = C; a.S = plan.S; a.cap_p = cap_h;
+    a.max_pairs = n_areas; a.cnt2 = W.cnt2; a.tau = W.tau; a.ovf = W.ovf; a.err = W.err;
+    a.tighten = idx->tighten; a.tighten_adaptive = idx->tighten_adaptive; a.k = k; a.margin = W.margin; a.hist = W.hist; a.hkey0 = W.hkey0; a.hshift = W.hshift;
+    const int pairs = std::min(S.max_pairs, te);
+    // wait for the first thresholds after the first tile: only when that tile's rows can place them (about half of
+    // pairs * 64 rows score above the histogram floor) and the shard is long enough to be worth it
+    if (!sel) {
+      a.first_wait_cycles = (N >= 8ll * pairs * kTileRows && 4ll * k <= static_cast<int64_t>(pairs) * kTileRows) ? 100000 : 0;
+    } else {   // the same rule on the selected rows of the listed tiles
+      const double density = static_cast<double>(sel->count) / (static_cast<double>(te) * kTileRows);
+      a.first_wait_cycles = (te >= 8 * pairs && 4.0 * k <= pairs * kTileRows * density) ? 100000 : 0;
+    }
+    {
+      ProfScope ps(idx, S, 0);
+      const dim3 g(2 * pairs);
       if (sel) {
-        lb = static_cast<int>(std::lower_bound(sel->ts_host.begin(), sel->ts_host.end(), tb) - sel->ts_host.begin());
-        le = static_cast<int>(std::lower_bound(sel->ts_host.begin(), sel->ts_host.end(), te) - sel->ts_host.begin());
+        if (i8) umma_score_select_kernel<true, true><<<g, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
+        else umma_score_select_kernel<false, true><<<g, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
+      } else {
+        if (i8) umma_score_select_kernel<true, false><<<g, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
+        else umma_score_select_kernel<false, false><<<g, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
       }
-      UmmaArgs a;
-      a.n_rows = N; a.tile_begin = lb; a.tile_end = le; a.nq = nqp; a.q16 = q16p;
-      a.sel_bits = sel ? sel->bits : nullptr; a.tile_list = sel ? sel->ts_tiles : nullptr;
-      a.qscale = qscalep; a.tscale = S.tscale;
-      a.dense = dense ? 1 : 0; a.cand = W.cand[cur]; a.C = C; a.S = plan.S; a.cap_p = cap_h;
-      a.max_pairs = n_areas; a.cnt2 = W.cnt2; a.tau = W.tau; a.ovf = W.ovf; a.err = W.err;
-      a.tighten = idx->tighten; a.tighten_adaptive = idx->tighten_adaptive; a.k = k; a.margin = W.margin; a.hist = W.hist; a.hkey0 = W.hkey0; a.hshift = W.hshift;
-      const int pairs = std::min(S.max_pairs, le - lb);
-      // wait for the first thresholds after the first tile: only when that tile's rows can place them (about half of
-      // pairs * 64 rows score above the histogram floor) and the shard is long enough to be worth it
-      a.count_exact_lower_bound = one_launch ? 1 : 0;
-      if (!sel) {
-        a.first_wait_cycles = (one_launch && N >= 8ll * pairs * kTileRows && 4ll * k <= static_cast<int64_t>(pairs) * kTileRows) ? 100000 : 0;
-      } else {   // the same rule on the selected rows of the listed tiles
-        const double density = static_cast<double>(sel->count) / (static_cast<double>(sel->n_ts) * kTileRows);
-        a.first_wait_cycles = (one_launch && le - lb >= 8 * pairs && 4.0 * k <= pairs * kTileRows * density) ? 100000 : 0;
-      }
-      if (pairs > 0) {   // a filtered phase may hold no listed tile
-        ProfScope ps(idx, S, 0);
-        const dim3 g(2 * pairs);
-        if (sel) {
-          if (i8) umma_score_select_kernel<true, true><<<g, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
-          else umma_score_select_kernel<false, true><<<g, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
-        } else {
-          if (i8) umma_score_select_kernel<true, false><<<g, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
-          else umma_score_select_kernel<false, false><<<g, kUmmaThreads, kUmmaSmemBytes, s>>>(tmap_p, a);
-        }
-      }
-      st.score_rows += sel ? static_cast<double>(le - lb) * kTileRows
-                           : static_cast<double>(std::min<int64_t>(N, static_cast<int64_t>(te) * kTileRows) - begin);
-    } else {
-      ScanArgs a;
-      a.x32 = S.x32; a.row_begin = begin; a.row_end = end; a.q32 = q32p; a.nq_pass = nqp;
-      a.dense = dense ? 1 : 0; a.dense_row0 = 0; a.cand = W.cand[cur]; a.cnt = W.cnt; a.C = C;
-      a.tau = W.tau; a.tauP = W.tauP; a.ovf = W.ovf; a.sel_bits = sel ? sel->bits : nullptr;
-      const int64_t groups = (end - begin + kScanRows - 1) / kScanRows;
-      const int blocks = static_cast<int>(std::min<int64_t>((groups + 7) / 8, static_cast<int64_t>(S.sm_count)));
-      const size_t sm = scan_smem_bytes(nqp, plan.exact);
-      {
-        ProfScope ps(idx, S, 0);
-        const dim3 g(std::max(blocks, 1));
-        if (sel) {
-          if (plan.exact) scan_kernel<true, true><<<g, kScanThreads, sm, s>>>(a);
-          else scan_kernel<false, true><<<g, kScanThreads, sm, s>>>(a);
-        } else {
-          if (plan.exact) scan_kernel<true, false><<<g, kScanThreads, sm, s>>>(a);
-          else scan_kernel<false, false><<<g, kScanThreads, sm, s>>>(a);
-        }
-      }
-      st.score_rows += static_cast<double>(end - begin);
-      if (dense) n_override = static_cast<int>(end - begin);
     }
     CU_TRY(cudaGetLastError());
-    if (tensor && end >= N) {   // the last refresh of a TS pass is part of finalize_kernel
-      st.launches += 1;
-      st.phases += 1;
-      begin = end;
-      ++phase;
-      break;
+    st.score_rows += sel ? static_cast<double>(te) * kTileRows : static_cast<double>(N);
+    st.launches += 1;
+    st.phases += 1;
+    return enqueue_finalize(idx, S, plan, q32p, nqp, k, cap_h, D_out, I_out, out_stride, ovf_dst);
+  }
+
+  // ---- SIMT scans: a dense first phase, then geometric growth (or, in exact mode, fixed-size phases that
+  // cannot overflow the candidate capacity even if every row passes), with refresh_kernel between phases ----
+  int cur = 0;
+  int64_t begin = 0;
+  while (begin < N) {
+    const bool dense = begin == 0;   // first phase: every score is stored
+    int64_t end;
+    if (dense) end = std::min<int64_t>(N, plan.n0);
+    else if (plan.exact) end = std::min<int64_t>(N, begin + (C - k));
+    else end = std::min<int64_t>(N, begin * std::max(2, idx->growth));
+    ScanArgs a;
+    a.x32 = S.x32; a.row_begin = begin; a.row_end = end; a.q32 = q32p; a.nq_pass = nqp;
+    a.dense = dense ? 1 : 0; a.dense_row0 = 0; a.cand = W.cand[cur]; a.cnt = W.cnt; a.C = C;
+    a.tau = W.tau; a.tauP = W.tauP; a.ovf = W.ovf; a.sel_bits = sel ? sel->bits : nullptr;
+    const int64_t groups = (end - begin + kScanRows - 1) / kScanRows;
+    const int blocks = static_cast<int>(std::min<int64_t>((groups + 7) / 8, static_cast<int64_t>(S.sm_count)));
+    const size_t sm = scan_smem_bytes(nqp, plan.exact);
+    {
+      ProfScope ps(idx, S, 0);
+      const dim3 g(std::max(blocks, 1));
+      if (sel) {
+        if (plan.exact) scan_kernel<true, true><<<g, kScanThreads, sm, s>>>(a);
+        else scan_kernel<false, true><<<g, kScanThreads, sm, s>>>(a);
+      } else {
+        if (plan.exact) scan_kernel<true, false><<<g, kScanThreads, sm, s>>>(a);
+        else scan_kernel<false, false><<<g, kScanThreads, sm, s>>>(a);
+      }
     }
-    if (tensor && idx->tighten && phase == 0) {   // TS bootstrap: select in shared memory + histogram seed
+    st.score_rows += static_cast<double>(end - begin);
+    CU_TRY(cudaGetLastError());
+    {
       ProfScope ps(idx, S, 1);
-      int P = 4096;
-      while (P < plan.n0 + plan.S && P < 16384) P <<= 1;   // longer lists are gathered to global memory
-      bootstrap_select_kernel<<<nqp, kFinThreads, static_cast<size_t>(P) * sizeof(uint64_t), s>>>(
-          W.cand[cur], W.cand[cur ^ 1], W.gath, W.cnt, C, k, W.margin, W.tau, plan.S, cap_h, n_areas, W.cnt2,
-          W.ovf, W.hist, W.hkey0, W.hshift, P);
-    } else {
-      ProfScope ps(idx, S, 1);
-      refresh_kernel<<<nqp, kSelThreads, 0, s>>>(W.cand[cur], W.cand[cur ^ 1], W.gath, W.cnt, C, k, plan.exact ? 1 : 0,
-                                                W.margin, W.tau, W.tauP, n_override, plan.S, cap_h,
-                                                tensor ? n_areas : 0, W.cnt2, W.ovf,
-                                                (tensor && idx->tighten && end < N) ? W.hist : nullptr, W.hkey0, W.hshift);
+      refresh_kernel<<<nqp, kSelThreads, 0, s>>>(W.cand[cur], W.cand[cur ^ 1], W.cnt, C, k, plan.exact ? 1 : 0,
+                                                W.margin, W.tau, W.tauP, dense ? static_cast<int>(end - begin) : -1, W.ovf);
     }
     CU_TRY(cudaGetLastError());
     cur ^= 1;
     st.launches += 2;
     st.phases += 1;
     begin = end;
-    ++phase;
-  }
-  if (tensor) {
-    ProfScope ps(idx, S, 1);
-    int PS = 1024;                       // survivors (bufB): >= S
-    while (PS < plan.S) PS <<= 1;
-    int P = 8192;                        // gathered list (bufA); longer lists go through global memory
-    while (P < PS) P <<= 1;
-    finalize_kernel<<<nqp, kFinThreads, static_cast<size_t>(P + PS) * sizeof(uint64_t), s>>>(
-        W.cand[cur], W.gath, W.cnt, C, k, W.margin, plan.S, cap_h, n_areas, W.cnt2, W.ovf, ovf_dst, q32p,
-        S.x32, S.segs_d, static_cast<int>(S.segs.size()), S.has_ids ? S.idmap : nullptr, D_out, I_out, out_stride, P,
-        idx->tighten ? W.tau : nullptr, S.mu);
-    CU_TRY(cudaGetLastError());
-    st.launches += 1;
-    st.passes += 1;
-    return B2F_OK;
   }
   {
     ProfScope ps(idx, S, 1);
@@ -1125,7 +1069,6 @@ int enqueue_search(b2f_index* idx, Shard& S, const float* q_d, int64_t nq, int k
       CU_TRY(cudaFuncSetAttribute(umma_qs_score_select_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kQsSmemLimit));
       CU_TRY(cudaFuncSetAttribute(umma_qs_score_select_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kQsSmemLimit));
       CU_TRY(cudaFuncSetAttribute(finalize_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * 8192 * 8));   // P + PS records
-      CU_TRY(cudaFuncSetAttribute(bootstrap_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 16384 * 8));
       attr_set[S.dev & 63] = true;
     }
   } else {
@@ -2293,17 +2236,17 @@ static int build_selector_part(b2f_index* idx, Shard& S, const SelDesc& desc_hos
   unsigned long long count = 0;
   std::memcpy(&count, flags.data(), 8);
   P.count = static_cast<int64_t>(count);
-  std::vector<int> qs;
+  std::vector<int> qs, ts;
   for (int64_t t = 0; t < n_qs; ++t)
     if (flags[8 + t]) qs.push_back(static_cast<int>(t));
   for (int64_t t = 0; t < n_ts; ++t)
-    if (flags[8 + n_qs + t]) P.ts_host.push_back(static_cast<int>(t));
+    if (flags[8 + n_qs + t]) ts.push_back(static_cast<int>(t));
   P.n_qs = static_cast<int>(qs.size());
-  P.n_ts = static_cast<int>(P.ts_host.size());
+  P.n_ts = static_cast<int>(ts.size());
   B2F_TRY(dev_alloc(&P.qs_tiles, qs.size()));
-  B2F_TRY(dev_alloc(&P.ts_tiles, P.ts_host.size()));
+  B2F_TRY(dev_alloc(&P.ts_tiles, ts.size()));
   if (!qs.empty()) CU_TRY(cudaMemcpy(P.qs_tiles, qs.data(), qs.size() * 4, cudaMemcpyHostToDevice));
-  if (!P.ts_host.empty()) CU_TRY(cudaMemcpy(P.ts_tiles, P.ts_host.data(), P.ts_host.size() * 4, cudaMemcpyHostToDevice));
+  if (!ts.empty()) CU_TRY(cudaMemcpy(P.ts_tiles, ts.data(), ts.size() * 4, cudaMemcpyHostToDevice));
   return B2F_OK;
 }
 
@@ -2407,14 +2350,14 @@ int b2f_set_option(b2f_index* idx, const char* key, int64_t value) {
     if (value < 0 || value > 8) return fail(B2F_ERR_INVALID, "l2_prefetch must be 0 (off) or a distance of 1..8 tiles");
     idx->l2_prefetch = static_cast<int>(value);
   } else if (k == "tighten") {
-    if (value < 0 || value > 1000000) return fail(B2F_ERR_INVALID, "tighten must be 0 (off) or a pause in ns <= 1e6");
+    if (value < 1 || value > 1000000)
+      return fail(B2F_ERR_INVALID, "tighten must be a refresher pause in ns in [1, 1e6] (0, the phased schedule without "
+                                   "in-kernel tightening, was retired)");
     idx->tighten = static_cast<int>(value);
   } else if (k == "tighten_adaptive") {
     idx->tighten_adaptive = value ? 1 : 0;
   } else if (k == "xchg_defer") {
     idx->xchg.defer = value ? 1 : 0;
-  } else if (k == "bootstrap") {
-    idx->bootstrap = value ? 1 : 0;
   } else if (k == "worst_case_margin") {
     idx->worst_case_margin = value ? 1 : 0;
   } else if (k == "profile") {

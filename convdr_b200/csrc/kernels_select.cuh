@@ -13,15 +13,13 @@ namespace b2f {
 constexpr int kSelThreads = 256;
 constexpr int kXchgMaxWorldMerge = 64;   // lists one merge handles (ranks of the exchange / shards of an index)
 constexpr int kSortCap = 2048;  // == B2F_MAX_K
-constexpr int kTightenBuckets = 512;  // == kHistBuckets of kernels_umma.cuh
-constexpr int kTightenStride = kTightenBuckets + kTightenBuckets / 16;  // == kHistStride: [512 fine][32 coarse] per query
 
 struct Seg {  // rows [local_start, local_start+count) of a shard carry ids global_start + i
   int64_t local_start, count, global_start;
 };
 
 struct SelectSmem {
-  unsigned int hist[512];   // 256 radix buckets; 512 when seeding the tightening histogram
+  unsigned int hist[256];   // radix buckets
   unsigned int warp_tot[kSelThreads / 32];
   unsigned int digit, remaining, count, nvalid;
 };
@@ -111,131 +109,41 @@ __device__ int block_compact(const uint64_t* __restrict__ in, int n, uint64_t T,
   return m;
 }
 
-// Gather the valid entries of a segmented candidate list (survivors [0,m) + one private area per
-// CTA pair, see kernels_umma.cuh UmmaArgs) into a dense array; returns the entry count, zeroes the
-// consumed private slots and clears the per-pair counters for the next launch.
-__device__ int block_gather_segments(uint64_t* __restrict__ in, int m, int S, int cap_p, int max_pairs,
-                                     int* __restrict__ cnt2q, uint64_t* __restrict__ gath, SelectSmem& sm,
-                                     int* seg_off /* smem [max_pairs] */) {
-  for (int i = threadIdx.x; i < m; i += kSelThreads) gath[i] = in[i];
-  int total = 0;
-  for (int p0 = 0; p0 < max_pairs; p0 += kSelThreads) {   // exclusive scan of the per-pair counts
-    const int p = p0 + threadIdx.x;
-    const unsigned int c = (p < max_pairs) ? static_cast<unsigned int>(cnt2q[p]) : 0u;
-    const unsigned int inc = block_inclusive_scan(c, sm);
-    if (p < max_pairs) seg_off[p] = total + static_cast<int>(inc - c);
-    if (threadIdx.x == kSelThreads - 1) sm.count = inc;
-    __syncthreads();
-    total += static_cast<int>(sm.count);
-    __syncthreads();
-  }
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  for (int p = warp; p < max_pairs; p += kSelThreads / 32) {
-    const int c = (p + 1 < max_pairs ? seg_off[p + 1] : total) - seg_off[p];
-    uint64_t* src = in + S + static_cast<int64_t>(p) * cap_p;
-    uint64_t* dst = gath + m + seg_off[p];
-    for (int e = lane; e < c; e += 32) {
-      dst[e] = src[e];
-      src[e] = 0ull;   // invariant of the tensor engine: private areas are all-zero between launches
-    }
-  }
-  __syncthreads();
-  for (int p = threadIdx.x; p < max_pairs; p += kSelThreads) cnt2q[p] = 0;
-  __syncthreads();
-  return m + total;
-}
-
-// Threshold refresh between phases, one block per query of the pass.
+// Threshold refresh between the phases of the SIMT scans, one block per query of the pass.
 //   approx mode (exact == 0): tau = (k-th largest approximate score) - margin[q], rounded down;
 //       survivors are the records with score >= tau.  Any true top-k row has an approximate score
 //       within margin/2 of its exact score, so it survives (DESIGN.md "exactness argument").
 //   exact mode: scores are final; tauP = the k-th largest record, survivors are exactly the top k.
 // With fewer than k valid records nothing can be rejected yet (tau = -inf / tauP = 0).
 __global__ void __launch_bounds__(kSelThreads) refresh_kernel(
-    uint64_t* __restrict__ cand_in, uint64_t* __restrict__ cand_out, uint64_t* __restrict__ gath,
-    int* __restrict__ cnt, int C, int k, int exact, const float* __restrict__ margin,
-    float* __restrict__ tau, uint64_t* __restrict__ tauP, int n_override, int S, int cap_p, int max_pairs,
-    int* __restrict__ cnt2, int* __restrict__ ovf, unsigned int* __restrict__ hist /* [nq][kTightenBuckets] or null */,
-    uint32_t* __restrict__ hkey0, int* __restrict__ hshift) {
+    const uint64_t* __restrict__ cand_in, uint64_t* __restrict__ cand_out, int* __restrict__ cnt, int C, int k,
+    int exact, const float* __restrict__ margin, float* __restrict__ tau, uint64_t* __restrict__ tauP,
+    int n_override, int* __restrict__ ovf) {
   __shared__ SelectSmem sm;
-  __shared__ int seg_off[256];
   const int q = blockIdx.x;
   const uint64_t* in = cand_in + static_cast<int64_t>(q) * C;
   uint64_t* out = cand_out + static_cast<int64_t>(q) * C;
-  int n;
-  int limit = C;
-  if (max_pairs > 0) {   // segmented list written by the tensor engine
-    uint64_t* g = gath + static_cast<int64_t>(q) * C;
-    n = block_gather_segments(cand_in + static_cast<int64_t>(q) * C, min(cnt[q], S), S, cap_p, max_pairs,
-                              cnt2 + q * max_pairs, g, sm, seg_off);
-    in = g;
-    limit = S;
-  } else {
-    n = n_override >= 0 ? n_override : cnt[q];
-    if (n > C) n = C;
-  }
+  int n = n_override >= 0 ? n_override : cnt[q];
+  if (n > C) n = C;
   const int nvalid = block_count_valid(in, n, sm);
   uint64_t T = 0ull;
   float t = -INFINITY;
-  uint32_t kth_key = 0xffffffffu;   // key of the k-th best approximate score (approx mode)
   if (nvalid >= k) {
     const uint64_t prefix = block_kth_prefix(in, n, k, exact ? 8 : 4, sm);
     if (exact) {
       T = prefix;
       t = key2f(static_cast<uint32_t>(prefix >> 32));
     } else {
-      kth_key = static_cast<uint32_t>(prefix >> 32);
       t = __fsub_rd(key2f(static_cast<uint32_t>(prefix >> 32)), margin[q]);
       T = static_cast<uint64_t>(fkey(t)) << 32;
     }
   }
-  const int m = block_compact(in, n, T, out, limit, sm);
+  const int m = block_compact(in, n, T, out, C, sm);
   if (threadIdx.x == 0) {
-    cnt[q] = min(m, limit);
+    cnt[q] = min(m, C);
     tau[q] = t;
     tauP[q] = T;
-    if (m > limit) ovf[q] = 1;   // more rows within the error margin of the k-th score than the list holds
-  }
-  if (hist != nullptr) {
-    // Seed the tensor engine's tightening histogram (kernels_umma.cuh, refresher role): buckets of
-    // 2^shift score keys starting at the key of the k-th best approximate score seen so far, sized
-    // so that kTightenBuckets of them span 4x the distance from that score to the best one (a
-    // Gaussian tail moves ~1.5x that distance from 5e3 to 4e7 rows; beyond the range the last
-    // bucket absorbs everything and tightening simply stops — never a correctness matter).
-    const uint32_t key0 = kth_key;
-    int shift = 0;
-    if (key0 != 0xffffffffu) {
-      uint32_t kmax = 0;
-      for (int i = threadIdx.x; i < n; i += kSelThreads) kmax = max(kmax, static_cast<uint32_t>(in[i] >> 32));
-#pragma unroll
-      for (int s2 = 16; s2 >= 1; s2 >>= 1) kmax = max(kmax, __shfl_xor_sync(0xffffffffu, kmax, s2));
-      if (threadIdx.x == 0) sm.digit = 0;
-      __syncthreads();
-      if ((threadIdx.x & 31) == 0) atomicMax(&sm.digit, kmax);
-      __syncthreads();
-      kmax = sm.digit;
-      __syncthreads();
-      const uint64_t span = 4ull * static_cast<uint64_t>(kmax - key0) + 1ull;
-      while ((static_cast<uint64_t>(kTightenBuckets) << shift) < span) ++shift;
-    }
-    for (int b = threadIdx.x; b < kTightenBuckets; b += kSelThreads) sm.hist[b] = 0;
-    __syncthreads();
-    if (key0 != 0xffffffffu) {
-      for (int i = threadIdx.x; i < n; i += kSelThreads) {
-        const uint32_t key = static_cast<uint32_t>(in[i] >> 32);
-        if (in[i] != 0ull && key >= key0)
-          atomicAdd(&sm.hist[min(static_cast<uint32_t>(kTightenBuckets - 1), (key - key0) >> shift)], 1u);
-      }
-    }
-    __syncthreads();
-    for (int b = threadIdx.x; b < kTightenBuckets; b += kSelThreads)
-      hist[static_cast<int64_t>(q) * kTightenStride + b] = sm.hist[b];
-    if (threadIdx.x < kTightenBuckets / 16) {
-      unsigned int c = 0;
-      for (int j = 0; j < 16; ++j) c += sm.hist[16 * threadIdx.x + j];
-      hist[static_cast<int64_t>(q) * kTightenStride + kTightenBuckets + threadIdx.x] = c;
-    }
-    if (threadIdx.x == 0) { hkey0[q] = key0; hshift[q] = shift; }
+    if (m > C) ovf[q] = 1;   // more rows within the error margin of the k-th score than the list holds
   }
 }
 
@@ -333,8 +241,8 @@ __global__ void __launch_bounds__(kSelThreads) final_kernel(
 }
 
 // ---------------------------------------------------------------------------------------------
-// Fused last step of a tensor-engine (TS) pass, one 1024-thread block per query:
-//   gather (survivors of the bootstrap + every CTA pair's private area)  ->  radix-select the k-th best
+// Fused last step of a tensor-engine pass (both variants), one kFinThreads-thread block per query:
+//   gather (every CTA's or CTA pair's private area)  ->  radix-select the k-th best
 //   approximate score  ->  keep everything within the error margin of it  ->  exact fp64-accumulated
 //   rescoring (one warp per survivor, two rows in flight per warp)  ->  bitonic sort by the total
 //   order  ->  row -> id translation, (D, I) rows and the overflow flag.
@@ -345,10 +253,9 @@ __global__ void __launch_bounds__(kSelThreads) final_kernel(
 constexpr int kFinThreads = 512;   // two blocks per SM: 173 queries fit one wave on 148 SMs
 
 struct FinSmem {
-  unsigned int hist[512];   // 256 radix buckets; 512 when seeding the tightening histogram
+  unsigned int hist[256];   // radix buckets
   unsigned int warp_tot[kFinThreads / 32];
   unsigned int digit, remaining, count, nvalid;
-  int seg_off[129];
 };
 
 __device__ __forceinline__ unsigned int fin_scan256(unsigned int v, FinSmem& sm) {
@@ -368,8 +275,8 @@ __device__ __forceinline__ unsigned int fin_scan256(unsigned int v, FinSmem& sm)
   return v + base;
 }
 
-// Front part shared by bootstrap_select_kernel and finalize_kernel (all kFinThreads threads call it):
-// gather the segmented list of query q (survivors [0,m) + one private area per CTA pair) into `bufA`
+// Front part of finalize_kernel (all kFinThreads threads call it):
+// gather the segmented list of query q ([0,m) + one private area per CTA or CTA pair) into `bufA`
 // (shared memory, P records; longer lists go to `gath_q` in global memory), radix-select the key of
 // the k-th best approximate score, derive the survivor threshold T = fkey(kth - margin) << 32.
 struct FinFront {
@@ -498,79 +405,6 @@ __device__ __forceinline__ FinFront fin_front(const uint64_t* __restrict__ list,
     f.T = static_cast<uint64_t>(fkey(f.tau)) << 32;
   }
   return f;
-}
-
-// Bootstrap step of a tensor-engine (TS) pass, one 512-thread block per query, after the dense launch:
-// select the k-th best approximate score of the first n0 rows (list held in shared memory), publish
-// tau, keep the survivors (records >= tau) in [0, S) of `cand_out`, seed the tightening histogram of
-// the main launch (kernels_umma.cuh, refresher role) and clear the per-pair counters.
-__global__ void __launch_bounds__(kFinThreads, 2) bootstrap_select_kernel(
-    const uint64_t* __restrict__ cand_in, uint64_t* __restrict__ cand_out, uint64_t* __restrict__ gath,
-    int* __restrict__ cnt, int C, int k, const float* __restrict__ margin, float* __restrict__ tau, int S, int cap_p,
-    int max_pairs, int* __restrict__ cnt2, int* __restrict__ ovf, unsigned int* __restrict__ hist,
-    uint32_t* __restrict__ hkey0, int* __restrict__ hshift, int P) {
-  extern __shared__ __align__(16) uint64_t fin_buf[];   // [P]
-  __shared__ FinSmem sm;
-  const int q = blockIdx.x;
-  const int tid = threadIdx.x, lane = tid & 31;
-  const FinFront f = fin_front(cand_in + static_cast<int64_t>(q) * C, gath + static_cast<int64_t>(q) * C, min(cnt[q], S), S,
-                               cap_p, max_pairs, cnt2 + q * max_pairs, k, margin[q], 0ull, fin_buf, P, sm);
-  uint64_t* out = cand_out + static_cast<int64_t>(q) * C;
-  // survivors -> [0, S) of the other list
-  for (int i0 = 0; i0 < f.n; i0 += kFinThreads) {
-    const int i = i0 + tid;
-    const uint64_t rec = (i < f.n) ? f.in[i] : 0ull;
-    const bool keep = rec != 0ull && rec >= f.T;
-    const unsigned int b = __ballot_sync(0xffffffffu, keep);
-    if (b) {
-      unsigned int base = 0;
-      if (lane == 0) base = atomicAdd(&sm.count, __popc(b));
-      base = __shfl_sync(0xffffffffu, base, 0);
-      const unsigned int pos = base + __popc(b & ((1u << lane) - 1u));
-      if (keep && pos < static_cast<unsigned int>(S)) out[pos] = rec;
-    }
-  }
-  // histogram seed: buckets of 2^shift keys from the k-th key, kTightenBuckets of them spanning 4x the
-  // distance to the best key seen (see refresh_kernel)
-  uint32_t kmax = 0;
-  for (int i = tid; i < f.n; i += kFinThreads) kmax = max(kmax, static_cast<uint32_t>(f.in[i] >> 32));
-#pragma unroll
-  for (int s2 = 16; s2 >= 1; s2 >>= 1) kmax = max(kmax, __shfl_xor_sync(0xffffffffu, kmax, s2));
-  if (tid == 0) sm.digit = 0;
-  for (int b = tid; b < kTightenBuckets; b += kFinThreads) sm.hist[b] = 0;
-  __syncthreads();
-  if (lane == 0) atomicMax(&sm.digit, kmax);
-  __syncthreads();
-  kmax = sm.digit;
-  const uint32_t key0 = f.kth_key;
-  int shift = 0;
-  if (key0 != 0xffffffffu) {
-    const uint64_t span = 4ull * static_cast<uint64_t>(kmax - key0) + 1ull;
-    while ((static_cast<uint64_t>(kTightenBuckets) << shift) < span) ++shift;
-    for (int i0 = 0; i0 < f.n; i0 += kFinThreads) {
-      const int i = i0 + tid;
-      const uint64_t rec = (i < f.n) ? f.in[i] : 0ull;
-      const uint32_t key = static_cast<uint32_t>(rec >> 32);
-      const bool on = rec != 0ull && key >= key0;
-      hist_add_aggregated(sm.hist, on, on ? min(static_cast<uint32_t>(kTightenBuckets - 1), (key - key0) >> shift) : 0u);
-    }
-  }
-  __syncthreads();
-  for (int b = tid; b < kTightenBuckets; b += kFinThreads) hist[static_cast<int64_t>(q) * kTightenStride + b] = sm.hist[b];
-  if (tid < kTightenBuckets / 16) {
-    unsigned int c = 0;
-    for (int j = 0; j < 16; ++j) c += sm.hist[16 * tid + j];
-    hist[static_cast<int64_t>(q) * kTightenStride + kTightenBuckets + tid] = c;
-  }
-  for (int p = tid; p < max_pairs; p += kFinThreads) cnt2[q * max_pairs + p] = 0;
-  if (tid == 0) {
-    const int msurv = static_cast<int>(sm.count);
-    cnt[q] = min(msurv, S);
-    tau[q] = f.tau;
-    hkey0[q] = key0;
-    hshift[q] = shift;
-    if (msurv > S) ovf[q] = 1;   // more rows within the error margin of the k-th score than the list holds
-  }
 }
 
 __global__ void __launch_bounds__(kFinThreads, 2) finalize_kernel(

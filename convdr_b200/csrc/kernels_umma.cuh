@@ -60,44 +60,34 @@ struct UmmaArgs {
   int tile_begin, tile_end;   // pair tiles of 128 rows
   int nq;                     // valid queries of the pass (<= 256)
   const __nv_bfloat16* q16;   // pass queries, row-major [>= nq, 768] bf16
-  int dense;                  // 1: store every score (bootstrap phase), 0: threshold filter
-  // Candidate list of query q: cand[q*C .. q*C+C).  [0, S) holds the survivors of earlier phases
-  // (written by refresh_kernel); the rest is split in `max_pairs` private areas of `cap_p` slots,
-  // TWO per CTA pair (one per half of a tile's 64 rows), so the thread that owns (query, pair, half)
-  // appends without any atomic.
+  // Candidate list of query q: cand[q*C .. q*C+C).  [0, S) is not written by this kernel; the rest is
+  // split in `max_pairs` private areas of `cap_p` slots, TWO per CTA pair (one per half of a tile's 64
+  // rows), so the thread that owns (query, pair, half) appends without any atomic.
   uint64_t* cand;
   int C, S, cap_p, max_pairs; // max_pairs = number of areas = 2 x CTA pairs of the largest grid
   int* cnt2;                  // [nq][max_pairs] entries written to each area in this launch
-  float* tau;                 // [nq] thresholds (raised in-kernel when tighten != 0)
+  float* tau;                 // [nq] thresholds, -inf at the start of the pass, raised in-kernel
   int* ovf;                   // [nq] set when a private area was too small
   int* err;                   // device error flag (barrier timeout)
-  // In-kernel threshold tightening (see the refresher role below).  Every hit is also counted in a
-  // per-query histogram over the score-key range above the bootstrap's k-th score:
+  // In-kernel threshold tightening (see the refresher role below).  Every hit is also counted, at s~ - eps
+  // (a lower bound of its EXACT score), in a per-query histogram over the score keys below R:
   //   bucket(key) = min(kHistBuckets-1, (key - hkey0[q]) >> hshift[q])   for key >= hkey0[q]
-  // so "k rows seen so far score at least edge(b)" is one suffix sum away.  Two ways to place the
-  // buckets (host option "bootstrap"):
-  //   0 (default): no bootstrap at all.  hkey0 = ((fkey(R) >> 17) - 511) << 17, hshift = 17 with
-  //      R >= any |score| of the query (Cauchy-Schwarz): 64 buckets per binade (1.6 % of the score)
-  //      over the eight binades below R.  tau starts at -inf, the first tile of every pair passes
-  //      entirely, and the thresholds rise from there — ONE launch streams the whole shard.
-  //   1: a dense bootstrap launch + bootstrap_select_kernel place 512 linear buckets above the k-th
-  //      best score of the first rows.
-  int tighten;                // >0: the idle warp of each CTA keeps raising tau[q] while the stream runs;
-                              //     the value is the minimum pause between its rounds in ns
+  // so "k rows seen so far score at least edge(b)" is one suffix sum away.  pass_init_kernel places the
+  // buckets: hkey0 = ((fkey(R) >> 17) - 511) << 17, hshift = 17 with R >= any |score| of the query
+  // (Cauchy-Schwarz): 64 buckets per binade (1.6 % of the score) over the eight binades below R.  tau
+  // starts at -inf, the first tile of every pair passes entirely, and the thresholds rise from there —
+  // ONE launch streams the whole shard.
+  int tighten;                // minimum pause of the refresher warp between its rounds, ns
   int tighten_adaptive;       // 1: the pause grows with the time since the kernel started (elapsed / 4, capped at
                               //     50 us): the pass rate falls like k / rows_seen, so a threshold of bounded
                               //     relative age costs a bounded fraction of extra hits whatever the moment,
                               //     and a launch needs ~50 polling rounds instead of thousands
   int k;
-  int count_exact_lower_bound; // 1 (one-launch schedule): hits are counted at s~ - eps, a lower bound of the EXACT score,
-                              //   so "k hits at or above edge e" bounds the k-th exact score itself and tau = e - eps;
-                              // 0 (phased schedules, whose histogram is seeded with raw approximate keys): count at
-                              //   s~, tau = e - 2 eps
-  int first_wait_cycles;      // one-launch schedule: after its first tile an epilogue thread waits this long at most
-                              // for its query's first threshold (0: no wait)
+  int first_wait_cycles;      // after its first tile an epilogue thread waits this long at most for its query's
+                              // first threshold (0: no wait)
   const float* margin;        // [nq] 2*eps of the prefilter
-  unsigned int* hist;         // [nq][kHistStride], initialised by pass_init_kernel / bootstrap_select_kernel
-  const uint32_t* hkey0;      // [nq] key of the bootstrap's k-th best approximate score (0xffffffff: none yet)
+  unsigned int* hist;         // [nq][kHistStride], initialised by pass_init_kernel
+  const uint32_t* hkey0;      // [nq] key of the lowest bucket
   const int* hshift;          // [nq] log2(keys per bucket)
   const float* qscale;        // int8 shadow: [nq] query scales sq (q16 then points at the int8 codes)
   const float4* tscale;       // int8 shadow: [row tiles of 32] tile scales {st, RD(1/st), RU(1/st), 0}
@@ -396,6 +386,62 @@ __device__ __forceinline__ bool any_ge32_s32(const uint32_t* v, int tau) {
   return r != 0u;
 }
 
+// One round of the refresher warp of both tensor-engine kernels for query q (the whole warp calls it): find
+// the highest histogram bucket b with >= k hits in buckets >= b and raise tau[q] to edge(b) - eps.  Hits
+// are counted at s~ - eps, a lower bound of their EXACT scores, so at least k rows seen so far have an exact
+// score >= edge(b) and the k-th best exact score of any superset is >= it; every true top-k row then has
+// s~ >= edge(b) - eps.  The bound of DESIGN.md section 4 holds for every intermediate value, whatever the
+// interleaving: counts only grow, and a stale read is a smaller suffix sum, i.e. a lower, still valid,
+// threshold.  key0: hkey0[q] (the caller's copy); last[qi]: the caller's cache of the thresholds it
+// published for its first four queries.
+__device__ __forceinline__ void refresh_threshold(const unsigned int* hist, uint32_t key0, const int* hshift,
+                                                  const float* margin, float* tau, int k, int q, int qi, int lane,
+                                                  float (&last)[4]) {
+  // lane l owns buckets [16l, 16l+16).  One 128-byte read of the 32 coarse counters per round; only the lane
+  // where the suffix sum crosses k reads its 16 fine buckets (192 B per query and round instead of 2 KB: the
+  // polling shares the L2 -> SM path with the 6 TB/s passage stream).
+  const unsigned int* hq = hist + static_cast<int64_t>(q) * kHistStride;
+  const unsigned int mine = __ldcv(hq + kHistBuckets + lane);
+  unsigned int suf = mine;               // hits in the buckets of lanes >= this one
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const unsigned int t = __shfl_down_sync(0xffffffffu, suf, o);
+    if (lane + o < 32) suf += t;
+  }
+  const unsigned int kk = static_cast<unsigned int>(k);
+  unsigned int above = suf - mine;
+  int b = -1;
+  if (suf >= kk && above < kk) {         // exactly one lane: walk its 16 fine buckets from the top
+    const uint4* hp = reinterpret_cast<const uint4*>(hq) + 4 * lane;
+#pragma unroll
+    for (int u = 3; u >= 0; --u) {
+      const uint4 h4 = __ldcv(hp + u);
+      const unsigned int c4[4] = {h4.x, h4.y, h4.z, h4.w};
+#pragma unroll
+      for (int j = 3; j >= 0; --j) {
+        if (b < 0) {
+          above += c4[j];
+          if (above >= kk) b = 16 * lane + 4 * u + j;
+        }
+      }
+    }
+  }
+  const unsigned int who = __ballot_sync(0xffffffffu, b >= 0);
+  if (who == 0u) return;
+  b = __shfl_sync(0xffffffffu, b, __ffs(who) - 1);
+  if (lane == 0) {
+    const uint64_t edge = static_cast<uint64_t>(key0) + (static_cast<uint64_t>(b) << hshift[q]);
+    if (edge <= 0xff7fffffull) {         // a finite score key
+      const float t = __fsub_rd(key2f(static_cast<uint32_t>(edge)), __fmul_ru(margin[q], 0.5f));   // e - eps
+      const float prev = (qi < 4) ? last[qi] : *reinterpret_cast<volatile float*>(tau + q);
+      if (t > prev) {
+        *reinterpret_cast<volatile float*>(tau + q) = t;
+        if (qi < 4) last[qi] = t;
+      }
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------------
 // The kernel.  Grid = 2 * (number of CTA pairs), cluster (2,1,1), 384 threads:
 //   warp 0 lane 0 : TMA producer (both CTAs stream their own 32 rows of every tile)
@@ -415,8 +461,7 @@ __device__ __forceinline__ bool any_ge32_s32(const uint32_t* v, int tau) {
 // the tile's reciprocal scale), the compare chain stays one instruction
 // per score, and the float score is only formed for a hit.
 // SEL: filtered search.  The roles walk the listed tiles only; the epilogue ANDs the row bitmap word of its 32 rows
-// into the hit mask (and stores empty records for unselected rows in the dense phase), so only selected rows are
-// ever appended or counted in the tightening histogram.
+// into the hit mask, so only selected rows are ever appended or counted in the tightening histogram.
 // ------------------------------------------------------------------------------------------
 template <bool I8, bool SEL>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
@@ -558,18 +603,17 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(mapa_u32(bar_qready, 0));
     }
-    float tau = (q_ok && !a.dense) ? a.tau[q] : INFINITY;
+    float tau = q_ok ? a.tau[q] : INFINITY;
     volatile float* tau_g = a.tau + (q_ok ? q : 0);
     const int area = 2 * pair + half;
     int* my_cnt = a.cnt2 + (q_ok ? q : 0) * a.max_pairs + area;
-    const bool live = a.tighten && q_ok && !a.dense;
-    const uint32_t hkey0 = live ? a.hkey0[q] : 0xffffffffu;
-    const int hshift = live ? a.hshift[q] : 0;
+    const uint32_t hkey0 = q_ok ? a.hkey0[q] : 0xffffffffu;
+    const int hshift = q_ok ? a.hshift[q] : 0;
     unsigned int* my_hist = a.hist + static_cast<int64_t>(q_ok ? q : 0) * kHistStride;
     uint64_t* my_list = a.cand + static_cast<int64_t>(q_ok ? q : 0) * a.C + a.S + static_cast<int64_t>(area) * a.cap_p;
     int n_mine = 0;   // entries this thread appended for (query q, this pair)
     // count a hit in the tightening histogram (fire-and-forget RED; hits are rare)
-    const float eps_cnt = (live && a.count_exact_lower_bound) ? __fmul_ru(a.margin[q], 0.5f) : 0.f;
+    const float eps_cnt = q_ok ? __fmul_ru(a.margin[q], 0.5f) : 0.f;
     auto count_hit = [&](uint32_t bits) {
       const uint32_t key = fkey(__fsub_rd(__uint_as_float(bits), eps_cnt));
       if (key >= hkey0) {
@@ -585,7 +629,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
     for (int ti = a.tile_begin + pair; ti < a.tile_end; ti += npairs, ++it) {
       const int tile = tile_at<SEL>(a.tile_list, ti);
       const uint32_t as = static_cast<uint32_t>(it) % kAccStages, aph = (static_cast<uint32_t>(it) / kAccStages) & 1u;
-      if (it == 1 && live && a.first_wait_cycles > 0) {
+      if (it == 1 && q_ok && a.first_wait_cycles > 0) {
         // The first tile of every pair passed unfiltered (thresholds start at -inf): together those rows place
         // every query's first threshold.  Waiting for it here (bounded) instead of streaming on keeps the
         // private areas from filling with rows the final selection would throw away — at full clocks a pair
@@ -593,8 +637,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
         const long long t0 = clock64();
         while (*tau_g == -INFINITY && clock64() - t0 < a.first_wait_cycles) __nanosleep(256);
       }
-      float tau_new = tau;
-      if (live) tau_new = *tau_g;            // issued before the wait: the L2 latency hides behind it
+      // issued before the wait: the L2 latency hides behind it.  Unpredicated: a padded lane reads tau[0] but its
+      // own tau stays +inf (fmaxf), so it never hits
+      const float tau_new = *tau_g;
       mbar_wait(bar_tfull + 8 * as, aph, a.err);
       tc_fence_after();
       if (I8 && tau_new > tau) u = i8_tau_over_sq(tau_new, sq);
@@ -612,69 +657,42 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
         // one integer threshold for this (query, shadow tile); scores as floats only where they are stored
         const float4 ts = n_valid > 0 ? __ldg(a.tscale + (row0 >> 5)) : make_float4(0.f, INFINITY, INFINITY, 0.f);
         const float st = ts.x;
-        if (a.dense) {
-          if (q_ok && n_mine + kHalfRows <= a.cap_p) {
-            uint64_t* dst = my_list + n_mine;
+        const int T = i8_threshold(u, ts);
+        if (__any_sync(0xffffffffu, any_ge32_s32(v, T))) {
+          uint32_t m = 0;
 #pragma unroll
-            for (int c = 0; c < kHalfRows; c += 2) {
-              ulonglong2 o;
-              o.x = (c < n_valid && ((sel_word >> c) & 1u)) ? pack_cand(i8_score(static_cast<int>(v[c]), sq, st), static_cast<uint32_t>(row0 + c)) : 0ull;
-              o.y = (c + 1 < n_valid && ((sel_word >> (c + 1)) & 1u)) ? pack_cand(i8_score(static_cast<int>(v[c + 1]), sq, st), static_cast<uint32_t>(row0 + c + 1)) : 0ull;
-              *reinterpret_cast<ulonglong2*>(dst + c) = o;
-            }
-          }
-          n_mine += kHalfRows;
-        } else {
-          const int T = i8_threshold(u, ts);
-          if (__any_sync(0xffffffffu, any_ge32_s32(v, T))) {
-            uint32_t m = 0;
+          for (int c = 0; c < kHalfRows; ++c) m |= (static_cast<int>(v[c]) >= T) ? (1u << c) : 0u;
+          if (n_valid < kHalfRows) m &= (n_valid > 0) ? ((1u << n_valid) - 1u) : 0u;   // shard tail
+          if constexpr (SEL) m &= sel_word;
+          uint32_t any = __reduce_or_sync(0xffffffffu, m);
+          if (__popc(any) > 6) {   // busy word: unrolled predicated stores, v[] stays in registers
+            if (m) {
 #pragma unroll
-            for (int c = 0; c < kHalfRows; ++c) m |= (static_cast<int>(v[c]) >= T) ? (1u << c) : 0u;
-            if (n_valid < kHalfRows) m &= (n_valid > 0) ? ((1u << n_valid) - 1u) : 0u;   // shard tail
-            if constexpr (SEL) m &= sel_word;
-            uint32_t any = __reduce_or_sync(0xffffffffu, m);
-            if (__popc(any) > 6) {   // busy word: unrolled predicated stores, v[] stays in registers
-              if (m) {
-#pragma unroll
-                for (int c = 0; c < kHalfRows; ++c) {
-                  if ((m >> c) & 1u) {
-                    const uint32_t bits = __float_as_uint(i8_score(static_cast<int>(v[c]), sq, st));
-                    const int slot = n_mine + __popc(m & ((1u << c) - 1u));
-                    if (slot < a.cap_p) my_list[slot] = pack_cand(__uint_as_float(bits), static_cast<uint32_t>(row0 + c));
-                    count_hit(bits);
-                  }
+              for (int c = 0; c < kHalfRows; ++c) {
+                if ((m >> c) & 1u) {
+                  const uint32_t bits = __float_as_uint(i8_score(static_cast<int>(v[c]), sq, st));
+                  const int slot = n_mine + __popc(m & ((1u << c) - 1u));
+                  if (slot < a.cap_p) my_list[slot] = pack_cand(__uint_as_float(bits), static_cast<uint32_t>(row0 + c));
+                  count_hit(bits);
                 }
-                n_mine += __popc(m);
               }
-              any = 0;
+              n_mine += __popc(m);
             }
-            while (any) {
-              const int c = __ffs(any) - 1;
-              any &= any - 1;
-              const uint32_t acc = tmem_ld_x1(col0 + c);
-              tmem_ld_wait();
-              if ((m >> c) & 1u) {
-                const uint32_t bits = __float_as_uint(i8_score(static_cast<int>(acc), sq, st));
-                if (n_mine < a.cap_p) my_list[n_mine] = pack_cand(__uint_as_float(bits), static_cast<uint32_t>(row0 + c));
-                ++n_mine;
-                count_hit(bits);
-              }
+            any = 0;
+          }
+          while (any) {
+            const int c = __ffs(any) - 1;
+            any &= any - 1;
+            const uint32_t acc = tmem_ld_x1(col0 + c);
+            tmem_ld_wait();
+            if ((m >> c) & 1u) {
+              const uint32_t bits = __float_as_uint(i8_score(static_cast<int>(acc), sq, st));
+              if (n_mine < a.cap_p) my_list[n_mine] = pack_cand(__uint_as_float(bits), static_cast<uint32_t>(row0 + c));
+              ++n_mine;
+              count_hit(bits);
             }
           }
         }
-      } else if (a.dense) {
-        // bootstrap: every score of this half tile goes to the private area (zeros for rows past the end)
-        if (q_ok && n_mine + kHalfRows <= a.cap_p) {
-          uint64_t* dst = my_list + n_mine;
-#pragma unroll
-          for (int c = 0; c < kHalfRows; c += 2) {
-            ulonglong2 o;
-            o.x = (c < n_valid && ((sel_word >> c) & 1u)) ? pack_cand(__uint_as_float(v[c]), static_cast<uint32_t>(row0 + c)) : 0ull;
-            o.y = (c + 1 < n_valid && ((sel_word >> (c + 1)) & 1u)) ? pack_cand(__uint_as_float(v[c + 1]), static_cast<uint32_t>(row0 + c + 1)) : 0ull;
-            *reinterpret_cast<ulonglong2*>(dst + c) = o;
-          }
-        }
-        n_mine += kHalfRows;
       } else if (__any_sync(0xffffffffu, any_ge32(v, tau))) {     // the common case is: no lane hits
         // One predicate bit per score; hits are handled in a warp-uniform loop over the columns any lane
         // flagged, re-reading that single column from TMEM (a dynamic register index would demote v[] to
@@ -721,69 +739,18 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1)
     }
     __syncwarp();
     if (lane == 0) atomicAdd(const_cast<int*>(epi_done_s), 1);
-  } else if (warp == kUmmaRefresherWarp && a.tighten && !a.dense) {
+  } else if (warp == kUmmaRefresherWarp) {
     // ===================== refresher: in-kernel threshold tightening =====================
-    // While the stream runs, this otherwise idle warp keeps reading, for the queries assigned to
-    // this CTA (q = blockIdx.x, + gridDim.x, ...), the histogram of hits above the bootstrap's k-th
-    // score and raises tau[q] to (lower edge of the highest bucket b with >= k hits in buckets >= b)
-    // - 2*eps.  At least k rows seen so far have an approximate score >= that edge, so the k-th best
-    // approximate score of any superset is >= it: the bound of DESIGN.md section 4 holds for every
-    // intermediate value, whatever the interleaving (counts only grow; a stale read is a smaller
-    // suffix sum, i.e. a lower, still valid, threshold).  Every hit with key >= hkey0 is counted by
-    // every pair because all thresholds in use are <= the current one.  Effect: the pass rate
-    // follows k/rows_seen continuously, so ONE launch streams the whole shard after the bootstrap.
+    // While the stream runs, this otherwise idle warp keeps raising tau[q] of the queries assigned to
+    // this CTA (q = blockIdx.x, + gridDim.x, ...) from their hit histograms (refresh_threshold).  Every
+    // hit with key >= hkey0 is counted by every pair because all thresholds in use are <= the current
+    // one.  Effect: the pass rate follows k/rows_seen continuously, so ONE launch streams the whole shard.
     float last[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
     const long long t_start = clock64();
     while (*epi_done_s < kUmmaEpiWarps) {
       int qi = 0;
-      for (int q = blockIdx.x; q < a.nq; q += gridDim.x, ++qi) {
-        const uint32_t key0 = a.hkey0[q];
-        if (key0 == 0xffffffffu) continue;     // fewer than k rows seen by the bootstrap: nothing to reject
-        // lane l owns buckets [16l, 16l+16).  One 128-byte read of the 32 coarse counters per round; only
-        // the lane where the suffix sum crosses k reads its 16 fine buckets (192 B per query and round
-        // instead of 2 KB: the polling shares the L2 -> SM path with the 6 TB/s passage stream).
-        const unsigned int* hq = a.hist + static_cast<int64_t>(q) * kHistStride;
-        const unsigned int mine = __ldcv(hq + kHistBuckets + lane);
-        unsigned int suf = mine;               // hits in the buckets of lanes >= this one
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const unsigned int t = __shfl_down_sync(0xffffffffu, suf, o);
-          if (lane + o < 32) suf += t;
-        }
-        const unsigned int kk = static_cast<unsigned int>(a.k);
-        unsigned int above = suf - mine;
-        int b = -1;
-        if (suf >= kk && above < kk) {         // exactly one lane: walk its 16 fine buckets from the top
-          const uint4* hp = reinterpret_cast<const uint4*>(hq) + 4 * lane;
-#pragma unroll
-          for (int u = 3; u >= 0; --u) {
-            const uint4 h4 = __ldcv(hp + u);
-            const unsigned int c4[4] = {h4.x, h4.y, h4.z, h4.w};
-#pragma unroll
-            for (int j = 3; j >= 0; --j) {
-              if (b < 0) {
-                above += c4[j];
-                if (above >= kk) b = 16 * lane + 4 * u + j;
-              }
-            }
-          }
-        }
-        const unsigned int who = __ballot_sync(0xffffffffu, b >= 0);
-        if (who == 0u) continue;
-        b = __shfl_sync(0xffffffffu, b, __ffs(who) - 1);
-        if (lane == 0) {
-          const uint64_t edge = static_cast<uint64_t>(key0) + (static_cast<uint64_t>(b) << a.hshift[q]);
-          if (edge <= 0xff7fffffull) {         // a finite score key
-            const float t = __fsub_rd(key2f(static_cast<uint32_t>(edge)),
-                                      a.count_exact_lower_bound ? __fmul_ru(a.margin[q], 0.5f) : a.margin[q]);
-            const float prev = (qi < 4) ? last[qi] : *reinterpret_cast<volatile float*>(a.tau + q);
-            if (t > prev) {
-              *reinterpret_cast<volatile float*>(a.tau + q) = t;
-              if (qi < 4) last[qi] = t;
-            }
-          }
-        }
-      }
+      for (int q = blockIdx.x; q < a.nq; q += gridDim.x, ++qi)
+        refresh_threshold(a.hist, a.hkey0[q], a.hshift, a.margin, a.tau, a.k, q, qi, lane, last);
       unsigned int pause = static_cast<unsigned int>(a.tighten);
       const long long age_ns = (clock64() - t_start) >> 1;       // cycles -> ns at ~2 GHz; only a pacing hint
       if (age_ns < 30000) pause = min(pause, 500u);              // start of the pass: epilogue threads wait for the first thresholds

@@ -577,60 +577,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
     if (lane == 0) atomicAdd(const_cast<int*>(epi_done_s), 1);
   } else if (warp == kQsRefresherWarp) {
     // ===================== refresher: in-kernel threshold tightening =====================
-    // Same scheme as the TS variant (kernels_umma.cuh): for the queries assigned to this CTA, read the
-    // histogram of hits (counted at s~ - eps), find the highest bucket b with >= k hits at or above it and
-    // publish tau[q] = edge(b) - eps; additionally copy ALL current thresholds into this CTA's shared memory,
-    // where the epilogue threads (one passage row each, all queries) read them.
+    // Same rule as the TS variant (refresh_threshold) for the queries assigned to this CTA; additionally copy
+    // ALL current thresholds into this CTA's shared memory, where the epilogue threads (one passage row each,
+    // all queries) read them.
     float last[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
     const long long t_start = clock64();
     while (*epi_done_s < kQsEpiWarps) {
       int qi = 0;
-      if (a.tighten) {
-        for (int q = blockIdx.x; q < a.nq; q += gridDim.x, ++qi) {
-          const uint32_t key0 = hkey0_s[q];
-          if (key0 == 0xffffffffu) continue;
-          const unsigned int* hq = a.hist + static_cast<int64_t>(q) * kHistStride;
-          const unsigned int mine = __ldcv(hq + kHistBuckets + lane);
-          unsigned int suf = mine;               // hits in the buckets of lanes >= this one
-#pragma unroll
-          for (int o = 1; o < 32; o <<= 1) {
-            const unsigned int tt = __shfl_down_sync(0xffffffffu, suf, o);
-            if (lane + o < 32) suf += tt;
-          }
-          const unsigned int kk = static_cast<unsigned int>(a.k);
-          unsigned int above = suf - mine;
-          int b = -1;
-          if (suf >= kk && above < kk) {         // exactly one lane: walk its 16 fine buckets from the top
-            const uint4* hp = reinterpret_cast<const uint4*>(hq) + 4 * lane;
-#pragma unroll
-            for (int u = 3; u >= 0; --u) {
-              const uint4 h4 = __ldcv(hp + u);
-              const unsigned int c4[4] = {h4.x, h4.y, h4.z, h4.w};
-#pragma unroll
-              for (int j = 3; j >= 0; --j) {
-                if (b < 0) {
-                  above += c4[j];
-                  if (above >= kk) b = 16 * lane + 4 * u + j;
-                }
-              }
-            }
-          }
-          const unsigned int who = __ballot_sync(0xffffffffu, b >= 0);
-          if (who == 0u) continue;
-          b = __shfl_sync(0xffffffffu, b, __ffs(who) - 1);
-          if (lane == 0) {
-            const uint64_t edge = static_cast<uint64_t>(key0) + (static_cast<uint64_t>(b) << a.hshift[q]);
-            if (edge <= 0xff7fffffull) {         // a finite score key
-              const float t = __fsub_rd(key2f(static_cast<uint32_t>(edge)), __fmul_ru(a.margin[q], 0.5f));   // e - eps
-              const float prev = (qi < 4) ? last[qi] : *reinterpret_cast<volatile float*>(a.tau + q);
-              if (t > prev) {
-                *reinterpret_cast<volatile float*>(a.tau + q) = t;
-                if (qi < 4) last[qi] = t;
-              }
-            }
-          }
-        }
-      }
+      for (int q = blockIdx.x; q < a.nq; q += gridDim.x, ++qi)
+        refresh_threshold(a.hist, hkey0_s[q], a.hshift, a.margin, a.tau, a.k, q, qi, lane, last);
       // thresholds published by every CTA -> this CTA's shared memory (they only rise)
       bool all_finite = true;
       for (int i = lane; i < a.nq; i += 32) {
@@ -643,7 +598,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kQsThreads, 1)
         all_finite = all_finite && (t > -INFINITY);
       }
       if (__all_sync(0xffffffffu, all_finite) && lane == 0) *tau_ready_s = 1;
-      unsigned int pause = static_cast<unsigned int>(a.tighten > 0 ? a.tighten : 2000);
+      unsigned int pause = static_cast<unsigned int>(a.tighten);
       if (*tau_ready_s == 0) pause = 500;     // start of the pass: epilogue warps are waiting for the first thresholds
       else if (a.tighten_adaptive) {
         const long long age_ns = (clock64() - t_start) >> 1;     // cycles -> ns at ~2 GHz; only a pacing hint

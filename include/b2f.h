@@ -297,12 +297,11 @@ void* b2f_stream(b2f_index* idx, int shard);
  *   "qs_half_stage" (QS: 8 KB half stages with the 64-byte swizzle when <= 5 full stages fit; default 0, measured slower),
  *   "synth_mean_shift" (b2f_add_synthetic: integer shift M of every component along a fixed sign
  *       vector per seed, 0 = isotropic rows; see convdr_b200/synth.py),
- *   "tighten" (TS engine: in-kernel threshold tightening, minimum pause of the refresher warp in
- *       ns, default 2000; 0 = geometric phases with a refresh kernel between them),
+ *   "tighten" (tensor engine: thresholds start at -inf and are tightened inside the one scoring
+ *       launch of a pass; minimum pause of the refresher warp in ns, 1..1000000, default 2000),
  *   "tighten_adaptive" (default 1: the pause grows with the elapsed kernel time),
- *   "bootstrap" (default 0: thresholds start at -inf inside the single launch; 1: dense bootstrap
- *       launch + bootstrap_select_kernel first), "growth" (phase growth factor of the phased
- *       schedules),
+ *   "growth" (phase growth factor of the SIMT scans' phased schedule; also sizes the private list
+ *       areas of the tensor engine),
  *   "profile" (1: CUDA events around every scoring / selection launch),
  *   "reset_stats" (any value: zero the counters below).                          */
 int b2f_set_option(b2f_index* idx, const char* key, int64_t value);
